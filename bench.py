@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (CUDA, sm_100a)
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 One "step" = one pass of the hot path over one batch of synthetic images PER GPU (weak scaling):
   training side    S3FD 640x640 pyramid (34 125 anchors), encode_anchors(match_mining=True), thresholds 0.4/0.4,
@@ -38,6 +39,7 @@ CPU_CFG = dict(kind="s3fd", size=IMAGE, pos=0.4, ign=0.4, mining=True, max_gt=50
 # kernels of one step (the memset node aside): enc_pass1, enc_pass2_find, enc_pass2_apply, enc_pass3, nms_greedy
 # (+ the NCCL kernel at N > 1)
 KERNELS_PER_STEP = 5
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def workload_config(batch, n_gpus):
@@ -254,6 +256,26 @@ def log(msg):
 _T0 = time.time()
 
 
+def step_outputs(hp, image_ids):
+    """What HotPath.step() handed its caller in the step that last used `hp`: the encode outputs and the detections, as
+    float32 host arrays (labels, counts and indices are integers below 2^24, exact in float32).  Above DUMP_LIMIT_BYTES
+    a fixed, seeded sample of the images is kept; `image_id` names the synthetic image of every row."""
+    import numpy as np
+    import torch
+    counts, scores, boxes = hp._slab.views()
+    targets, labels, enc_scores, matched = hp._enc_out[:4]
+    out = {"enc_targets": targets, "enc_labels": labels, "enc_scores": enc_scores, "enc_matched_gt": matched,
+           "det_boxes": boxes, "det_scores": scores, "det_counts": counts, "det_anchor_index": hp._aux[0], "det_keep_pos": hp._aux[1]}
+    n = len(image_ids)
+    per_image = 8 + sum(4 * t[0].numel() for t in out.values())
+    keep = min(n, DUMP_LIMIT_BYTES // per_image)
+    rows = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    idx = torch.from_numpy(rows).to(boxes.device)
+    res = {name: t.index_select(0, idx).float().cpu().numpy() for name, t in out.items()}
+    res["image_id"] = np.asarray(image_ids, np.float64)[rows]
+    return res
+
+
 def run_cuda(args):
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -352,7 +374,7 @@ def run_cuda(args):
         hp = pipeline.HotPath(a_train[:4], a_train[4], enc_params, pp_params, anchors_eval=a_eval[:4],
                               workspaces=ws_lanes[r % L], overlap=not args.no_overlap, device_gather=gathers[r % L],
                               recv_buffer=None if peers is not None else recv, peer_exchange=peers, peer_set=r)
-        sets.append({"host": h, "dev": d, "hp": hp, "recv": recv, "total_gt": int(offs[-1])})
+        sets.append({"host": h, "dev": d, "hp": hp, "recv": recv, "total_gt": int(offs[-1]), "image_id": [base + i for i in order]})
     total_gt_mean = float(np.mean([s["total_gt"] for s in sets]))
 
     # kernels of this library per step: enc_pass1, enc_pass2_find, enc_pass2_apply, enc_pass3, nms_greedy (+ the warp table of
@@ -459,11 +481,17 @@ def run_cuda(args):
         barrier()
         return e0.elapsed_time(e1)
 
-    serial_ms = timed(True) if L > 1 else None       # one step at a time: the latency of a step
-    elapsed_ms = timed(False)
-    log("timed regions done: %.3f ms/step" % (elapsed_ms / K))
-    run_steps(n_tail)                                # keep the GPU busy a little longer: the clock sampler sees the loaded state
-    clocks = sampler.stop() if sampler else None
+    dumped = None
+    try:
+        serial_ms = timed(True) if L > 1 else None       # one step at a time: the latency of a step
+        elapsed_ms = timed(False)
+        log("timed regions done: %.3f ms/step" % (elapsed_ms / K))
+        if args.dump_outputs and rank == 0:
+            last = sets[(W + K - 1) % R]                 # the buffer set of the last timed step
+            dumped = step_outputs(last["hp"], last["image_id"])
+        run_steps(n_tail)                                # keep the GPU busy a little longer: the clock sampler sees the loaded state
+    finally:
+        clocks = sampler.stop() if sampler else None     # never leave nvidia-smi running
     t = torch.tensor([elapsed_ms, serial_ms if serial_ms is not None else elapsed_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -686,6 +714,10 @@ def run_cuda(args):
                                   "frac": enc_flops / (kernel_ms["enc_pass1"] * 1e-3) / p_fp32},
     }
 
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if rank == 0:
         line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
                 "ms_per_step": elapsed_ms / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -745,7 +777,14 @@ def main():
     ap.add_argument("--no-overlap", action="store_true", help="run encode and postprocess on one stream")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-layout-hint", action="store_true", help="encode without the pyramid layout hint (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one (rank 0's encode outputs and detections, "
+                         "float32, at most 64 MB) as DIR/<name>.npy; the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs needs the CUDA arm")
     if args.impl == "reference":
         return run_reference(args)
     return run_cuda(args)

@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import torch
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 COMMON = ["metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",
           "dtype", "data", "config", "e2e", "cpu_baseline"]
@@ -66,3 +69,41 @@ def test_rank_pinning_helpers():
                 assert not (mine0 & mine1)
         finally:
             os.sched_setaffinity(0, before)
+
+
+def test_step_outputs_for_dump(monkeypatch):
+    """--dump-outputs: every output of the step as float32 with one row per image (image_id float64), and above the size
+    limit the same seeded sample of the images on every call."""
+    sys.path.insert(0, ROOT)
+    import bench
+    from dan_b200 import pipeline
+
+    class Step(object):
+        pass
+    B, N, K = 6, 40, 5
+    gen = torch.Generator().manual_seed(0)
+    hp = Step()
+    hp._slab = pipeline.DetectionSlab(B, 1, K, "cpu")
+    hp._slab.buf.copy_(torch.rand(hp._slab.words, generator=gen))
+    hp._slab.views()[0].copy_(torch.arange(B, dtype=torch.int32).view(B, 1))
+    hp._enc_out = (torch.rand(B, N, 4, generator=gen), torch.randint(-1, 2, (B, N), generator=gen), torch.rand(B, N, generator=gen),
+                   torch.rand(B, N, 4, generator=gen), None)
+    hp._aux = tuple(torch.randint(-1, 5000, (B, 1, K), dtype=torch.int32, generator=gen) for _ in range(2))
+    ids = [100 + i for i in range(B)]
+    full = bench.step_outputs(hp, ids)
+    assert set(full) == {"enc_targets", "enc_labels", "enc_scores", "enc_matched_gt", "det_boxes", "det_scores", "det_counts",
+                         "det_anchor_index", "det_keep_pos", "image_id"}
+    assert full["image_id"].dtype == np.float64 and all(v.dtype == np.float32 for k, v in full.items() if k != "image_id")
+    assert all(v.shape[0] == B for v in full.values())
+    np.testing.assert_array_equal(full["enc_labels"], hp._enc_out[1].numpy())
+    np.testing.assert_array_equal(full["det_counts"][:, 0], np.arange(B))
+    np.testing.assert_array_equal(full["det_keep_pos"], hp._aux[1].numpy())
+
+    per_image = sum(v[0].nbytes for v in full.values())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 3 * per_image + 1)
+    a, b = bench.step_outputs(hp, ids), bench.step_outputs(hp, ids)
+    assert a["image_id"].shape == (3,) and sum(v.nbytes for v in a.values()) <= bench.DUMP_LIMIT_BYTES
+    rows = (a["image_id"] - 100).astype(np.int64)
+    for name in full:
+        np.testing.assert_array_equal(a[name], b[name])
+        np.testing.assert_array_equal(a[name], full[name][rows])
