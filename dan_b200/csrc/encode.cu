@@ -138,24 +138,36 @@ DAN_D AnchorBox load_anchor(const EncArgs& A, int a) {
   return ab;
 }
 
+// The original anchor box in centre form: all that the encode of a positive row and the signs of a negative row need.
+struct AnchorCtr {
+  float cy, cx, h, w;
+};
+
+DAN_D AnchorCtr anchor_ctr(float y0, float x0, float y1, float x1) {
+  AnchorCtr c;
+  point2center(y0, x0, y1, x1, c.cy, c.cx, c.h, c.w);
+  return c;
+}
+
 // Encode anchor `a` of image `b` against GT box g (anchor_manipulator.py:306-326 /
-// :366-387) and write every output row of a POSITIVE anchor.
-DAN_D void write_positive(const EncArgs& A, int64_t row, const AnchorBox& ab, float4 g, float score, int gt_index) {
+// :366-387) and write every output row of a POSITIVE anchor.  raw() returns the original anchor box, which only the
+// debug mode writes.
+template <typename RawBox>
+DAN_D void write_positive(const EncArgs& A, int64_t row, const AnchorCtr& ac, RawBox raw, float4 g, float score, int gt_index) {
   float4 t;
   if (A.debug) {
-    t = make_float4(ab.y0, ab.x0, ab.y1, ab.x1);
+    t = raw();
   } else {
-    float gcy, gcx, gh, gw, acy, acx, ah, aw;
+    float gcy, gcx, gh, gw;
     point2center(g.x, g.y, g.z, g.w, gcy, gcx, gh, gw);
-    point2center(ab.y0, ab.x0, ab.y1, ab.x1, acy, acx, ah, aw);
-    t.x = fdiv(fdiv(fsub(gcy, acy), ah), A.ps0);
-    t.y = fdiv(fdiv(fsub(gcx, acx), aw), A.ps1);
+    t.x = fdiv(fdiv(fsub(gcy, ac.cy), ac.h), A.ps0);
+    t.y = fdiv(fdiv(fsub(gcx, ac.cx), ac.w), A.ps1);
     if (A.pa_scale > 0.f) {
-      t.z = fdiv(cephes_logf(fdiv(fmul(gh, A.pa_scale), ah)), A.ps2);
-      t.w = fdiv(cephes_logf(fdiv(fmul(gw, A.pa_scale), aw)), A.ps3);
+      t.z = fdiv(cephes_logf(fdiv(fmul(gh, A.pa_scale), ac.h)), A.ps2);
+      t.w = fdiv(cephes_logf(fdiv(fmul(gw, A.pa_scale), ac.w)), A.ps3);
     } else {
-      t.z = fdiv(cephes_logf(fdiv(gh, ah)), A.ps2);
-      t.w = fdiv(cephes_logf(fdiv(gw, aw)), A.ps3);
+      t.z = fdiv(cephes_logf(fdiv(gh, ac.h)), A.ps2);
+      t.w = fdiv(cephes_logf(fdiv(gw, ac.w)), A.ps3);
     }
   }
   A.targets[row] = t;
@@ -163,6 +175,17 @@ DAN_D void write_positive(const EncArgs& A, int64_t row, const AnchorBox& ab, fl
   A.scores[row] = score;
   if (A.matched != nullptr) A.matched[row] = g;
   if (A.match32 != nullptr) A.match32[row] = gt_index;
+}
+
+// the original anchor box, for the debug mode of fused pass 1 (which keeps the centre form only): out of line, so that
+// the common path does not carry its loads
+__device__ __noinline__ float4 raw_anchor(const float* y0, const float* x0, const float* y1, const float* x1, int a) {
+  return make_float4(y0[a], x0[a], y1[a], x1[a]);
+}
+
+DAN_D void write_positive(const EncArgs& A, int64_t row, const AnchorBox& ab, float4 g, float score, int gt_index) {
+  write_positive(A, row, anchor_ctr(ab.y0, ab.x0, ab.y1, ab.x1), [&] { return make_float4(ab.y0, ab.x0, ab.y1, ab.x1); }, g,
+                 score, gt_index);
 }
 
 // ---------------------------------------------------------------------------
@@ -477,26 +500,47 @@ __global__ void __launch_bounds__(kEncThreads) enc_pass2_kernel(const EncArgs A)
 
 // ---------------------------------------------------------------------------
 // FUSED path, passes 1 and 2 as warp-autonomous kernels.
-//   * a warp owns 32 consecutive anchors and walks kEncImgPerWarp images with them: the anchor loads, the PA
-//     transform, the areas and the warp bounding box are paid once per group of images;
+//   * a CTA of pass 1 owns a chunk of kFusedThreads anchors (a warp: 32 of them) and walks one image or, on the fine
+//     pyramid levels, a group of images with them: the anchor loads, the mask, the warp -> anchors table,
+//     the PA transform, the warp bounding box and the anchors' centre form are paid once per CTA;
 //   * no shared memory and no CTA barrier: the ground truth of an image is a few hundred bytes, read through the
 //     read-only path (32 boxes per coalesced load for the cull test, broadcast loads for the hits);
 //   * per-GT column maxima of pass 1 are reduced in the warp (redux.sync) and the lane that loaded GT k issues one
 //     atomicMax for it, so the atomics of a warp go to 32 different addresses.
 // The dense-matrix kernels above keep the tiled shared-memory scheme (they have to transpose the matrix).
 // ---------------------------------------------------------------------------
-// images per warp pass: runtime (DAN_ENC_IMAGES_PER_WARP, default 1: more, smaller CTAs balance better on 148 SMs)
+constexpr int kFusedThreads = 128;
 
-struct WarpAnchors {
-  AnchorBox ab;
-  WarpBox wb;
-  bool valid, active;
-  int a;
-};
-
-// index of the calling warp of fused pass 1 (wbest / wbox / queue entries are per warp).  Recomputed where it is needed
-// rather than kept: the kernel runs under a 32-register cap.
-DAN_D int fused_warp_id() { return (gridDim.y - 1 - blockIdx.y) * (blockDim.x >> 5) + (threadIdx.x >> 5); }
+// Timeline of fused pass 1, for tools/pass1_timeline.py: with -DDAN_PASS1_TIMELINE lane 0 of every warp writes the
+// global timer (ns) at its start and end and the number of images it walked; otherwise the macros are empty.
+#ifdef DAN_PASS1_TIMELINE
+constexpr int kTimelineWarps = 1 << 16;
+__device__ unsigned long long g_p1_timeline[3 * kTimelineWarps];
+DAN_D unsigned long long global_ns() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+#define DAN_P1_MARK(slot, value)                                                          \
+  do {                                                                                    \
+    const unsigned w__ = blockIdx.x * (kFusedThreads / 32) + (threadIdx.x >> 5);        \
+    if ((threadIdx.x & 31) == 0 && w__ < kTimelineWarps) g_p1_timeline[3 * w__ + (slot)] = (value); \
+  } while (0)
+#else
+#define DAN_P1_MARK(slot, value) do { } while (0)
+#endif
+// Images per CTA of pass 1 on the fine levels.  A warp there meets ~2 GTs per image (~150 warp instructions) against
+// ~350 instructions of per-(warp, image) bookkeeping, so it walks several images; a warp of a coarse level meets every
+// GT of the image and keeps one, so that it does not become the tail of the launch (profiles/r03_pass1_breakdown.md).
+// Measured on B200 at batch 32: 2 images give back 3.5 % of the rate with steps in flight, 8 add 1 % to it but make a
+// lone pass 1 30 % longer.
+#ifndef DAN_ENC_FINE_IMAGES
+#define DAN_ENC_FINE_IMAGES 4
+#endif
+constexpr int kFineImages = DAN_ENC_FINE_IMAGES;
+// a hinted level of at least this many cells (32 warps) counts as fine: at 640^2 the 160^2 / 80^2 / 40^2 levels
+// (2.1 / 2.7 / 4.4 culled GTs per warp and image), not the 20^2 one (11.8)
+constexpr int kFineMinCells = 1024;
 
 // Which anchor lane `lane` of warp `wid` owns.  Without a layout hint a warp holds 32 consecutive anchors: on a pyramid
 // level that is a 32 x 1 strip of cells, whose bounding box meets far more ground-truth boxes than its anchors do.
@@ -507,29 +551,6 @@ DAN_D int warp_anchor(const EncArgs& A, int wid, int lane) {
   if (A.warp_map == nullptr) return wid * 32 + lane;
   const int2 m = __ldg(A.warp_map + wid);
   return m.x + (lane >> 3) * m.y + (lane & 7);
-}
-
-template <bool TILED>
-DAN_D WarpAnchors load_warp_anchors(const EncArgs& A) {
-  WarpAnchors w;
-  // grid = (image groups, anchor chunks): CTAs are dispatched x-fastest, so all images of one anchor chunk start
-  // together, and the chunks are walked from the END of the anchor array: the coarse pyramid levels live there, their
-  // warps see every GT and run the longest, so they must not be the tail of the launch
-  if (TILED) {
-    const int wid = fused_warp_id();
-    w.a = (wid < ((A.n + 31) >> 5)) ? warp_anchor(A, wid, threadIdx.x & 31) : A.n;
-  } else {
-    w.a = (gridDim.y - 1 - blockIdx.y) * blockDim.x + threadIdx.x;
-  }
-  w.valid = w.a < A.n;
-  w.ab = AnchorBox{};
-  w.active = false;
-  if (w.valid) {
-    w.ab = load_anchor(A, w.a);
-    w.active = (A.mask == nullptr) || (A.mask[w.a] != 0);
-  }
-  w.wb = warp_bbox(w.active, w.ab);
-  return w;
 }
 
 // stage 1 of either matcher from the row maximum (small_mining_match.cc:85-93 / anchor_manipulator.py:67-76)
@@ -582,18 +603,18 @@ DAN_D uint32_t log_ratio_sign(float num, float den) {
 
 // every output row of a NON-positive anchor; the 44 B/anchor of a step are written once and not read again by the
 // encode kernels: streaming stores
-DAN_D void write_negative(const EncArgs& A, int64_t row, const AnchorBox& ab, const NegCtx& c, float score, int match) {
+template <typename RawBox>
+DAN_D void write_negative(const EncArgs& A, int64_t row, const AnchorCtr& ac, RawBox raw, const NegCtx& c, float score, int match) {
   float4 t;
   if (A.debug) {
-    t = make_float4(__uint_as_float(sign_of(ab.y0)), __uint_as_float(sign_of(ab.x0)), __uint_as_float(sign_of(ab.y1)),
-                    __uint_as_float(sign_of(ab.x1)));
+    const float4 r = raw();
+    t = make_float4(__uint_as_float(sign_of(r.x)), __uint_as_float(sign_of(r.y)), __uint_as_float(sign_of(r.z)),
+                    __uint_as_float(sign_of(r.w)));
   } else {
-    float acy, acx, ah, aw;
-    point2center(ab.y0, ab.x0, ab.y1, ab.x1, acy, acx, ah, aw);
-    t.x = __uint_as_float(sign_of(fsub(c.gcy, acy)) ^ sign_of(ah) ^ c.ps_sign[0]);
-    t.y = __uint_as_float(sign_of(fsub(c.gcx, acx)) ^ sign_of(aw) ^ c.ps_sign[1]);
-    t.z = __uint_as_float(log_ratio_sign(c.gh, ah) ^ c.ps_sign[2]);
-    t.w = __uint_as_float(log_ratio_sign(c.gw, aw) ^ c.ps_sign[3]);
+    t.x = __uint_as_float(sign_of(fsub(c.gcy, ac.cy)) ^ sign_of(ac.h) ^ c.ps_sign[0]);
+    t.y = __uint_as_float(sign_of(fsub(c.gcx, ac.cx)) ^ sign_of(ac.w) ^ c.ps_sign[1]);
+    t.z = __uint_as_float(log_ratio_sign(c.gh, ac.h) ^ c.ps_sign[2]);
+    t.w = __uint_as_float(log_ratio_sign(c.gw, ac.w) ^ c.ps_sign[3]);
   }
   __stcs(A.targets + row, t);
   __stcs(reinterpret_cast<long long*>(A.labels) + row, (long long)((match < -1) ? -1 : 0));   // anchor_manipulator.py:300-302
@@ -613,22 +634,56 @@ DAN_D void write_negative(const EncArgs& A, int64_t row, const AnchorBox& ab, co
 #define DAN_ENC_TILED_BLOCKS 6   // 40 registers: no spills (A/B on B200: +1 % over the 32-register build)
 #endif
 template <bool NEED_ROW, bool MINING, bool TILED>
-__global__ void __launch_bounds__(kEncThreads, TILED ? DAN_ENC_TILED_BLOCKS : 8) enc_pass1_fused_kernel(const EncArgs A, int batch, int ipw) {
+__global__ void __launch_bounds__(kEncThreads, TILED ? DAN_ENC_TILED_BLOCKS : 6)
+enc_pass1_fused_kernel(const EncArgs A, int batch, int coarse_chunks) {
+  DAN_P1_MARK(0, global_ns());
   const int lane = threadIdx.x & 31;
-  const WarpAnchors W = load_warp_anchors<TILED>(A);
   const int nwarps = (A.n + 31) >> 5;
-  if (blockIdx.x == 0 && lane == 0 && (TILED ? fused_warp_id() : (W.a >> 5)) < nwarps)
-    A.wbox[TILED ? fused_warp_id() : (W.a >> 5)] = make_float4(W.wb.y0, W.wb.x0, W.wb.y1, W.wb.x1);
-  const int b_end = min(batch, (int)(blockIdx.x + 1) * ipw);
-  for (int b = blockIdx.x * ipw; b < b_end; ++b) {
+  const int nchunks = (A.n + kFusedThreads - 1) / kFusedThreads;
+  // CTA -> (anchor chunk, images [b0, b_end)).  The chunks are walked from the END of the anchor array: the coarse
+  // pyramid levels live there, their warps see every GT and run the longest, so they must not be the tail of the
+  // launch.  The last `coarse_chunks` chunks come first, one CTA per image, all images of a chunk next to each other;
+  // then the fine chunks, one CTA per group of kFineImages images.  Fine chunks exist only with the layout hint, i.e. in
+  // the TILED instantiation.
+  int from_end, b0, b_end;
+  const int coarse_ctas = coarse_chunks * batch;
+  if (!TILED || (int)blockIdx.x < coarse_ctas) {
+    from_end = blockIdx.x / batch;
+    b0 = blockIdx.x - from_end * batch;
+    b_end = b0 + 1;
+  } else {
+    const int groups = (batch + kFineImages - 1) / kFineImages;
+    const int j = blockIdx.x - coarse_ctas;
+    const int c = j / groups;
+    from_end = coarse_chunks + c;
+    b0 = (j - c * groups) * kFineImages;
+    b_end = min(batch, b0 + kFineImages);
+  }
+  // the warp's index (wbest / wbox / queue entries are per warp) and its anchors
+  const int wid = (nchunks - 1 - from_end) * (kFusedThreads / 32) + (threadIdx.x >> 5);
+  const int a = TILED ? ((wid < nwarps) ? warp_anchor(A, wid, lane) : A.n) : wid * 32 + lane;
+  const bool valid = a < A.n;
+  AnchorBox ab = {};
+  AnchorCtr ac = {};
+  bool active = false;
+  if (valid) {
+    ab = load_anchor(A, a);
+    ac = anchor_ctr(ab.y0, ab.x0, ab.y1, ab.x1);
+    active = (A.mask == nullptr) || (A.mask[a] != 0);
+  }
+  const WarpBox wb = warp_bbox(active, ab);
+  if (b0 == 0 && lane == 0 && wid < nwarps) A.wbox[wid] = make_float4(wb.y0, wb.x0, wb.y1, wb.x1);
+  const auto raw = [&] { return raw_anchor(A.ay0, A.ax0, A.ay1, A.ax1, a); };
+  for (int b = b0; b < b_end; ++b) {
     const ImageGt ig = image_gt<false>(A, b);
-    const NegCtx neg = neg_ctx(A, ig);
     float best = 0.f;
     int best_gt = 0;
     for (int k0 = 0; k0 < ig.m_eff; k0 += 32) {
       const int k = k0 + lane;
-      const float4 gk = (k < ig.m_eff) ? gt_box(A, ig, k) : make_float4(0.f, 0.f, 0.f, 0.f);
-      unsigned hits = __ballot_sync(0xffffffffu, (k < ig.m_eff) && may_hit(W.wb, gk));
+      // (gt_box(A, ig, k) for k < m_eff; the lanes beyond m_eff stay out of the ballot and are never broadcast)
+      float4 gk = make_float4(0.f, 0.f, 1.f, 1.f);
+      if (k < ig.m_real) gk = __ldg(A.gt + ig.off0 + k);
+      unsigned hits = __ballot_sync(0xffffffffu, (k < ig.m_eff) && may_hit(wb, gk));
       const float gk_area = box_area(gk.x, gk.y, gk.z, gk.w);      // once per GT, broadcast with the box below
       uint32_t my_colmax = 0u;            // column maximum of GT k over this warp's anchors
       while (hits) {
@@ -640,7 +695,7 @@ __global__ void __launch_bounds__(kEncThreads, TILED ? DAN_ENC_TILED_BLOCKS : 8)
         const float g_area = __shfl_sync(0xffffffffu, gk_area, kl);
         bool hit = false;
         float ov = 0.f;
-        if (W.active) ov = pair_iou(W.ab.my0, W.ab.mx0, W.ab.my1, W.ab.mx1, W.ab.marea, g.x, g.y, g.z, g.w, g_area, hit);
+        if (active) ov = pair_iou(ab.my0, ab.mx0, ab.my1, ab.mx1, ab.marea, g.x, g.y, g.z, g.w, g_area, hit);
         const uint32_t wmax = __reduce_max_sync(0xffffffffu, (ov > 0.f) ? __float_as_uint(ov) : 0u);
         if (lane == kl) my_colmax = wmax;
         if (ov > best) { best = ov; best_gt = k0 + kl; }      // first strictly-greatest GT wins (tf.argmax / :76-83)
@@ -649,27 +704,28 @@ __global__ void __launch_bounds__(kEncThreads, TILED ? DAN_ENC_TILED_BLOCKS : 8)
           // unmatched is only known after stage 2, pass 3 filters on that
           const int pos = atomicAdd(A.fill + ig.slot0 + k0 + kl, 1);
           if (pos < kBucketCap)
-            A.bucket[(int64_t)(ig.slot0 + k0 + kl) * kBucketCap + pos] = HeapItem{ov, W.a};
+            A.bucket[(int64_t)(ig.slot0 + k0 + kl) * kBucketCap + pos] = HeapItem{ov, a};
         }
       }
       if (my_colmax != 0u) atomicMax(A.colmax + ig.slot0 + k, my_colmax);
     }
     // no overlap of this warp exceeds the largest row maximum of its lanes: pass 2 uses it to skip the warp
     const uint32_t wbest = __reduce_max_sync(0xffffffffu, __float_as_uint(best));
-    if (lane == 0 && (TILED ? fused_warp_id() : (W.a >> 5)) < nwarps)
-      A.wbest[(int64_t)b * nwarps + (TILED ? fused_warp_id() : (W.a >> 5))] = __uint_as_float(wbest);     // (the last CTA may hold a warp beyond the anchors)
-    if (W.valid) {
+    if (lane == 0 && wid < nwarps) A.wbest[(int64_t)b * nwarps + wid] = __uint_as_float(wbest);   // (the last CTA may hold a warp beyond the anchors)
+    if (valid) {
       const int match = stage1_match<MINING>(A, best, best_gt);
-      const int64_t row = (int64_t)b * A.n + W.a;
+      const int64_t row = (int64_t)b * A.n + a;
       if (match >= 0) {
         if (MINING) atomicAdd(A.cnt + ig.slot0 + match, 1);
         if (NEED_ROW) A.haspos[ig.slot0 + match] = 1;          // anchor-side positive (anchor_manipulator.py:67-76)
-        write_positive(A, row, W.ab, gt_box(A, ig, match), best, match);
+        write_positive(A, row, ac, raw, gt_box(A, ig, match), best, match);
       } else {
-        write_negative(A, row, W.ab, neg, best, match);
+        write_negative(A, row, ac, raw, neg_ctx(A, ig), best, match);
       }
     }
   }
+  DAN_P1_MARK(1, global_ns());
+  DAN_P1_MARK(2, (unsigned long long)(b_end - b0) | ((unsigned long long)from_end << 32));
 }
 
 // pass 2 (fused path): stage 2 of the mining matcher (small_mining_match.cc:160-197) / the GT-side claim of the dual
@@ -1319,28 +1375,33 @@ static void bind_workspace(EncArgs& A, void* workspace, const WsLayout& w) {
   A.queue = reinterpret_cast<int2*>(base + w.queue);
 }
 
+// Fused pass 1.  fine_chunks: the leading chunks of kFusedThreads anchors that lie on fine pyramid levels; their CTAs
+// walk kFineImages images each.
+template <bool NEED_ROW, bool MINING, bool TILED>
+static void launch_pass1(const EncArgs& A, int batch, int fine_chunks, cudaStream_t st) {
+  const int coarse_chunks = (A.n + kFusedThreads - 1) / kFusedThreads - fine_chunks;
+  const int grid = coarse_chunks * batch + fine_chunks * ((batch + kFineImages - 1) / kFineImages);
+  enc_pass1_fused_kernel<NEED_ROW, MINING, TILED><<<grid, kFusedThreads, 0, st>>>(A, batch, coarse_chunks);
+}
+
 // ev (optional, 4 events): recorded before pass 1 and after each pass, for the profile entry point
 template <bool DENSE>
-static int run_passes(const EncArgs& A, bool mining, bool need_row, int batch, cudaStream_t st, cudaEvent_t* ev = nullptr) {
+static int run_passes(const EncArgs& A, bool mining, bool need_row, int batch, cudaStream_t st, cudaEvent_t* ev = nullptr,
+                      int fine_chunks = 0) {
   const dim3 grid((A.n + kEncThreads - 1) / kEncThreads, batch);
-  // sparse path: 128-thread CTAs, one image per CTA (sweeps on B200: 64/256 threads and 2-8 images per warp are
-  // within 2 % of this)
-  const int ipw = 1;
-  const int fthreads = 128;
-  const dim3 fgrid((batch + ipw - 1) / ipw, (A.n + fthreads - 1) / fthreads);
   if (ev) DAN_CUDA(cudaEventRecord(ev[0], st));
   if (DENSE) {
     if (need_row) enc_pass1_kernel<true, true><<<grid, kEncThreads, 0, st>>>(A);
     else enc_pass1_kernel<true, false><<<grid, kEncThreads, 0, st>>>(A);
   } else {
     if (A.warp_map != nullptr) {
-      if (mining) enc_pass1_fused_kernel<false, true, true><<<fgrid, fthreads, 0, st>>>(A, batch, ipw);
-      else if (need_row) enc_pass1_fused_kernel<true, false, true><<<fgrid, fthreads, 0, st>>>(A, batch, ipw);
-      else enc_pass1_fused_kernel<false, false, true><<<fgrid, fthreads, 0, st>>>(A, batch, ipw);
+      if (mining) launch_pass1<false, true, true>(A, batch, fine_chunks, st);
+      else if (need_row) launch_pass1<true, false, true>(A, batch, fine_chunks, st);
+      else launch_pass1<false, false, true>(A, batch, fine_chunks, st);
     } else {
-      if (mining) enc_pass1_fused_kernel<false, true, false><<<fgrid, fthreads, 0, st>>>(A, batch, ipw);
-      else if (need_row) enc_pass1_fused_kernel<true, false, false><<<fgrid, fthreads, 0, st>>>(A, batch, ipw);
-      else enc_pass1_fused_kernel<false, false, false><<<fgrid, fthreads, 0, st>>>(A, batch, ipw);
+      if (mining) launch_pass1<false, true, false>(A, batch, fine_chunks, st);
+      else if (need_row) launch_pass1<true, false, false>(A, batch, fine_chunks, st);
+      else launch_pass1<false, false, false>(A, batch, fine_chunks, st);
     }
   }
   DAN_LAUNCH_CHECK("enc_pass1_kernel");
@@ -1393,6 +1454,13 @@ static int timed_sequence(int n_events, float* h_ms, Fn fn) {
 using namespace dan;
 
 extern "C" {
+
+#ifdef DAN_PASS1_TIMELINE
+int dan_debug_pass1_timeline(unsigned long long* h_out, int32_t warps) {
+  if (warps < 0 || warps > kTimelineWarps) return DAN_ERR_INVALID_ARGUMENT;
+  return cudaMemcpyFromSymbol(h_out, g_p1_timeline, sizeof(unsigned long long) * 3 * warps) == cudaSuccess ? DAN_OK : -3;
+}
+#endif
 
 size_t dan_match_workspace_bytes(int32_t num_anchors, int32_t num_gt) {
   if (num_anchors < 0 || num_gt < 0) return 0;
@@ -1516,6 +1584,7 @@ static int encode_core(const dan_encode_params* p, const float* a_ymin, const fl
   A.match32 = out_match;
   bind_workspace(A, workspace, w);
   DAN_CUDA(cudaMemsetAsync(workspace, 0, w.zero_bytes, st));
+  int fine_end = 0;
   if (p->num_grids > 0) {
     // layout hint: levels of one anchor per cell, row major.  The tiles need whole warps and whole 8 x 4 blocks.
     DAN_REQUIRE(p->num_grids <= DAN_MAX_GRIDS, DAN_ERR_INVALID_ARGUMENT, "num_grids must be in [0, %d], got %d", DAN_MAX_GRIDS, p->num_grids);
@@ -1531,13 +1600,15 @@ static int encode_core(const dan_encode_params* p, const float* a_ymin, const fl
       H.start[g] = (int)gs; H.w[g] = (int)gw; H.h[g] = (int)gh;
       prev_end = gs + gw * gh;
     }
+    // the fine levels of pass 1: the hinted grids of at least kFineMinCells cells from anchor 0 on
+    for (int g = 0; g < H.n && H.start[g] == fine_end && H.w[g] * H.h[g] >= kFineMinCells; ++g) fine_end += H.w[g] * H.h[g];
     int2* map = reinterpret_cast<int2*>(static_cast<char*>(workspace) + w.warp_map);
     const int nwarps = (num_anchors + 31) / 32;
     enc_warp_map_kernel<<<(nwarps + 255) / 256, 256, 0, st>>>(map, nwarps, H);
     DAN_LAUNCH_CHECK("enc_warp_map_kernel");
     A.warp_map = map;
   }
-  return run_passes<false>(A, mining, !mining && !A.gt_max_first, batch, st, ev);
+  return run_passes<false>(A, mining, !mining && !A.gt_max_first, batch, st, ev, fine_end / kFusedThreads);
 }
 
 int dan_encode_batch(const dan_encode_params* p, const float* a_ymin, const float* a_xmin, const float* a_ymax,
