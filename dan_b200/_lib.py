@@ -18,6 +18,11 @@ DAN_MAX_LAYERS = 16
 DAN_MAX_DEPTH_TOTAL = 128
 DAN_MATCH_DUAL = 0
 DAN_MATCH_MINING = 1
+# element types of the predictions of the *_typed entry points (results bit-identical to fp32 on the widened values)
+DAN_DTYPE_F32 = 0
+DAN_DTYPE_F16 = 1
+DAN_DTYPE_BF16 = 2
+PRED_DTYPES = {torch.float32: DAN_DTYPE_F32, torch.float16: DAN_DTYPE_F16, torch.bfloat16: DAN_DTYPE_BF16}
 
 c_i32 = ctypes.c_int32
 c_i64 = ctypes.c_int64
@@ -101,6 +106,8 @@ _SIGNATURES = {
                                                 c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp,
                                                 ctypes.POINTER(c_f32)]),
     "dan_decode_batch": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, ctypes.POINTER(c_f32), c_vp, c_vp]),
+    "dan_decode_batch_typed": (ctypes.c_int, [c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, ctypes.POINTER(c_f32), c_vp,
+                                              c_vp]),
     "dan_softmax": (ctypes.c_int, [c_vp, c_i64, c_i32, c_vp, c_vp]),
     "dan_select_bboxes": (ctypes.c_int, [c_vp, c_i32, c_i32, c_vp, c_i64, c_f32, c_vp, c_vp, c_vp]),
     "dan_clip_bboxes": (ctypes.c_int, [c_vp, c_i64, c_f32, c_f32, c_vp, c_vp]),
@@ -134,6 +141,9 @@ _SIGNATURES = {
     "dan_postprocess_batch_peers": (ctypes.c_int, [ctypes.POINTER(PostprocessParams), c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
                                                    c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_sz,
                                                    ctypes.POINTER(PeerExchangeArgs), c_vp]),
+    "dan_postprocess_batch_typed": (ctypes.c_int, [ctypes.POINTER(PostprocessParams), c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                                   c_vp, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_sz,
+                                                   ctypes.POINTER(PeerExchangeArgs), c_vp, ctypes.POINTER(c_f32)]),
     "dan_wait_detections": (ctypes.c_int, [c_vp, c_vp, c_i32, c_vp]),
     "dan_nccl_load": (ctypes.c_int, [ctypes.c_char_p]),
     "dan_nccl_version": (ctypes.c_int, []),
@@ -193,6 +203,19 @@ def dev_ptr(t, dtype=None, name="tensor", allow_pinned=False):
     if not t.is_contiguous():
         raise ValueError("%s must be contiguous" % name)
     return ctypes.c_void_p(t.data_ptr())
+
+
+def pred_dtype(t, name="pred"):
+    """DAN_DTYPE_* code of a prediction tensor (fp32, fp16 or bf16); TypeError for any other dtype."""
+    code = PRED_DTYPES.get(getattr(t, "dtype", None))
+    if code is None:
+        raise TypeError("%s must be float32, float16 or bfloat16, got %s" % (name, getattr(t, "dtype", type(t).__name__)))
+    return code
+
+
+def is_half_cuda(t):
+    """A CUDA tensor of fp16 / bf16 predictions, which the typed entry points take as they are."""
+    return isinstance(t, torch.Tensor) and t.is_cuda and t.dtype in (torch.float16, torch.bfloat16)
 
 
 def as_f32(t, device=None):

@@ -108,13 +108,15 @@ __global__ void __launch_bounds__(256) iou_matrix_kernel(const float* __restrict
 // ---------------------------------------------------------------------------
 // decode_anchors / batch_decode_anchors, anchor_manipulator.py:389-424
 // ---------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) decode_kernel(const float4* __restrict__ pred, const float* __restrict__ ay0,
+// T: element type of pred (float, __half, __nv_bfloat16), widened to fp32 at the load
+template <typename T>
+__global__ void __launch_bounds__(256) decode_kernel(const typename PredRow<T>::type* __restrict__ pred, const float* __restrict__ ay0,
                                                      const float* __restrict__ ax0, const float* __restrict__ ay1,
                                                      const float* __restrict__ ax1, int n, int64_t total, float ps0, float ps1,
                                                      float ps2, float ps3, float4* __restrict__ out) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     const int a = (int)(i % n);
-    out[i] = decode_box(pred[i], ay0[a], ax0[a], ay1[a], ax1[a], ps0, ps1, ps2, ps3);
+    out[i] = decode_box(PredRow<T>::widen(pred[i]), ay0[a], ax0[a], ay1[a], ax1[a], ps0, ps1, ps2, ps3);
   }
 }
 
@@ -192,6 +194,15 @@ __global__ void __launch_bounds__(256) convert_kernel(const float4* __restrict__
   }
 }
 
+template <typename T>
+static int decode_launch(const void* pred, const float* a_ymin, const float* a_xmin, const float* a_ymax, const float* a_xmax,
+                         int32_t num_anchors, int64_t total, const float* ps, float* out_boxes, cudaStream_t st) {
+  decode_kernel<T><<<grid_for(total), 256, 0, st>>>(static_cast<const typename PredRow<T>::type*>(pred), a_ymin, a_xmin, a_ymax, a_xmax,
+                                                    num_anchors, total, ps[0], ps[1], ps[2], ps[3], reinterpret_cast<float4*>(out_boxes));
+  DAN_LAUNCH_CHECK("decode_kernel");
+  return DAN_OK;
+}
+
 }  // namespace dan
 
 using namespace dan;
@@ -240,19 +251,30 @@ int dan_intersection_matrix(const float* a_ymin, const float* a_xmin, const floa
   return pairwise_matrix(1, a_ymin, a_xmin, a_ymax, a_xmax, nullptr, num_anchors, gt_boxes, num_gt, out_inter, stream);
 }
 
-int dan_decode_batch(const float* pred, const float* a_ymin, const float* a_xmin, const float* a_ymax, const float* a_xmax,
-                     int32_t num_anchors, int32_t batch, const float* h_prior_scaling, float* out_boxes, void* stream) {
+int dan_decode_batch_typed(int32_t pred_dtype, const void* pred, const float* a_ymin, const float* a_xmin, const float* a_ymax,
+                           const float* a_xmax, int32_t num_anchors, int32_t batch, const float* h_prior_scaling, float* out_boxes,
+                           void* stream) {
+  const int esize = dtype_bytes(pred_dtype);
+  DAN_REQUIRE(esize != 0, DAN_ERR_INVALID_ARGUMENT, "unknown pred_dtype %d", pred_dtype);
   DAN_REQUIRE(num_anchors >= 0 && batch >= 0, DAN_ERR_INVALID_ARGUMENT, "negative size");
   if (num_anchors == 0 || batch == 0) return DAN_OK;
   DAN_REQUIRE(pred && a_ymin && a_xmin && a_ymax && a_xmax && out_boxes && h_prior_scaling, DAN_ERR_INVALID_ARGUMENT, "NULL pointer");
-  DAN_REQUIRE(aligned16(pred) && aligned16(out_boxes), DAN_ERR_INVALID_ARGUMENT, "pred/out_boxes must be 16-byte aligned");
+  DAN_REQUIRE((reinterpret_cast<uintptr_t>(pred) & (uintptr_t)(4 * esize - 1)) == 0 && aligned16(out_boxes), DAN_ERR_INVALID_ARGUMENT,
+              "pred must be %d-byte aligned, out_boxes 16-byte aligned", 4 * esize);
   const int64_t total = (int64_t)num_anchors * batch;
-  decode_kernel<<<grid_for(total), 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const float4*>(pred), a_ymin, a_xmin, a_ymax, a_xmax,
-                                                                  num_anchors, total, h_prior_scaling[0], h_prior_scaling[1],
-                                                                  h_prior_scaling[2], h_prior_scaling[3],
-                                                                  reinterpret_cast<float4*>(out_boxes));
-  DAN_LAUNCH_CHECK("decode_kernel");
-  return DAN_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  switch (pred_dtype) {
+    case DAN_DTYPE_F16: return decode_launch<__half>(pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, total, h_prior_scaling, out_boxes, st);
+    case DAN_DTYPE_BF16:
+      return decode_launch<__nv_bfloat16>(pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, total, h_prior_scaling, out_boxes, st);
+    default: return decode_launch<float>(pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, total, h_prior_scaling, out_boxes, st);
+  }
+}
+
+int dan_decode_batch(const float* pred, const float* a_ymin, const float* a_xmin, const float* a_ymax, const float* a_xmax,
+                     int32_t num_anchors, int32_t batch, const float* h_prior_scaling, float* out_boxes, void* stream) {
+  return dan_decode_batch_typed(DAN_DTYPE_F32, pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling, out_boxes,
+                                stream);
 }
 
 int dan_softmax(const float* logits, int64_t rows, int32_t num_classes, float* out, void* stream) {

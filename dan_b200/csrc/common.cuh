@@ -7,6 +7,8 @@
 // contract into FMA (the build also passes -fmad=false as a second guard).
 #pragma once
 
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -174,6 +176,47 @@ DAN_D float4 decode_box(float4 p, float ay0, float ax0, float ay1, float ax1, fl
   float4 o;
   center2point(pcy, pcx, ph, pw, o.x, o.y, o.z, o.w);
   return o;
+}
+
+// prediction element types (DAN_DTYPE_*) ---------------------------------------
+// fp16 and bf16 predictions are widened to fp32 where they are loaded.  The widening is exact, so everything after the
+// load is the fp32 code and its results are those of the fp32 path on the widened inputs.
+static inline int dtype_bytes(int32_t dtype) {
+  return dtype == DAN_DTYPE_F32 ? 4 : (dtype == DAN_DTYPE_F16 || dtype == DAN_DTYPE_BF16) ? 2 : 0;
+}
+
+DAN_D float widen(float v) { return v; }
+DAN_D float widen(__half v) { return __half2float(v); }
+DAN_D float widen(__nv_bfloat16 v) { return __uint_as_float((uint32_t)__bfloat16_as_ushort(v) << 16); }
+
+// two packed 16-bit values (the lower one first in memory)
+template <typename T> DAN_D float2 widen2(uint32_t bits);
+template <> DAN_D float2 widen2<__half>(uint32_t bits) { return __half22float2(*reinterpret_cast<const __half2*>(&bits)); }
+template <> DAN_D float2 widen2<__nv_bfloat16>(uint32_t bits) {
+  return make_float2(__uint_as_float(bits << 16), __uint_as_float(bits & 0xffff0000u));
+}
+
+// one anchor's four box values: a 16-byte row (fp32) or an 8-byte row (fp16 / bf16)
+template <typename T> struct PredRow {
+  typedef uint2 type;
+  DAN_D static float4 widen(uint2 r) {
+    const float2 lo = widen2<T>(r.x), hi = widen2<T>(r.y);
+    return make_float4(lo.x, lo.y, hi.x, hi.y);
+  }
+};
+template <> struct PredRow<float> {
+  typedef float4 type;
+  DAN_D static float4 widen(float4 r) { return r; }
+};
+
+// the two logits of one anchor (two classes); x must be aligned to 2 * sizeof(T)
+DAN_D float2 ld_pair(const float* x) { return *reinterpret_cast<const float2*>(x); }
+template <typename T> DAN_D float2 ld_pair(const T* x) { return widen2<T>(*reinterpret_cast<const uint32_t*>(x)); }
+
+// logit pair j of a 16-byte vector of four fp16 / bf16 anchors
+template <typename T> DAN_D float2 vec_pair(const float4& q, int j) {
+  const float w = j == 0 ? q.x : j == 1 ? q.y : j == 2 ? q.z : q.w;
+  return widen2<T>(__float_as_uint(w));
 }
 
 // warp helpers ---------------------------------------------------------------

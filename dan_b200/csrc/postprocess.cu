@@ -40,9 +40,10 @@ __device__ long long g_phase[32];
 
 struct PpArgs {
   // inputs
-  const float* cls;       // [B, N, C] logits
-  const float4* loc;      // [B, N, 4] offsets (or NULL)
-  const float4* boxes;    // [B, N, 4] decoded boxes (or NULL)
+  // inputs of element type T (float, __half or __nv_bfloat16: the T of the kernel templates)
+  const void* cls;        // [B, N, C] logits
+  const void* loc;        // [B, N, 4] offsets (or NULL)
+  const void* boxes;      // [B, N, 4] decoded boxes (or NULL)
   const float* ay0;
   const float* ax0;
   const float* ay1;
@@ -110,14 +111,16 @@ struct RawBox {
   float4 anchor;   // ymin, xmin, ymax, xmax (only when decoding)
 };
 
+template <typename T>
 DAN_D RawBox pp_load(const PpArgs& A, int b, int a) {
+  typedef typename PredRow<T>::type Row;
   const int64_t row = (int64_t)b * A.n + a;
   RawBox r;
   if (A.loc != nullptr) {
-    r.v = A.loc[row];
+    r.v = PredRow<T>::widen(static_cast<const Row*>(A.loc)[row]);
     r.anchor = make_float4(A.ay0[a], A.ax0[a], A.ay1[a], A.ax1[a]);
   } else {
-    r.v = A.boxes[row];
+    r.v = PredRow<T>::widen(static_cast<const Row*>(A.boxes)[row]);
     r.anchor = make_float4(0.f, 0.f, 0.f, 0.f);
   }
   return r;
@@ -129,7 +132,8 @@ DAN_D float4 pp_finish(const PpArgs& A, const RawBox& r) {
   return pp_clip(bx, A.img_h, A.img_w);
 }
 
-DAN_D float4 pp_box(const PpArgs& A, int b, int a) { return pp_finish(A, pp_load(A, b, a)); }
+template <typename T>
+DAN_D float4 pp_box(const PpArgs& A, int b, int a) { return pp_finish(A, pp_load<T>(A, b, a)); }
 
 // ---------------------------------------------------------------------------
 // K3: filter + compaction.  grid (ceil(N/256), B)
@@ -139,18 +143,18 @@ constexpr int kFilterPerThread = 4;     // anchors per thread: 4 independent log
 // exact per-anchor path: softmax, threshold, decode + clip, min-size, warp-aggregated append of the survivors.
 // STAGED (two classes = one list per image): the keys are collected in the CTA's shared memory and appended to the list
 // with ONE global atomic per CTA; per-warp atomics on the same counter serialise in L2 (ncu: 20 % of the stall samples).
-template <bool STAGED>
+template <bool STAGED, typename T>
 DAN_D void filter_one(const PpArgs& A, int b, int a, bool live, int lane, unsigned long long* s_keys, int* s_cnt) {
   const int C = A.num_classes;
-  const float* x = A.cls + ((int64_t)b * A.n + (live ? a : 0)) * C;
+  const T* x = static_cast<const T*>(A.cls) + ((int64_t)b * A.n + (live ? a : 0)) * C;
   // tf.nn.softmax: exp(x - max) * (1 / sum(exp(x - max))), sum in class order
   float mx = 0.f, inv = 0.f;
   if (live) {
-    mx = x[0];
-    for (int k = 1; k < C; ++k) mx = fmaxf(mx, x[k]);
+    mx = widen(x[0]);
+    for (int k = 1; k < C; ++k) mx = fmaxf(mx, widen(x[k]));
     float s = 0.f;
     for (int k = 0; k < C; ++k) {
-      const float e = cephes_expf(fsub(x[k], mx));
+      const float e = cephes_expf(fsub(widen(x[k]), mx));
       s = (k == 0) ? e : fadd(s, e);
     }
     inv = fdiv(1.f, s);
@@ -161,10 +165,10 @@ DAN_D void filter_one(const PpArgs& A, int b, int a, bool live, int lane, unsign
     bool pass = false;
     float p = 0.f;
     if (live) {
-      p = fmul(cephes_expf(fsub(x[c], mx)), inv);
+      p = fmul(cephes_expf(fsub(widen(x[c]), mx)), inv);
       if (p > A.select_thr) {                       // select_bboxes :24-36
         if (!have_box) {
-          box = pp_box(A, b, a);
+          box = pp_box<T>(A, b, a);
           have_box = true;
           if (A.stash != nullptr) A.stash[(int64_t)b * A.n + a] = box;
         }
@@ -189,6 +193,7 @@ DAN_D void filter_one(const PpArgs& A, int b, int a, bool live, int lane, unsign
   }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(256) pp_filter_kernel(const PpArgs A) {
   __shared__ unsigned long long s_keys[256 * kFilterPerThread];
   __shared__ int s_cnt, s_base;
@@ -201,13 +206,16 @@ __global__ void __launch_bounds__(256) pp_filter_kernel(const PpArgs A) {
   // Two classes: softmax_1 = sigmoid(x1 - x0).  An anchor whose logit difference is more than 0.05 below
   // logit(threshold) cannot pass (the fp32 evaluation is accurate to ~1e-6 relative), so the ~98 % background anchors
   // leave after one subtraction.  The exact path runs per 32-anchor group when any of its lanes may pass.
+  // Two classes come here only when cls_pred is not aligned to an anchor's pair of logits (the NMS kernel filters
+  // aligned ones itself), so the pair is read as two scalars.
   bool maybe[kFilterPerThread];
   if (A.num_classes == 2) {
     float2 xx[kFilterPerThread];
 #pragma unroll
     for (int u = 0; u < kFilterPerThread; ++u) {
       const int a = a0 + u * 256;
-      xx[u] = (a < A.n) ? __ldcs(reinterpret_cast<const float2*>(A.cls + ((int64_t)b * A.n + a) * 2)) : make_float2(0.f, 0.f);   // read once: streaming
+      const T* x = static_cast<const T*>(A.cls) + ((int64_t)b * A.n + (a < A.n ? a : 0)) * 2;
+      xx[u] = (a < A.n) ? make_float2(widen(__ldcs(x)), widen(__ldcs(x + 1))) : make_float2(0.f, 0.f);   // read once: streaming
     }
 #pragma unroll
     for (int u = 0; u < kFilterPerThread; ++u)
@@ -231,8 +239,8 @@ __global__ void __launch_bounds__(256) pp_filter_kernel(const PpArgs A) {
   __syncwarp();
   for (int j = 0; j < total; j += 32) {
     const bool live = j + lane < total;
-    if (staged) filter_one<true>(A, b, live ? mylist[j + lane] : 0, live, lane, s_keys, &s_cnt);
-    else filter_one<false>(A, b, live ? mylist[j + lane] : 0, live, lane, s_keys, &s_cnt);
+    if (staged) filter_one<true, T>(A, b, live ? mylist[j + lane] : 0, live, lane, s_keys, &s_cnt);
+    else filter_one<false, T>(A, b, live ? mylist[j + lane] : 0, live, lane, s_keys, &s_cnt);
   }
   if (staged) {
     __syncthreads();
@@ -498,7 +506,8 @@ __device__ __noinline__ void resolve_chunk_serially(const uint32_t* T, uint32_t*
 #endif
 constexpr int kMaybeCap = 4096;                        // indices kept in shared memory (the rest goes to the workspace)
 
-template <bool DECODE, int WHERE, bool FILTER>
+// T: element type of the predictions (DECODE only; the standalone sort / NMS instantiations take fp32 scores and boxes)
+template <bool DECODE, int WHERE, bool FILTER, typename T>
 __global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __restrict__ src_scores,
                                                                      const float4* __restrict__ src_boxes) {
   extern __shared__ __align__(16) unsigned char dyn_smem[];
@@ -579,10 +588,15 @@ __global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __
       else gmaybe[pos] = a;
     };
     auto push = [&](int a) { put(atomicAdd(&s_nmaybe, 1), a); };
-    // the image's logits as 16-byte vectors (two anchors); the row of an image starts 8-byte aligned only
-    const float* x = A.cls + (int64_t)b * A.n * 2;
-    const int head = (reinterpret_cast<uintptr_t>(x) & 15u) ? 1 : 0;
-    const int nvec = (A.n - head) >> 1;
+    // The image's logits as 16-byte vectors of kVA anchors (2 for fp32, 4 for fp16 / bf16).  The row of an image starts
+    // aligned to one anchor only (8 or 4 bytes): the `head` anchors before the first 16-byte boundary and the ones behind
+    // the last whole vector are read as pairs after the loop.
+    constexpr int kVA = 16 / (2 * (int)sizeof(T));
+    const T* x = static_cast<const T*>(A.cls) + (int64_t)b * A.n * 2;
+    // (fp32 keeps the statements it had before fp16 / bf16 were added, so that it compiles to the same instructions)
+    const int head = kVA == 2 ? ((reinterpret_cast<uintptr_t>(x) & 15u) ? 1 : 0)
+                              : min((int)(((16u - (unsigned)(reinterpret_cast<uintptr_t>(x) & 15u)) & 15u) / (2 * sizeof(T))), A.n);
+    const int nvec = kVA == 2 ? (A.n - head) >> 1 : (int)((unsigned)(A.n - head) / kVA);
     const float4* xv = reinterpret_cast<const float4*>(x + 2 * head);
     for (int v0 = 0; v0 < nvec; v0 += 4 * kSortThreads) {
       float4 q[4];
@@ -593,39 +607,83 @@ __global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __
       }
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
-        // A warp looks at 64 consecutive anchors here.  Its survivors enter the list in ANCHOR order with one atomic per
-        // warp: the exact pass below then reads neighbouring box rows from neighbouring lanes, i.e. whole sectors - which
-        // matters when the rows live in host memory and every sector is a PCIe read.
+        // A warp looks at 32 * kVA consecutive anchors here.  Its survivors enter the list in ANCHOR order with one atomic
+        // per warp: the exact pass below then reads neighbouring box rows from neighbouring lanes, i.e. whole sectors -
+        // which matters when the rows live in host memory and every sector is a PCIe read.
         const int v = v0 + u * kSortThreads + tid;
-        const bool p0 = v < nvec && f2_maybe(A, q[u].x, q[u].y);
-        const bool p1 = v < nvec && f2_maybe(A, q[u].z, q[u].w);
-        const unsigned m0 = __ballot_sync(0xffffffffu, p0), m1 = __ballot_sync(0xffffffffu, p1);
-        if ((m0 | m1) != 0u) {
-          int base = 0;
-          if (lane == 0) base = atomicAdd(&s_nmaybe, __popc(m0) + __popc(m1));
-          base = __shfl_sync(0xffffffffu, base, 0);
-          int pos = base + __popc(m0 & lt_mask) + __popc(m1 & lt_mask);
-          if (p0) put(pos++, head + 2 * v);
-          if (p1) put(pos, head + 2 * v + 1);
+        if constexpr (kVA == 2) {
+          const bool p0 = v < nvec && f2_maybe(A, q[u].x, q[u].y);
+          const bool p1 = v < nvec && f2_maybe(A, q[u].z, q[u].w);
+          const unsigned m0 = __ballot_sync(0xffffffffu, p0), m1 = __ballot_sync(0xffffffffu, p1);
+          if ((m0 | m1) != 0u) {
+            int base = 0;
+            if (lane == 0) base = atomicAdd(&s_nmaybe, __popc(m0) + __popc(m1));
+            base = __shfl_sync(0xffffffffu, base, 0);
+            int pos = base + __popc(m0 & lt_mask) + __popc(m1 & lt_mask);
+            if (p0) put(pos++, head + 2 * v);
+            if (p1) put(pos, head + 2 * v + 1);
+          }
+        } else {
+          bool pj[kVA];
+          unsigned mj[kVA], any = 0u;
+#pragma unroll
+          for (int j = 0; j < kVA; ++j) {
+            const float2 xx = vec_pair<T>(q[u], j);
+            pj[j] = v < nvec && f2_maybe(A, xx.x, xx.y);
+          }
+#pragma unroll
+          for (int j = 0; j < kVA; ++j) {
+            mj[j] = __ballot_sync(0xffffffffu, pj[j]);
+            any |= mj[j];
+          }
+          if (any != 0u) {
+            int nj = 0, below = 0;
+#pragma unroll
+            for (int j = 0; j < kVA; ++j) {
+              nj += __popc(mj[j]);
+              below += __popc(mj[j] & lt_mask);
+            }
+            int base = 0;
+            if (lane == 0) base = atomicAdd(&s_nmaybe, nj);
+            base = __shfl_sync(0xffffffffu, base, 0);
+            int pos = base + below;
+#pragma unroll
+            for (int j = 0; j < kVA; ++j)
+              if (pj[j]) put(pos++, head + kVA * v + j);
+          }
         }
       }
     }
-    if (tid == 0 && head == 1 && f2_maybe(A, x[0], x[1])) push(0);
-    if (tid == 1 && head + 2 * nvec < A.n && f2_maybe(A, x[2 * (A.n - 1)], x[2 * (A.n - 1) + 1])) push(A.n - 1);
+    if constexpr (kVA == 2) {                          // fp32: at most one anchor on either side
+      if (tid == 0 && head == 1 && f2_maybe(A, x[0], x[1])) push(0);
+      if (tid == 1 && head + 2 * nvec < A.n && f2_maybe(A, x[2 * (A.n - 1)], x[2 * (A.n - 1) + 1])) push(A.n - 1);
+    } else {
+      // head: threads [0, head); tail (fewer than kVA anchors behind the vectors): threads [kVA - 1, 2 kVA - 1)
+      const int rest = head + kVA * nvec;
+      const int t = tid - (kVA - 1);
+      if (tid < head) {
+        const float2 xx = make_float2(widen(x[2 * tid]), widen(x[2 * tid + 1]));
+        if (f2_maybe(A, xx.x, xx.y)) push(tid);
+      }
+      if (t >= 0 && rest + t < A.n) {
+        const float2 xx = make_float2(widen(x[2 * (rest + t)]), widen(x[2 * (rest + t) + 1]));
+        if (f2_maybe(A, xx.x, xx.y)) push(rest + t);
+      }
+    }
     __syncthreads();
     const int nmaybe = s_nmaybe;
     for (int i0 = 0; i0 < nmaybe; i0 += kSortThreads) {
       const int i = i0 + tid;
       if (i < nmaybe) {
         const int a = (i < kMaybeCap) ? s_maybe[i] : gmaybe[i];
-        const float2 xx = *reinterpret_cast<const float2*>(x + 2 * a);
+        const float2 xx = ld_pair(x + 2 * a);
         // tf.nn.softmax: exp(x - max) * (1 / sum(exp(x - max))), sum in class order
         const float mx = fmaxf(xx.x, xx.y);
         const float e0 = cephes_expf(fsub(xx.x, mx));
         const float e1 = cephes_expf(fsub(xx.y, mx));
         const float pr = fmul(e1, fdiv(1.f, fadd(e0, e1)));
         if (pr > A.select_thr) {                            // select_bboxes :24-36
-          const float4 box = pp_box(A, b, a);
+          const float4 box = pp_box<T>(A, b, a);
           if (A.stash != nullptr) A.stash[(int64_t)b * A.n + a] = box;
           const float w = fadd(fsub(box.w, box.y), 1.f);    // filter_bboxes :50-59
           const float h = fadd(fsub(box.z, box.x), 1.f);
@@ -675,7 +733,7 @@ __global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __
     __syncthreads();
     if (r < K) {
       const uint32_t idx = key_index(key);
-      const NmsBox nb = nms_norm(DECODE ? (A.stash != nullptr ? A.stash[(int64_t)b * A.n + idx] : pp_box(A, b, (int)idx)) : src_boxes[idx]);
+      const NmsBox nb = nms_norm(DECODE ? (A.stash != nullptr ? A.stash[(int64_t)b * A.n + idx] : pp_box<T>(A, b, (int)idx)) : src_boxes[idx]);
       cbox[r] = make_float4(nb.y0, nb.x0, nb.y1, nb.x1);
       carea[r] = nb.area;
     }
@@ -880,12 +938,12 @@ __global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __
     // d. relaxation: thread v owns survivor v (the first kSurv threads)
     int sweeps = 0;
     if (tid < kSurv) {
-      uint32_t T[kSurvWords];
+      uint32_t trow[kSurvWords];
       const int vw = tid >> 5;
       const uint32_t vbit = 1u << (tid & 31);
       const bool mine = tid < ns;
 #pragma unroll
-      for (int w = 0; w < kSurvWords; ++w) T[w] = (mine && (w << 5) < tid) ? s_T[tid][w] : 0u;
+      for (int w = 0; w < kSurvWords; ++w) trow[w] = (mine && (w << 5) < tid) ? s_T[tid][w] : 0u;
       bool decided = !mine;
       bool open = true;
       while (open && sweeps < kMaxSweeps) {
@@ -894,8 +952,8 @@ __global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __
 #pragma unroll
           for (int w = 0; w < kSurvWords; ++w) {
             const uint32_t kw = s_keptm[w], sw = s_supm[w];
-            hitm |= T[w] & kw;
-            pendm |= T[w] & ~(kw | sw);
+            hitm |= trow[w] & kw;
+            pendm |= trow[w] & ~(kw | sw);
           }
         }
         bar_sync_chunk();                              // every thread has read the masks of the previous sweep
@@ -1087,16 +1145,16 @@ static void pp_bind(PpArgs& A, void* ws, const PpLayout& w) {
 
 // opt-in to > 48 KB of dynamic shared memory; the attribute belongs to the (function, device) pair, so it is set on
 // every call (a few hundred ns of host time) rather than cached in a process-wide flag
-template <bool DECODE, int WHERE, bool FILTER>
+template <bool DECODE, int WHERE, bool FILTER, typename T>
 static int launch_greedy(const PpArgs& A, int lists, size_t smem, const float* src_scores, const float4* src_boxes, cudaStream_t st) {
-  DAN_CUDA(cudaFuncSetAttribute(nms_greedy_kernel<DECODE, WHERE, FILTER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  nms_greedy_kernel<DECODE, WHERE, FILTER><<<lists, kSortThreads, smem, st>>>(A, src_scores, src_boxes);
+  DAN_CUDA(cudaFuncSetAttribute(nms_greedy_kernel<DECODE, WHERE, FILTER, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  nms_greedy_kernel<DECODE, WHERE, FILTER, T><<<lists, kSortThreads, smem, st>>>(A, src_scores, src_boxes);
   DAN_LAUNCH_CHECK("nms_greedy_kernel");
   return DAN_OK;
 }
 
 // [filter +] sort + greedy NMS for `lists` lists
-template <bool DECODE, bool FILTER>
+template <bool DECODE, bool FILTER, typename T>
 static int run_sort_nms(const PpArgs& A_in, int lists, const float* src_scores, const float4* src_boxes, cudaStream_t st) {
   PpArgs A = A_in;
   const GreedyPlan g = greedy_plan(A.n, A.keep_topk, A.nms_cap);
@@ -1107,9 +1165,26 @@ static int run_sort_nms(const PpArgs& A_in, int lists, const float* src_scores, 
   A.dyn_smem_bytes = (int)g.smem;
   A.cand_global = g.cand_global;
   A.kept_global = g.kept_global;
-  if (g.kept_global) return launch_greedy<DECODE, 2, FILTER>(A, lists, g.smem, src_scores, src_boxes, st);
-  if (g.cand_global) return launch_greedy<DECODE, 1, FILTER>(A, lists, g.smem, src_scores, src_boxes, st);
-  return launch_greedy<DECODE, 0, FILTER>(A, lists, g.smem, src_scores, src_boxes, st);
+  if (g.kept_global) return launch_greedy<DECODE, 2, FILTER, T>(A, lists, g.smem, src_scores, src_boxes, st);
+  if (g.cand_global) return launch_greedy<DECODE, 1, FILTER, T>(A, lists, g.smem, src_scores, src_boxes, st);
+  return launch_greedy<DECODE, 0, FILTER, T>(A, lists, g.smem, src_scores, src_boxes, st);
+}
+
+// the launches of one postprocess call: [filter kernel +] the per-list NMS kernel, with T the prediction type
+template <typename T>
+static int postprocess_launch(const PpArgs& A, bool fused, int lists, cudaStream_t st, cudaEvent_t* ev) {
+  if (ev) DAN_CUDA(cudaEventRecord(ev[0], st));
+  if (!fused) {
+    DAN_CUDA(cudaMemsetAsync(A.key_count, 0, (size_t)lists * 4, st));
+    if (A.n > 0) {
+      pp_filter_kernel<T><<<dim3((A.n + 256 * kFilterPerThread - 1) / (256 * kFilterPerThread), A.batch), 256, 0, st>>>(A);
+      DAN_LAUNCH_CHECK("pp_filter_kernel");
+    }
+  }
+  if (ev) DAN_CUDA(cudaEventRecord(ev[1], st));
+  int rc = fused ? run_sort_nms<true, true, T>(A, lists, nullptr, nullptr, st) : run_sort_nms<true, false, T>(A, lists, nullptr, nullptr, st);
+  if (ev && rc == DAN_OK) DAN_CUDA(cudaEventRecord(ev[2], st));
+  return rc;
 }
 
 }  // namespace dan
@@ -1137,11 +1212,13 @@ size_t dan_nms_workspace_bytes(int64_t n, int32_t nms_topk) {
   return pp_layout(n, 1, n > 0 ? n : 1, true).total;
 }
 
-static int postprocess_core(const dan_postprocess_params* p, const float* cls_pred, const float* loc_pred, const float* boxes_pred,
-                            const float* a_ymin, const float* a_xmin, const float* a_ymax, const float* a_xmax, int32_t num_anchors,
-                            int32_t batch, float* out_boxes, float* out_scores, int32_t* out_counts, int32_t* out_anchor_index,
-                            int32_t* out_keep_pos, void* workspace, size_t workspace_bytes, void* stream, cudaEvent_t* ev,
-                            const dan_peer_exchange* peers = nullptr) {
+// pred_dtype has been checked by the caller
+static int postprocess_core(const dan_postprocess_params* p, int32_t pred_dtype, const void* cls_pred, const void* loc_pred,
+                            const void* boxes_pred, const float* a_ymin, const float* a_xmin, const float* a_ymax, const float* a_xmax,
+                            int32_t num_anchors, int32_t batch, float* out_boxes, float* out_scores, int32_t* out_counts,
+                            int32_t* out_anchor_index, int32_t* out_keep_pos, void* workspace, size_t workspace_bytes, void* stream,
+                            cudaEvent_t* ev, const dan_peer_exchange* peers) {
+  const int esize = dtype_bytes(pred_dtype);
   DAN_REQUIRE(p != nullptr, DAN_ERR_INVALID_ARGUMENT, "params is NULL");
   DAN_REQUIRE(p->num_classes >= 2, DAN_ERR_INVALID_ARGUMENT, "num_classes must be >= 2 (class 0 is background), got %d", p->num_classes);
   DAN_REQUIRE(num_anchors >= 0 && batch >= 0, DAN_ERR_INVALID_ARGUMENT, "negative size");
@@ -1153,7 +1230,12 @@ static int postprocess_core(const dan_postprocess_params* p, const float* cls_pr
   if (batch == 0) return DAN_OK;
   DAN_REQUIRE(cls_pred && out_boxes && out_scores, DAN_ERR_INVALID_ARGUMENT, "NULL pointer");
   DAN_REQUIRE(loc_pred == nullptr || (a_ymin && a_xmin && a_ymax && a_xmax), DAN_ERR_INVALID_ARGUMENT, "anchors needed to decode loc_pred");
-  DAN_REQUIRE(aligned16(loc_pred) && aligned16(boxes_pred) && aligned16(out_boxes), DAN_ERR_INVALID_ARGUMENT, "box tensors must be 16-byte aligned");
+  DAN_REQUIRE(aligned16(out_boxes), DAN_ERR_INVALID_ARGUMENT, "out_boxes must be 16-byte aligned");
+  {
+    const uintptr_t row_mask = (uintptr_t)(4 * esize - 1);      // one row of 4 values per anchor: 16 (fp32) or 8 bytes
+    DAN_REQUIRE(((reinterpret_cast<uintptr_t>(loc_pred) | reinterpret_cast<uintptr_t>(boxes_pred)) & row_mask) == 0,
+                DAN_ERR_INVALID_ARGUMENT, "loc_pred / boxes_pred must be %d-byte aligned", 4 * esize);
+  }
   const int lists = batch * (p->num_classes - 1);
   const PpLayout w = pp_layout(num_anchors, lists, p->keep_topk, true, (int64_t)batch * num_anchors);
   DAN_REQUIRE(workspace != nullptr && workspace_bytes >= w.total, DAN_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", w.total,
@@ -1161,8 +1243,8 @@ static int postprocess_core(const dan_postprocess_params* p, const float* cls_pr
   cudaStream_t st = (cudaStream_t)stream;
   PpArgs A = {};
   A.cls = cls_pred;
-  A.loc = reinterpret_cast<const float4*>(loc_pred);
-  A.boxes = reinterpret_cast<const float4*>(boxes_pred);
+  A.loc = loc_pred;
+  A.boxes = boxes_pred;
   A.ay0 = a_ymin; A.ax0 = a_xmin; A.ay1 = a_ymax; A.ax1 = a_xmax;
   A.n = num_anchors;
   A.batch = batch;
@@ -1203,34 +1285,59 @@ static int postprocess_core(const dan_postprocess_params* p, const float* cls_pr
   // the kernels read only the rows of the anchors that pass the score threshold (~3 %), straight over PCIe, and keep
   // the decoded box of such a row in the workspace so that the row is fetched once.  Pageable memory is refused.
   {
-    const void* geo = loc_pred != nullptr ? static_cast<const void*>(loc_pred) : static_cast<const void*>(boxes_pred);
+    const void* geo = loc_pred != nullptr ? loc_pred : boxes_pred;
     cudaPointerAttributes pa;
     const cudaError_t e = cudaPointerGetAttributes(&pa, geo);
     if (e != cudaSuccess) {
       (void)cudaGetLastError();
     } else if (pa.type == cudaMemoryTypeHost) {
       DAN_REQUIRE(pa.devicePointer != nullptr, DAN_ERR_INVALID_ARGUMENT, "loc_pred / boxes_pred: host memory that is not mapped for the device");
-      if (loc_pred != nullptr) A.loc = reinterpret_cast<const float4*>(pa.devicePointer);
-      else A.boxes = reinterpret_cast<const float4*>(pa.devicePointer);
+      if (loc_pred != nullptr) A.loc = pa.devicePointer;
+      else A.boxes = pa.devicePointer;
       A.stash = reinterpret_cast<float4*>(static_cast<char*>(workspace) + w.stash);
     } else {
       DAN_REQUIRE(pa.type != cudaMemoryTypeUnregistered, DAN_ERR_INVALID_ARGUMENT,
                   "loc_pred / boxes_pred is pageable host memory: pass device memory or page-locked (pinned) host memory");
     }
   }
-  // two classes: the NMS kernel filters its own image (one launch for the whole evaluation side)
-  const bool fused = p->num_classes == 2 && (reinterpret_cast<uintptr_t>(cls_pred) & 7u) == 0;
-  if (ev) DAN_CUDA(cudaEventRecord(ev[0], st));
-  if (!fused) {
-    DAN_CUDA(cudaMemsetAsync(A.key_count, 0, (size_t)lists * 4, st));
-    if (num_anchors > 0) {
-      pp_filter_kernel<<<dim3((num_anchors + 256 * kFilterPerThread - 1) / (256 * kFilterPerThread), batch), 256, 0, st>>>(A);
-      DAN_LAUNCH_CHECK("pp_filter_kernel");
-    }
+  // two classes: the NMS kernel filters its own image (one launch for the whole evaluation side) when every anchor's pair
+  // of logits is aligned for one load
+  const bool fused = p->num_classes == 2 && (reinterpret_cast<uintptr_t>(cls_pred) & (uintptr_t)(2 * esize - 1)) == 0;
+  switch (pred_dtype) {
+    case DAN_DTYPE_F16: return postprocess_launch<__half>(A, fused, lists, st, ev);
+    case DAN_DTYPE_BF16: return postprocess_launch<__nv_bfloat16>(A, fused, lists, st, ev);
+    default: return postprocess_launch<float>(A, fused, lists, st, ev);
   }
-  if (ev) DAN_CUDA(cudaEventRecord(ev[1], st));
-  int rc = fused ? run_sort_nms<true, true>(A, lists, nullptr, nullptr, st) : run_sort_nms<true, false>(A, lists, nullptr, nullptr, st);
-  if (ev && rc == DAN_OK) DAN_CUDA(cudaEventRecord(ev[2], st));
+}
+
+int dan_postprocess_batch_typed(const dan_postprocess_params* p, int32_t pred_dtype, const void* cls_pred, const void* loc_pred,
+                                const void* boxes_pred, const float* a_ymin, const float* a_xmin, const float* a_ymax,
+                                const float* a_xmax, int32_t num_anchors, int32_t batch, float* out_boxes, float* out_scores,
+                                int32_t* out_counts, int32_t* out_anchor_index, int32_t* out_keep_pos, void* workspace,
+                                size_t workspace_bytes, const dan_peer_exchange* peers, void* stream, float* h_kernel_ms) {
+  DAN_REQUIRE(dtype_bytes(pred_dtype) != 0, DAN_ERR_INVALID_ARGUMENT, "unknown pred_dtype %d", pred_dtype);
+  DAN_REQUIRE(peers == nullptr || h_kernel_ms == nullptr, DAN_ERR_INVALID_ARGUMENT,
+              "h_peers and h_kernel_ms: the profiling call does not take part in a peer exchange");
+  if (h_kernel_ms == nullptr) {
+    DAN_REQUIRE(batch > 0 || peers == nullptr || peers->num_destinations == 0, DAN_ERR_INVALID_ARGUMENT,
+                "a rank without images cannot take part in the peer exchange (its flag would never rise)");
+    return postprocess_core(p, pred_dtype, cls_pred, loc_pred, boxes_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch,
+                            out_boxes, out_scores, out_counts, out_anchor_index, out_keep_pos, workspace, workspace_bytes, stream,
+                            nullptr, peers);
+  }
+  // profiling: events around the two launches, then wait for them
+  h_kernel_ms[0] = h_kernel_ms[1] = 0.f;
+  cudaEvent_t ev[3];
+  for (int i = 0; i < 3; ++i) DAN_CUDA(cudaEventCreate(&ev[i]));
+  int rc = postprocess_core(p, pred_dtype, cls_pred, loc_pred, boxes_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch,
+                            out_boxes, out_scores, out_counts, out_anchor_index, out_keep_pos, workspace, workspace_bytes, stream, ev,
+                            nullptr);
+  if (rc == DAN_OK && batch > 0) {
+    cudaError_t e = cudaEventSynchronize(ev[2]);
+    if (e != cudaSuccess) rc = cuda_fail(e, "cudaEventSynchronize");
+    else for (int i = 0; i < 2; ++i) cudaEventElapsedTime(&h_kernel_ms[i], ev[i], ev[i + 1]);
+  }
+  for (int i = 0; i < 3; ++i) cudaEventDestroy(ev[i]);
   return rc;
 }
 
@@ -1238,8 +1345,9 @@ int dan_postprocess_batch(const dan_postprocess_params* p, const float* cls_pred
                           const float* a_ymin, const float* a_xmin, const float* a_ymax, const float* a_xmax, int32_t num_anchors,
                           int32_t batch, float* out_boxes, float* out_scores, int32_t* out_counts, int32_t* out_anchor_index,
                           int32_t* out_keep_pos, void* workspace, size_t workspace_bytes, void* stream) {
-  return postprocess_core(p, cls_pred, loc_pred, boxes_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, out_boxes, out_scores,
-                          out_counts, out_anchor_index, out_keep_pos, workspace, workspace_bytes, stream, nullptr);
+  return dan_postprocess_batch_typed(p, DAN_DTYPE_F32, cls_pred, loc_pred, boxes_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors,
+                                     batch, out_boxes, out_scores, out_counts, out_anchor_index, out_keep_pos, workspace,
+                                     workspace_bytes, nullptr, stream, nullptr);
 }
 
 int dan_postprocess_batch_peers(const dan_postprocess_params* p, const float* cls_pred, const float* loc_pred, const float* boxes_pred,
@@ -1247,10 +1355,9 @@ int dan_postprocess_batch_peers(const dan_postprocess_params* p, const float* cl
                                 int32_t batch, float* out_boxes, float* out_scores, int32_t* out_counts, int32_t* out_anchor_index,
                                 int32_t* out_keep_pos, void* workspace, size_t workspace_bytes, const dan_peer_exchange* peers,
                                 void* stream) {
-  DAN_REQUIRE(batch > 0 || peers == nullptr || peers->num_destinations == 0, DAN_ERR_INVALID_ARGUMENT,
-              "a rank without images cannot take part in the peer exchange (its flag would never rise)");
-  return postprocess_core(p, cls_pred, loc_pred, boxes_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, out_boxes, out_scores,
-                          out_counts, out_anchor_index, out_keep_pos, workspace, workspace_bytes, stream, nullptr, peers);
+  return dan_postprocess_batch_typed(p, DAN_DTYPE_F32, cls_pred, loc_pred, boxes_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors,
+                                     batch, out_boxes, out_scores, out_counts, out_anchor_index, out_keep_pos, workspace,
+                                     workspace_bytes, peers, stream, nullptr);
 }
 
 int dan_wait_detections(const int32_t* flags, const int32_t* state, int32_t world_size, void* stream) {
@@ -1301,18 +1408,9 @@ int dan_postprocess_batch_profile(const dan_postprocess_params* p, const float* 
                                   int32_t* out_counts, int32_t* out_anchor_index, int32_t* out_keep_pos, void* workspace,
                                   size_t workspace_bytes, void* stream, float* h_kernel_ms) {
   DAN_REQUIRE(h_kernel_ms != nullptr, DAN_ERR_INVALID_ARGUMENT, "h_kernel_ms is NULL");
-  h_kernel_ms[0] = h_kernel_ms[1] = 0.f;
-  cudaEvent_t ev[3];
-  for (int i = 0; i < 3; ++i) DAN_CUDA(cudaEventCreate(&ev[i]));
-  int rc = postprocess_core(p, cls_pred, loc_pred, boxes_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, out_boxes,
-                            out_scores, out_counts, out_anchor_index, out_keep_pos, workspace, workspace_bytes, stream, ev);
-  if (rc == DAN_OK && batch > 0) {
-    cudaError_t e = cudaEventSynchronize(ev[2]);
-    if (e != cudaSuccess) rc = cuda_fail(e, "cudaEventSynchronize");
-    else for (int i = 0; i < 2; ++i) cudaEventElapsedTime(&h_kernel_ms[i], ev[i], ev[i + 1]);
-  }
-  for (int i = 0; i < 3; ++i) cudaEventDestroy(ev[i]);
-  return rc;
+  return dan_postprocess_batch_typed(p, DAN_DTYPE_F32, cls_pred, loc_pred, boxes_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors,
+                                     batch, out_boxes, out_scores, out_counts, out_anchor_index, out_keep_pos, workspace,
+                                     workspace_bytes, nullptr, stream, h_kernel_ms);
 }
 
 int dan_sort_bboxes(const float* scores, const float* boxes, int64_t n, int32_t keep_topk, float* out_scores, float* out_boxes,
@@ -1368,7 +1466,7 @@ int dan_nms_bboxes(const float* scores, const float* boxes, int64_t n, int32_t n
   pp_bind(A, workspace, w);
   key_build_kernel<<<grid_for(n), 256, 0, st>>>(scores, n, A.keys, A.key_count);
   DAN_LAUNCH_CHECK("key_build_kernel");
-  return run_sort_nms<false, false>(A, 1, scores, reinterpret_cast<const float4*>(boxes), st);
+  return run_sort_nms<false, false, float>(A, 1, scores, reinterpret_cast<const float4*>(boxes), st);
 }
 
 }  // extern "C"

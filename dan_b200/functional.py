@@ -258,18 +258,19 @@ def encode_batch(params, ymin, xmin, ymax, xmax, inside_mask, gt_boxes, gt_offse
 # decode
 # ----------------------------------------------------------------------------------
 def decode_batch(pred_location, ymin, xmin, ymax, xmax, prior_scaling):
+    """pred_location [batch, num_preds, 4] in fp32, fp16 or bf16 -> fp32 boxes [batch, num_preds, 4]."""
     L.require_device()
     pred = pred_location.contiguous()
-    if pred.dtype != torch.float32 or pred.dim() != 3 or pred.shape[-1] != 4:
-        raise TypeError("pred_location must be fp32 [batch, num_preds, 4]")
+    if pred.dtype not in L.PRED_DTYPES or pred.dim() != 3 or pred.shape[-1] != 4:
+        raise TypeError("pred_location must be fp32, fp16 or bf16 [batch, num_preds, 4]")
     batch, n = pred.shape[0], pred.shape[1]
     if n != ymin.numel():
         raise ValueError("pred_location has %d rows but there are %d anchors" % (n, ymin.numel()))
-    out = torch.empty_like(pred)
+    out = torch.empty(pred.shape, dtype=torch.float32, device=_dev(pred))
     ps = (ctypes.c_float * 4)(*[float(v) for v in prior_scaling])
     with torch.cuda.device(_dev(pred)):
-        L.check(L.lib().dan_decode_batch(L.dev_ptr(pred), *_anchor_ptrs(ymin, xmin, ymax, xmax), n, batch, ps,
-                                         L.dev_ptr(out), L.stream_ptr()))
+        L.check(L.lib().dan_decode_batch_typed(L.pred_dtype(pred), L.dev_ptr(pred), *_anchor_ptrs(ymin, xmin, ymax, xmax), n,
+                                               batch, ps, L.dev_ptr(out), L.stream_ptr()))
     return out
 
 
@@ -393,12 +394,18 @@ def postprocess_batch(params, cls_pred, loc_pred=None, boxes_pred=None, anchors=
                       workspace=None, profile=False, peers=None):
     """Batched fused parse_by_class (bbox_util.py:103-119).  cls_pred [B,N,C]; give loc_pred [B,N,4]
     (+ anchors = (ymin,xmin,ymax,xmax)) or boxes_pred [B,N,4].  Returns Detections indexed [b, c-1].
+    The predictions are fp32, fp16 or bf16, one dtype for all of them; the outputs are fp32 and bit-identical to the
+    fp32 call on the widened predictions.
     loc_pred / boxes_pred may be PINNED HOST tensors: the kernels then read only the rows of the anchors that pass the
     score threshold, in place over PCIe (host-resident geometry, include/dan_b200.h)."""
     L.require_device()
     cls_pred = cls_pred.contiguous()
     if cls_pred.dim() != 3:
         raise TypeError("cls_pred must be [batch, num_anchors, num_classes]")
+    dtype = L.pred_dtype(cls_pred, "cls_pred")
+    geo_name, geo = ("loc_pred", loc_pred) if loc_pred is not None else ("boxes_pred", boxes_pred)
+    if isinstance(geo, torch.Tensor) and geo.dtype != cls_pred.dtype:
+        raise TypeError("cls_pred is %s but %s is %s: the predictions must share one dtype" % (cls_pred.dtype, geo_name, geo.dtype))
     batch, n, c = cls_pred.shape
     if c != params.num_classes:
         raise ValueError("cls_pred has %d classes, params say %d" % (c, params.num_classes))
@@ -422,20 +429,19 @@ def postprocess_batch(params, cls_pred, loc_pred=None, boxes_pred=None, anchors=
         aptr = [ctypes.c_void_p(0)] * 4
     nbytes = L.lib().dan_postprocess_workspace_bytes(n, batch, c, params.keep_topk)
     ws = (workspace or _ws).get(nbytes, dev)
-    args = [ctypes.byref(params), L.dev_ptr(cls_pred, torch.float32, "cls_pred"),
-            L.dev_ptr(loc_pred, torch.float32, "loc_pred", allow_pinned=True),
-            L.dev_ptr(boxes_pred, torch.float32, "boxes_pred", allow_pinned=True), *aptr, n, batch,
-            L.dev_ptr(boxes), L.dev_ptr(scores), L.dev_ptr(counts), L.dev_ptr(aidx), L.dev_ptr(kpos), L.dev_ptr(ws), nbytes,
-            L.stream_ptr()]
+    ms = (ctypes.c_float * 2)() if profile else None          # [filter, top-k/sort + NMS] in ms (synchronises)
+    # peers (L.PeerExchangeArgs): the NMS kernel also stores the slab rows into the other ranks' buffers; a profiling
+    # call takes no part in the exchange
+    exchange = ctypes.byref(peers) if peers is not None and not profile else None
     with torch.cuda.device(dev):
-        if profile:   # [filter, top-k/sort + NMS] in ms (synchronises)
-            ms = (ctypes.c_float * 2)()
-            L.check(L.lib().dan_postprocess_batch_profile(*args, ms))
-            return Detections(boxes, scores, counts, aidx, kpos), list(ms)
-        if peers is not None:   # L.PeerExchangeArgs: the NMS kernel also stores the slab rows into the other ranks' buffers
-            L.check(L.lib().dan_postprocess_batch_peers(*args[:-1], ctypes.byref(peers), args[-1]))
-            return Detections(boxes, scores, counts, aidx, kpos)
-        L.check(L.lib().dan_postprocess_batch(*args))
+        L.check(L.lib().dan_postprocess_batch_typed(
+            ctypes.byref(params), dtype, L.dev_ptr(cls_pred, cls_pred.dtype, "cls_pred"),
+            L.dev_ptr(loc_pred, cls_pred.dtype, "loc_pred", allow_pinned=True),
+            L.dev_ptr(boxes_pred, cls_pred.dtype, "boxes_pred", allow_pinned=True), *aptr, n, batch,
+            L.dev_ptr(boxes), L.dev_ptr(scores), L.dev_ptr(counts), L.dev_ptr(aidx), L.dev_ptr(kpos), L.dev_ptr(ws), nbytes,
+            exchange, L.stream_ptr(), ms))
+    if profile:
+        return Detections(boxes, scores, counts, aidx, kpos), list(ms)
     return Detections(boxes, scores, counts, aidx, kpos)
 
 

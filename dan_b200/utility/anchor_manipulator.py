@@ -173,13 +173,14 @@ class AnchorEncoder(object):
 
     # ---- :389-424 ------------------------------------------------------------------
     def batch_decode_anchors(self, pred_location, anchors_ymin, anchors_xmin, anchors_ymax, anchors_xmax):
-        """pred_location [batch, num_preds, 4] in yxhw format -> boxes [batch, num_preds, 4]."""
-        return F.decode_batch(L.as_f32(pred_location), anchors_ymin, anchors_xmin, anchors_ymax, anchors_xmax,
-                              self._prior_scaling)
+        """pred_location [batch, num_preds, 4] in yxhw format -> boxes [batch, num_preds, 4] (fp32; fp16 / bf16 CUDA
+        predictions are widened inside the kernel)."""
+        pred = pred_location if L.is_half_cuda(pred_location) else L.as_f32(pred_location)
+        return F.decode_batch(pred, anchors_ymin, anchors_xmin, anchors_ymax, anchors_xmax, self._prior_scaling)
 
     def decode_anchors(self, pred_location, anchors_ymin, anchors_xmin, anchors_ymax, anchors_xmax):
-        """pred_location [num_preds, 4] in yxhw format -> boxes [num_preds, 4]."""
-        pred = L.as_f32(pred_location)
+        """pred_location [num_preds, 4] in yxhw format -> boxes [num_preds, 4] (fp32, as batch_decode_anchors)."""
+        pred = pred_location if L.is_half_cuda(pred_location) else L.as_f32(pred_location)
         return F.decode_batch(pred.unsqueeze(0), anchors_ymin, anchors_xmin, anchors_ymax, anchors_xmax,
                               self._prior_scaling)[0]
 

@@ -71,9 +71,13 @@ def bbox_center2point(bboxes, name=None):
 
 def parse_by_class(image_shape, cls_pred, bboxes_pred, num_classes, select_threshold, min_size, keep_topk, nms_topk,
                    nms_threshold):
-    """bbox_util.py:103-119 -> ({class: boxes [nms_topk,4]}, {class: scores [nms_topk]})."""
-    cls_pred = L.as_f32(cls_pred)
-    bboxes_pred = L.as_f32(bboxes_pred)
+    """bbox_util.py:103-119 -> ({class: boxes [nms_topk,4]}, {class: scores [nms_topk]}).  fp16 / bf16 CUDA predictions
+    of ONE dtype on one device are read as they are (fp32 results, bit-identical to the call on the widened values);
+    any other pair, e.g. half logits with the fp32 boxes of decode_anchors, goes through as_f32 as a whole."""
+    if not (L.is_half_cuda(cls_pred) and L.is_half_cuda(bboxes_pred) and cls_pred.dtype == bboxes_pred.dtype
+            and cls_pred.device == bboxes_pred.device):
+        cls_pred = L.as_f32(cls_pred)
+        bboxes_pred = L.as_f32(bboxes_pred)
     params = F.postprocess_params(num_classes, image_shape, select_threshold, min_size, keep_topk, nms_topk,
                                   nms_threshold)
     det = F.postprocess_batch(params, cls_pred.unsqueeze(0), boxes_pred=bboxes_pred.unsqueeze(0), want_index=False)

@@ -50,6 +50,14 @@ extern "C" {
 #define DAN_MATCH_DUAL 0   /* do_dual_max_match, utility/anchor_manipulator.py:54-105 */
 #define DAN_MATCH_MINING 1 /* SmallMiningMatch,  cpp/ExtraLib/small_mining_match.cc   */
 
+/* element type of the predictions of the *_typed entry points.  fp16 and bf16 values
+ * are widened to fp32 as they are loaded (exact), and all arithmetic after the load is
+ * the fp32 path's: the results are bit-identical to the fp32 call on the widened
+ * predictions.  Outputs are always fp32. */
+#define DAN_DTYPE_F32 0
+#define DAN_DTYPE_F16 1
+#define DAN_DTYPE_BF16 2
+
 int dan_version(void);
 const char* dan_last_error(void);
 /* 1 when a CUDA device of compute capability 10.x is visible, else 0 (no error set). */
@@ -180,6 +188,12 @@ int dan_encode_batch_profile(const dan_encode_params* h_params, const float* a_y
 int dan_decode_batch(const float* pred, const float* a_ymin, const float* a_xmin, const float* a_ymax,
                      const float* a_xmax, int32_t num_anchors, int32_t batch,
                      const float* h_prior_scaling, float* out_boxes, void* stream);
+/* The same with pred of element type pred_dtype (DAN_DTYPE_*): 16-byte aligned for
+ * fp32, 8-byte aligned (one row per anchor) for fp16 / bf16.  out_boxes is fp32. */
+int dan_decode_batch_typed(int32_t pred_dtype, const void* pred, const float* a_ymin,
+                           const float* a_xmin, const float* a_ymax, const float* a_xmax,
+                           int32_t num_anchors, int32_t batch, const float* h_prior_scaling,
+                           float* out_boxes, void* stream);
 
 /* ------------------------------------------------------------------------- *
  * (a12-a18) utility/bbox_util.py helpers, one kernel each (elementwise).
@@ -235,6 +249,7 @@ int dan_nms_bboxes(const float* scores, const float* boxes, int64_t n, int32_t n
  * 24 bytes per anchor of a host-side caller's input are not transferred at all.
  * `cls_pred` is read in full and must be device memory.  Pageable host memory is
  * refused with DAN_ERR_INVALID_ARGUMENT.
+ * fp16 / bf16 predictions: dan_postprocess_batch_typed (section (e) below).
  * ------------------------------------------------------------------------- */
 typedef struct dan_postprocess_params {
   int32_t num_classes;
@@ -424,6 +439,31 @@ int dan_postprocess_batch_peers(const dan_postprocess_params* h_params, const fl
                                 int32_t* out_counts, int32_t* out_anchor_index, int32_t* out_keep_pos,
                                 void* workspace, size_t workspace_bytes,
                                 const dan_peer_exchange* h_peers, void* stream);
+
+/* dan_postprocess_batch / _peers / _profile with the element type of the predictions as
+ * an argument (DAN_DTYPE_*, one type for cls_pred and loc_pred / boxes_pred).  A detection
+ * head run under autocast hands over fp16 / bf16 predictions without a conversion pass,
+ * and a host-side caller sends half the bytes.  Outputs, the workspace and
+ * dan_postprocess_workspace_bytes are those of the fp32 call.
+ *   alignment: fp32 as dan_postprocess_batch; fp16 / bf16 loc_pred / boxes_pred 8-byte
+ *       aligned (one 8-byte row per anchor).  Two classes run fused into the NMS kernel
+ *       when cls_pred is aligned to one anchor's two logits (8 bytes fp32, 4 bytes
+ *       fp16 / bf16), else through the separate filter kernel.
+ *   host-resident geometry works as for fp32: the 8-byte rows are read in place and the
+ *       decoded fp32 boxes are kept in the workspace.  cls_pred must be device memory.
+ *   h_peers: NULL = no exchange (else as dan_postprocess_batch_peers).
+ *   h_kernel_ms: NULL = enqueue only (graph capturable); non-NULL = the synchronising
+ *       semantics of dan_postprocess_batch_profile.
+ *   h_peers and h_kernel_ms both non-NULL, or an unknown pred_dtype:
+ *       DAN_ERR_INVALID_ARGUMENT before anything is enqueued. */
+int dan_postprocess_batch_typed(const dan_postprocess_params* h_params, int32_t pred_dtype,
+                                const void* cls_pred, const void* loc_pred, const void* boxes_pred,
+                                const float* a_ymin, const float* a_xmin, const float* a_ymax,
+                                const float* a_xmax, int32_t num_anchors, int32_t batch,
+                                float* out_boxes, float* out_scores, int32_t* out_counts,
+                                int32_t* out_anchor_index, int32_t* out_keep_pos, void* workspace,
+                                size_t workspace_bytes, const dan_peer_exchange* h_peers,
+                                void* stream, float* h_kernel_ms);
 int dan_wait_detections(const int32_t* flags, const int32_t* state, int32_t world_size, void* stream);
 
 int dan_nccl_load(const char* path);
