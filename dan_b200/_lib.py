@@ -11,7 +11,7 @@ import os
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# DAN_B200_LIB: an alternative build of the same library (tuning experiments, -DDAN_PHASE_TIMING builds)
+# DAN_B200_LIB: an alternative build of the same library (tuning experiments, tools/variant.sh)
 LIB_PATH = os.environ.get("DAN_B200_LIB") or os.path.join(_HERE, "libdan_b200.so")
 
 DAN_MAX_LAYERS = 16

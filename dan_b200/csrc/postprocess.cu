@@ -23,20 +23,20 @@
 
 namespace dan {
 
-// phase timestamps (SM cycles) of the per-list kernels, written by thread 0 of the CTA of the longest list when the
-// library is built with -DDAN_PHASE_TIMING (tools/phase_timing.py); otherwise the macro is empty
-#ifdef DAN_PHASE_TIMING
-__device__ long long g_phase[32];
-#define DAN_PHASE(slot) do { if (threadIdx.x == 0 && blockIdx.x == 0 && blockIdx.y == 0) g_phase[slot] = clock64(); } while (0)
-#else
-#define DAN_PHASE(slot) do { } while (0)
-#endif
-
-#ifndef DAN_PP_THREADS
-#define DAN_PP_THREADS 1024           // threads of the per-list kernels (512 was measured: +20 % latency, no gain from sharing the SM
-#endif                                // with the encode CTAs)
-#define DAN_SORT_THREADS DAN_PP_THREADS
 #include "sort.cuh"
+
+// Dynamic shared memory of one nms_greedy_kernel launch (greedy_plan).  Offsets are in bytes from the start of the
+// dynamic shared memory, 16-byte aligned; the candidate boxes start at 0, over the keys.
+struct GreedyPlan {
+  int where;            // the kernel's WHERE: 0 = candidates and kept list in shared memory, 1 = candidates in the
+                        // workspace, 2 = both in the workspace (very long lists)
+  int smem;             // dynamic shared memory of the launch
+  int sort_bytes;       // bytes reserved for the keys while they are sorted
+  int slots;            // candidate slots per list (cand_slots): also the per-list stride of the workspace arrays
+  int wcap;             // 32-bit words per stripe bitset = ceil(nms_cap / 32)
+  int cand_area, cand_mask;                      // where == 0
+  int kept_box, kept_area, kept_rank, stripes;   // where <= 1; stripes: [2][32][wcap]
+};
 
 struct PpArgs {
   // inputs
@@ -56,10 +56,7 @@ struct PpArgs {
   int keep_topk, nms_topk;
   int nms_cap;                // kept-list capacity = min(nms_topk, keep_topk)
   float nms_thr;
-  // shared-memory plan of the NMS kernel (greedy_plan)
-  int sort_bytes, kcap, wcap, cand_global, kept_global;
-  int kstride;                // per-list stride of the candidate arrays = min(keep_topk, n)
-  int dyn_smem_bytes;         // dynamic shared memory of the launch
+  GreedyPlan plan;             // shared-memory plan of the NMS kernel
   // workspace
   unsigned long long* keys;   // [L, n]  L = batch * (C-1) lists
   int32_t* key_count;         // [L]
@@ -69,8 +66,8 @@ struct PpArgs {
   float* s_scores;            // sort_bboxes outputs [keep_topk]
   float4* s_boxes;
   int32_t* s_index;
-  unsigned long long* s_key;  // [L, kstride] sorted keys
-  unsigned long long* s_key2; // [L, kstride] merge buffer of lists longer than the in-shared-memory sort
+  unsigned long long* s_key;  // [L, slots] sorted keys
+  unsigned long long* s_key2; // [L, slots] merge buffer of lists longer than the in-shared-memory sort
   float4* s_box;              // [L, keep_topk] normalised corners (y0, x0, y1, x1), rank order (lists too long for shared memory)
   float* s_area;              // [L, keep_topk] (y1-y0)*(x1-x0)
   float4* g_kept_box;         // [L, keep_topk] kept list of the NMS when it does not fit shared memory
@@ -344,45 +341,27 @@ DAN_D bool f2_maybe(const PpArgs& A, float x0, float x1) {
 }
 
 // ---------------------------------------------------------------------------
-// K4+K5: one CTA per (image, class) list does everything after the filter:
-//   1. top-k select + sort of the surviving keys in shared memory (select_and_sort, sort.cuh);
-//   2. decode + clip + normalise the K best boxes (shared memory, or the workspace for very long lists);
-//   3. greedy NMS exactly as tf.image.non_max_suppression runs it - a candidate is tested against the boxes KEPT so
-//      far, never against all earlier candidates - but kChunk candidates at a time:
-//        a. every candidate of the chunk against the kept list, which is indexed by 32 x 32 stripes of the image
-//           (bitsets over the kept boxes, see the kernel): a candidate only meets the few kept boxes that share a
-//           stripe with it on both axes and leaves at the first suppressor.  Final for the candidates it suppresses,
-//           because the kept list only grows;
-//        b. the survivors are compacted in rank order;
-//        c. their mutual suppression bits T[v] = { u < v : IoU(u, v) > thr } (<= kChunk^2 / 2 tests);
-//        d. kept(v) = no kept u in T[v], evaluated by relaxation (a survivor is decided once one of its suppressors is
-//           known kept, or all are known suppressed): the number of sweeps is the longest dependency chain inside the
-//           chunk, a handful; chains longer than kMaxSweeps are finished serially by one warp;
-//        e. the kept survivors are appended to the kept list in rank order; the loop ends when nms_topk boxes are kept
-//           (max_output_size) or the candidates run out.
-//      The detections of a trained detector are clusters of near duplicates around each face: almost every candidate
-//      is removed in step a by its cluster's head after one or two exact tests, instead of the K^2 / 2 pair tests of a
-//      suppression matrix.
-//   4. the first nms_topk kept boxes are written out in rank order, zero padded (bbox_util.py:80-90).
+// K4+K5: nms_greedy_kernel, one CTA per (image, class) list, does everything after the filter.  Its steps, numbered as
+// in DESIGN.md §4b:
+//   0  filter_image        (FILTER) the two-class filter of the list's image, keys straight into shared memory
+//   1  top_k_sort          top-k select + sort of the keys (sort.cuh)
+//   2  decode_candidates   decode + clip + normalise the K best, in rank order
+//      init_stripes        the 32 x 32 stripe grid over the candidates, their stripe masks, empty bitsets and hints
+//   3  greedy NMS exactly as tf.image.non_max_suppression runs it, over a window of kWin candidates per round:
+//      a  test_window        live candidates against the kept list: cell hints, then the stripe search
+//      b  compact_survivors  the first kSurv survivors of the window, in rank order
+//      c  survivor_bits      their mutual suppression bits
+//      d  relax_survivors    kept / suppressed by relaxation
+//      e  append_kept        the kept survivors join the kept list, its stripe bitsets and hints
+//   4  write_outputs       the first nms_topk kept boxes in rank order, zero padded (bbox_util.py:80-90), peer copies
+//      release_peers       (peer exchange) the last CTA raises this rank's flag in every destination
 // ---------------------------------------------------------------------------
 constexpr int kWin = kSortThreads;                     // candidates in the window: one per thread
-#ifndef DAN_NMS_SURV
-#define DAN_NMS_SURV 128
-#endif
-constexpr int kSurv = DAN_NMS_SURV;                    // survivors resolved per round
+constexpr int kSurv = 128;                             // survivors resolved per round
 constexpr int kSurvWords = kSurv / 32;
 constexpr int kMaxSweeps = 12;
 constexpr int kHintCells = 32 * 32;                    // one hint pair per (y stripe, x stripe) cell of a box centre
 constexpr size_t kGreedySmemMax = 186 * 1024;          // dynamic part (the kernel has ~38 KB of static shared memory)
-
-struct GreedyPlan {
-  size_t smem;          // dynamic shared memory
-  int sort_bytes;       // bytes reserved for the keys while they are sorted
-  int kcap;             // candidate slots
-  int wcap;             // 32-bit words per stripe bitset = ceil(nms_cap / 32)
-  int cand_global;      // candidates live in the workspace instead of shared memory
-  int kept_global;      // so do the kept list and its stripe bitsets
-};
 
 static int next_pow2(int64_t v) {
   int p = 1;
@@ -390,26 +369,37 @@ static int next_pow2(int64_t v) {
   return p;
 }
 
+// candidate slots of a list of n anchors: min(keep_topk, n), at least one.  No upper limit: the workspace holds the
+// candidates of lists too long for shared memory.
+static int64_t cand_slots(int64_t n, int64_t keep_topk) { return keep_topk < n ? keep_topk : (n > 0 ? n : 1); }
+
 static GreedyPlan greedy_plan(int64_t n, int keep_topk, int nms_cap) {
-  GreedyPlan g;
+  GreedyPlan g = {};
   const int sort_n = (int)(n < kSortCap ? (n > 0 ? n : 1) : kSortCap);
   g.sort_bytes = next_pow2(sort_n) * 8;
-  g.kcap = (int)(keep_topk < n ? keep_topk : (n > 0 ? n : 1));      // candidate slots: no upper limit (the workspace holds them then)
+  g.slots = (int)cand_slots(n, keep_topk);
   g.wcap = (nms_cap + 31) / 32;
-  const size_t kept_bytes = align_up((size_t)nms_cap * 16, 16) + 2 * align_up((size_t)nms_cap * 4, 16) + (size_t)64 * g.wcap * 4;
-  const size_t cand_box = align_up((size_t)g.kcap * 16, 16);
+  const size_t cand_box = align_up((size_t)g.slots * 16, 16);
   const size_t region0 = cand_box > (size_t)g.sort_bytes ? cand_box : (size_t)g.sort_bytes;
-  const size_t full = region0 + align_up((size_t)g.kcap * 4, 16) + align_up((size_t)g.kcap * 8, 16) + kept_bytes;
-  g.cand_global = g.kept_global = 0;
-  g.smem = full;
-  if (full > kGreedySmemMax) {
-    g.cand_global = 1;
-    g.smem = (size_t)g.sort_bytes + kept_bytes;
-    if (g.smem > kGreedySmemMax) {
-      g.kept_global = 1;
-      g.smem = (size_t)g.sort_bytes;
-    }
+  const size_t cand_bytes = region0 + align_up((size_t)g.slots * 4, 16) + align_up((size_t)g.slots * 8, 16);
+  const size_t kept_bytes = align_up((size_t)nms_cap * 16, 16) + 2 * align_up((size_t)nms_cap * 4, 16) + (size_t)64 * g.wcap * 4;
+  size_t off = g.sort_bytes;
+  auto take = [&](size_t bytes) { const size_t at = off; off += align_up(bytes, 16); return (int)at; };
+  if (cand_bytes + kept_bytes <= kGreedySmemMax) {
+    g.where = 0;
+    off = region0;
+    g.cand_area = take((size_t)g.slots * 4);
+    g.cand_mask = take((size_t)g.slots * 8);
+  } else {
+    g.where = (size_t)g.sort_bytes + kept_bytes <= kGreedySmemMax ? 1 : 2;
   }
+  if (g.where <= 1) {
+    g.kept_box = take((size_t)nms_cap * 16);
+    g.kept_area = take((size_t)nms_cap * 4);
+    g.kept_rank = take((size_t)nms_cap * 4);
+    g.stripes = take((size_t)64 * g.wcap * 4);
+  }
+  g.smem = (int)off;
   return g;
 }
 
@@ -429,7 +419,7 @@ DAN_D void block_minmax(float lo, float hi, float& out_lo, float& out_hi) {
   __syncthreads();
 }
 
-// stripe masks of the broad phase (see the kernel); monotone in the coordinate, so overlapping intervals share a bit
+// stripe masks of the broad phase (see init_stripes); monotone in the coordinate, so overlapping intervals share a bit
 struct Stripes {
   float ylo, yinv, xlo, xinv;
   bool all;
@@ -471,9 +461,6 @@ DAN_D bool bar_or_chunk(bool pred) {
   return r != 0;
 }
 
-// WHERE: 0 = candidates and kept list in shared memory (the usual case), 1 = candidates in the workspace, 2 = both in the
-// workspace (very long lists).  A template parameter rather than a run-time pointer choice so that the shared-memory
-// accesses compile to LDS / STS / ATOMS instead of generic-address instructions.
 // A dependency chain longer than kMaxSweeps inside a chunk: one warp finishes the chunk serially (when it reaches an
 // undecided survivor every earlier one is decided); lane w holds word w of the masks.  Out of line (rare).
 __device__ __noinline__ void resolve_chunk_serially(const uint32_t* T, uint32_t* keptm, uint32_t* supm, int ns) {
@@ -495,237 +482,244 @@ __device__ __noinline__ void resolve_chunk_serially(const uint32_t* T, uint32_t*
   if (lane < kSurvWords) { keptm[lane] = kw; supm[lane] = sw; }
 }
 
-// FILTER (two classes, one list per image): the CTA also runs K3 for its image - it streams the image's logits, keeps
-// the indices of the few anchors the quick reject lets through, runs them through the exact path (softmax in
-// tf.nn.softmax's op order, threshold, decode, clip, min-size) on dense warps, and the surviving keys land directly in
-// the shared memory the sort works in: no filter launch, no key list in HBM, no global atomics.
-#ifndef DAN_NMS_REGS
-#define DAN_NMS_BOUNDS __launch_bounds__(kSortThreads, 1024 / kSortThreads)
-#else                                     // experiment: cap the registers so that CTAs of other kernels fit beside this one
-#define DAN_NMS_BOUNDS __maxnreg__(DAN_NMS_REGS)
-#endif
 constexpr int kMaybeCap = 4096;                        // indices kept in shared memory (the rest goes to the workspace)
 
-// T: element type of the predictions (DECODE only; the standalone sort / NMS instantiations take fp32 scores and boxes)
-template <bool DECODE, int WHERE, bool FILTER, typename T>
-__global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __restrict__ src_scores,
-                                                                     const float4* __restrict__ src_boxes) {
-  extern __shared__ __align__(16) unsigned char dyn_smem[];
-  __shared__ SortScratch sc;
-  __shared__ unsigned char s_alive[kWin];              // ring over the window: candidate r lives in slot r % kWin
-  __shared__ unsigned short s_list[kWin];              // step a: window offsets of the candidates that need the full search
-  __shared__ int s_surv[kSurv];                        // step b: rank of survivor u
-  __shared__ float4 s_sbox[kSurv];
-  __shared__ float s_sarea[kSurv];
-  __shared__ uint32_t s_T[kSurv][kSurvWords];
-  __shared__ uint32_t s_keptm[kSurvWords], s_supm[kSurvWords];
-  __shared__ uint2 s_smask[kSurv];
-  __shared__ int s_hint[2][kHintCells];                // suppressor hints per cell: [0] first kept box centred there, [1] last suppressor found
-  __shared__ int s_wcnt[kSortThreads / 32];
-  __shared__ int s_next[2];                            // work counters of steps a and c
-  __shared__ int s_nlist, s_cnext;
+// A list's candidates and kept list, where the carve of the kernel put them, and the state that lives across rounds.
+struct GreedyList {
+  float4* cbox;            // candidates in rank order: normalised corners (y0, x0, y1, x1)
+  float* carea;
+  uint2* cmask;            // their stripe masks
+  float4* kbox;            // kept list in the order kept
+  float* karea;
+  int* krank;              // rank of each kept box
+  uint32_t* xs;            // [32][wcap] stripe bitsets of the kept list: kept boxes touching x stripe s
+  uint32_t* ys;            // ... y stripe s
+  int wcap;
+  Stripes sg;
+  int K;                   // candidates
+  int L;                   // kept boxes so far (CTA-uniform)
+  int L_prev;              // ... when the previous round tested its window
+  int w_end_prev;          // end of the previous round's window: candidates below it carry state
+  int c0;                  // first candidate of this round's window
+};
 
-  const int list = blockIdx.x;
+// the kernel's static shared memory that steps a-e pass to each other
+struct RoundSmem {
+  unsigned char* alive;             // [kWin] ring over the window: candidate r lives in slot r % kWin
+  unsigned short* list;             // [kWin] step a: window offsets of the candidates that need the full search
+  int* surv;                        // [kSurv] step b: rank of survivor u, its box, area and stripe masks
+  float4* sbox;
+  float* sarea;
+  uint2* smask;
+  uint32_t (*T)[kSurvWords];        // [kSurv] step c: suppression bits of survivor v
+  uint32_t* keptm;                  // step d: survivors known kept / suppressed
+  uint32_t* supm;
+  int (*hint)[kHintCells];          // [2] suppressor hints per cell: [0] first kept box centred there, [1] last suppressor found
+  int* next;                        // [2] work counters of steps a and c
+  int* nlist;                       // candidates in `list`
+};
+
+// WHERE: 0 = candidates and kept list in shared memory (the usual case), 1 = candidates in the workspace, 2 = both in the
+// workspace (very long lists).  A template parameter rather than a run-time pointer choice so that the shared-memory
+// accesses compile to LDS / STS / ATOMS instead of generic-address instructions.
+template <int WHERE>
+DAN_D GreedyList carve(const PpArgs& A, unsigned char* dyn_smem, int list) {
+  const GreedyPlan& P = A.plan;
+  const int64_t o = (int64_t)list * P.slots;
+  GreedyList g;
+  if (WHERE >= 1) {
+    g.cbox = A.s_box + o;
+    g.carea = A.s_area + o;
+    g.cmask = A.s_mask + o;
+  } else {
+    g.cbox = reinterpret_cast<float4*>(dyn_smem);                                  // aliases the keys (see step 2)
+    g.carea = reinterpret_cast<float*>(dyn_smem + P.cand_area);
+    g.cmask = reinterpret_cast<uint2*>(dyn_smem + P.cand_mask);
+  }
+  uint32_t* stripes;
+  if (WHERE >= 2) {
+    g.kbox = A.g_kept_box + o;
+    g.karea = A.g_kept_area + o;
+    g.krank = A.g_kept_rank + o;
+    stripes = A.g_stripes + (int64_t)list * 64 * ((P.slots + 31) / 32);
+  } else {
+    g.kbox = reinterpret_cast<float4*>(dyn_smem + P.kept_box);
+    g.karea = reinterpret_cast<float*>(dyn_smem + P.kept_area);
+    g.krank = reinterpret_cast<int*>(dyn_smem + P.kept_rank);
+    stripes = reinterpret_cast<uint32_t*>(dyn_smem + P.stripes);
+  }
+  g.wcap = P.wcap;
+  g.xs = stripes;
+  g.ys = stripes + 32 * g.wcap;
+  g.L = g.L_prev = g.w_end_prev = g.c0 = 0;
+  return g;
+}
+
+// ---- 0. FILTER (two classes, one list per image): the CTA also runs K3 for its image - it streams the image's logits,
+// keeps the indices of the few anchors the quick reject lets through, runs them through the exact path (softmax in
+// tf.nn.softmax's op order, threshold, decode, clip, min-size) on dense warps, and the surviving keys land directly in
+// the shared memory the sort works in: no filter launch, no key list in HBM, no global atomics.  Returns the number of
+// keys; beyond the sort's shared memory they are in gkeys.
+template <typename T>
+DAN_D int filter_image(const PpArgs& A, int list, int b, unsigned long long* keys, unsigned long long* gkeys) {
+  __shared__ int s_maybe[kMaybeCap];
+  __shared__ int s_nmaybe, s_nkeys;
   const int tid = threadIdx.x;
   const int lane = tid & 31;
-  const int warp = tid >> 5;
   const unsigned lt_mask = (1u << lane) - 1u;
-  const int b = list / max(A.num_classes - 1, 1);
-  const int64_t o = (int64_t)list * A.kstride;
-  const float thr = A.nms_thr;
-
-  // ---- carve
-  unsigned long long* keys = reinterpret_cast<unsigned long long*>(dyn_smem);
-  float4* cbox;
-  float* carea;
-  uint2* cmask;
-  unsigned char* p;
-  if (WHERE >= 1) {
-    cbox = A.s_box + o;
-    carea = A.s_area + o;
-    cmask = A.s_mask + o;
-    p = dyn_smem + A.sort_bytes;
-  } else {
-    const size_t cand_box = ((size_t)A.kcap * 16 + 15) / 16 * 16;
-    cbox = reinterpret_cast<float4*>(dyn_smem);                                    // aliases the keys (see step 2)
-    carea = reinterpret_cast<float*>(dyn_smem + (cand_box > (size_t)A.sort_bytes ? cand_box : (size_t)A.sort_bytes));
-    cmask = reinterpret_cast<uint2*>(reinterpret_cast<unsigned char*>(carea) + ((size_t)A.kcap * 4 + 15) / 16 * 16);
-    p = reinterpret_cast<unsigned char*>(cmask) + ((size_t)A.kcap * 8 + 15) / 16 * 16;
-  }
-  float4* kbox;
-  float* karea;
-  int* krank;
-  uint32_t* stripes;                                   // [2][32][wcap]: kept boxes touching x stripe s / y stripe s
-  const int wcap = A.wcap;
-  if (WHERE >= 2) {
-    const int64_t ok = (int64_t)list * A.kstride;
-    kbox = A.g_kept_box + ok;
-    karea = A.g_kept_area + ok;
-    krank = A.g_kept_rank + ok;
-    stripes = A.g_stripes + (int64_t)list * 64 * ((A.kstride + 31) / 32);
-  } else {
-    kbox = reinterpret_cast<float4*>(p); p += ((size_t)A.nms_cap * 16 + 15) / 16 * 16;
-    karea = reinterpret_cast<float*>(p); p += ((size_t)A.nms_cap * 4 + 15) / 16 * 16;
-    krank = reinterpret_cast<int*>(p); p += ((size_t)A.nms_cap * 4 + 15) / 16 * 16;
-    stripes = reinterpret_cast<uint32_t*>(p);
-  }
-  uint32_t* xs = stripes;
-  uint32_t* ys = stripes + 32 * wcap;
-
-  // ---- 0. filter (FILTER) or the number of keys the filter kernel left in the workspace
-  DAN_PHASE(0);
-  unsigned long long* gkeys = A.keys + (int64_t)list * A.n;
-  int cnt;
-  if (FILTER) {
-    __shared__ int s_maybe[kMaybeCap];
-    __shared__ int s_nmaybe, s_nkeys;
-    int* gmaybe = A.maybe + (int64_t)list * A.n;
-    const int key_cap = A.sort_bytes / 8;              // keys that fit the sort's shared memory
-    if (tid == 0) { s_nmaybe = 0; s_nkeys = 0; }
-    __syncthreads();
-    auto put = [&](int pos, int a) {
-      if (pos < kMaybeCap) s_maybe[pos] = a;
-      else gmaybe[pos] = a;
-    };
-    auto push = [&](int a) { put(atomicAdd(&s_nmaybe, 1), a); };
-    // The image's logits as 16-byte vectors of kVA anchors (2 for fp32, 4 for fp16 / bf16).  The row of an image starts
-    // aligned to one anchor only (8 or 4 bytes): the `head` anchors before the first 16-byte boundary and the ones behind
-    // the last whole vector are read as pairs after the loop.
-    constexpr int kVA = 16 / (2 * (int)sizeof(T));
-    const T* x = static_cast<const T*>(A.cls) + (int64_t)b * A.n * 2;
-    // (fp32 keeps the statements it had before fp16 / bf16 were added, so that it compiles to the same instructions)
-    const int head = kVA == 2 ? ((reinterpret_cast<uintptr_t>(x) & 15u) ? 1 : 0)
-                              : min((int)(((16u - (unsigned)(reinterpret_cast<uintptr_t>(x) & 15u)) & 15u) / (2 * sizeof(T))), A.n);
-    const int nvec = kVA == 2 ? (A.n - head) >> 1 : (int)((unsigned)(A.n - head) / kVA);
-    const float4* xv = reinterpret_cast<const float4*>(x + 2 * head);
-    for (int v0 = 0; v0 < nvec; v0 += 4 * kSortThreads) {
-      float4 q[4];
+  int* gmaybe = A.maybe + (int64_t)list * A.n;
+  const int key_cap = A.plan.sort_bytes / 8;           // keys that fit the sort's shared memory
+  if (tid == 0) { s_nmaybe = 0; s_nkeys = 0; }
+  __syncthreads();
+  auto put = [&](int pos, int a) {
+    if (pos < kMaybeCap) s_maybe[pos] = a;
+    else gmaybe[pos] = a;
+  };
+  auto push = [&](int a) { put(atomicAdd(&s_nmaybe, 1), a); };
+  // The image's logits as 16-byte vectors of kVA anchors (2 for fp32, 4 for fp16 / bf16).  The row of an image starts
+  // aligned to one anchor only (8 or 4 bytes): the `head` anchors before the first 16-byte boundary and the ones behind
+  // the last whole vector are read as pairs after the loop.
+  constexpr int kVA = 16 / (2 * (int)sizeof(T));
+  const T* x = static_cast<const T*>(A.cls) + (int64_t)b * A.n * 2;
+  // (fp32 keeps the statements it had before fp16 / bf16 were added, so that it compiles to the same instructions)
+  const int head = kVA == 2 ? ((reinterpret_cast<uintptr_t>(x) & 15u) ? 1 : 0)
+                            : min((int)(((16u - (unsigned)(reinterpret_cast<uintptr_t>(x) & 15u)) & 15u) / (2 * sizeof(T))), A.n);
+  const int nvec = kVA == 2 ? (A.n - head) >> 1 : (int)((unsigned)(A.n - head) / kVA);
+  const float4* xv = reinterpret_cast<const float4*>(x + 2 * head);
+  for (int v0 = 0; v0 < nvec; v0 += 4 * kSortThreads) {
+    float4 q[4];
 #pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const int v = v0 + u * kSortThreads + tid;
-        q[u] = (v < nvec) ? __ldcs(xv + v) : make_float4(0.f, 0.f, 0.f, 0.f);       // read once: streaming
-      }
+    for (int u = 0; u < 4; ++u) {
+      const int v = v0 + u * kSortThreads + tid;
+      q[u] = (v < nvec) ? __ldcs(xv + v) : make_float4(0.f, 0.f, 0.f, 0.f);       // read once: streaming
+    }
 #pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        // A warp looks at 32 * kVA consecutive anchors here.  Its survivors enter the list in ANCHOR order with one atomic
-        // per warp: the exact pass below then reads neighbouring box rows from neighbouring lanes, i.e. whole sectors -
-        // which matters when the rows live in host memory and every sector is a PCIe read.
-        const int v = v0 + u * kSortThreads + tid;
-        if constexpr (kVA == 2) {
-          const bool p0 = v < nvec && f2_maybe(A, q[u].x, q[u].y);
-          const bool p1 = v < nvec && f2_maybe(A, q[u].z, q[u].w);
-          const unsigned m0 = __ballot_sync(0xffffffffu, p0), m1 = __ballot_sync(0xffffffffu, p1);
-          if ((m0 | m1) != 0u) {
-            int base = 0;
-            if (lane == 0) base = atomicAdd(&s_nmaybe, __popc(m0) + __popc(m1));
-            base = __shfl_sync(0xffffffffu, base, 0);
-            int pos = base + __popc(m0 & lt_mask) + __popc(m1 & lt_mask);
-            if (p0) put(pos++, head + 2 * v);
-            if (p1) put(pos, head + 2 * v + 1);
-          }
-        } else {
-          bool pj[kVA];
-          unsigned mj[kVA], any = 0u;
+    for (int u = 0; u < 4; ++u) {
+      // A warp looks at 32 * kVA consecutive anchors here.  Its survivors enter the list in ANCHOR order with one atomic
+      // per warp: the exact pass below then reads neighbouring box rows from neighbouring lanes, i.e. whole sectors -
+      // which matters when the rows live in host memory and every sector is a PCIe read.
+      const int v = v0 + u * kSortThreads + tid;
+      if constexpr (kVA == 2) {
+        const bool p0 = v < nvec && f2_maybe(A, q[u].x, q[u].y);
+        const bool p1 = v < nvec && f2_maybe(A, q[u].z, q[u].w);
+        const unsigned m0 = __ballot_sync(0xffffffffu, p0), m1 = __ballot_sync(0xffffffffu, p1);
+        if ((m0 | m1) != 0u) {
+          int base = 0;
+          if (lane == 0) base = atomicAdd(&s_nmaybe, __popc(m0) + __popc(m1));
+          base = __shfl_sync(0xffffffffu, base, 0);
+          int pos = base + __popc(m0 & lt_mask) + __popc(m1 & lt_mask);
+          if (p0) put(pos++, head + 2 * v);
+          if (p1) put(pos, head + 2 * v + 1);
+        }
+      } else {
+        bool pj[kVA];
+        unsigned mj[kVA], any = 0u;
+#pragma unroll
+        for (int j = 0; j < kVA; ++j) {
+          const float2 xx = vec_pair<T>(q[u], j);
+          pj[j] = v < nvec && f2_maybe(A, xx.x, xx.y);
+        }
+#pragma unroll
+        for (int j = 0; j < kVA; ++j) {
+          mj[j] = __ballot_sync(0xffffffffu, pj[j]);
+          any |= mj[j];
+        }
+        if (any != 0u) {
+          int nj = 0, below = 0;
 #pragma unroll
           for (int j = 0; j < kVA; ++j) {
-            const float2 xx = vec_pair<T>(q[u], j);
-            pj[j] = v < nvec && f2_maybe(A, xx.x, xx.y);
+            nj += __popc(mj[j]);
+            below += __popc(mj[j] & lt_mask);
           }
+          int base = 0;
+          if (lane == 0) base = atomicAdd(&s_nmaybe, nj);
+          base = __shfl_sync(0xffffffffu, base, 0);
+          int pos = base + below;
 #pragma unroll
-          for (int j = 0; j < kVA; ++j) {
-            mj[j] = __ballot_sync(0xffffffffu, pj[j]);
-            any |= mj[j];
-          }
-          if (any != 0u) {
-            int nj = 0, below = 0;
-#pragma unroll
-            for (int j = 0; j < kVA; ++j) {
-              nj += __popc(mj[j]);
-              below += __popc(mj[j] & lt_mask);
-            }
-            int base = 0;
-            if (lane == 0) base = atomicAdd(&s_nmaybe, nj);
-            base = __shfl_sync(0xffffffffu, base, 0);
-            int pos = base + below;
-#pragma unroll
-            for (int j = 0; j < kVA; ++j)
-              if (pj[j]) put(pos++, head + kVA * v + j);
-          }
+          for (int j = 0; j < kVA; ++j)
+            if (pj[j]) put(pos++, head + kVA * v + j);
         }
       }
     }
-    if constexpr (kVA == 2) {                          // fp32: at most one anchor on either side
-      if (tid == 0 && head == 1 && f2_maybe(A, x[0], x[1])) push(0);
-      if (tid == 1 && head + 2 * nvec < A.n && f2_maybe(A, x[2 * (A.n - 1)], x[2 * (A.n - 1) + 1])) push(A.n - 1);
-    } else {
-      // head: threads [0, head); tail (fewer than kVA anchors behind the vectors): threads [kVA - 1, 2 kVA - 1)
-      const int rest = head + kVA * nvec;
-      const int t = tid - (kVA - 1);
-      if (tid < head) {
-        const float2 xx = make_float2(widen(x[2 * tid]), widen(x[2 * tid + 1]));
-        if (f2_maybe(A, xx.x, xx.y)) push(tid);
-      }
-      if (t >= 0 && rest + t < A.n) {
-        const float2 xx = make_float2(widen(x[2 * (rest + t)]), widen(x[2 * (rest + t) + 1]));
-        if (f2_maybe(A, xx.x, xx.y)) push(rest + t);
-      }
+  }
+  if constexpr (kVA == 2) {                            // fp32: at most one anchor on either side
+    if (tid == 0 && head == 1 && f2_maybe(A, x[0], x[1])) push(0);
+    if (tid == 1 && head + 2 * nvec < A.n && f2_maybe(A, x[2 * (A.n - 1)], x[2 * (A.n - 1) + 1])) push(A.n - 1);
+  } else {
+    // head: threads [0, head); tail (fewer than kVA anchors behind the vectors): threads [kVA - 1, 2 kVA - 1)
+    const int rest = head + kVA * nvec;
+    const int t = tid - (kVA - 1);
+    if (tid < head) {
+      const float2 xx = make_float2(widen(x[2 * tid]), widen(x[2 * tid + 1]));
+      if (f2_maybe(A, xx.x, xx.y)) push(tid);
     }
-    __syncthreads();
-    const int nmaybe = s_nmaybe;
-    for (int i0 = 0; i0 < nmaybe; i0 += kSortThreads) {
-      const int i = i0 + tid;
-      if (i < nmaybe) {
-        const int a = (i < kMaybeCap) ? s_maybe[i] : gmaybe[i];
-        const float2 xx = ld_pair(x + 2 * a);
-        // tf.nn.softmax: exp(x - max) * (1 / sum(exp(x - max))), sum in class order
-        const float mx = fmaxf(xx.x, xx.y);
-        const float e0 = cephes_expf(fsub(xx.x, mx));
-        const float e1 = cephes_expf(fsub(xx.y, mx));
-        const float pr = fmul(e1, fdiv(1.f, fadd(e0, e1)));
-        if (pr > A.select_thr) {                            // select_bboxes :24-36
-          const float4 box = pp_box<T>(A, b, a);
-          if (A.stash != nullptr) A.stash[(int64_t)b * A.n + a] = box;
-          const float w = fadd(fsub(box.w, box.y), 1.f);    // filter_bboxes :50-59
-          const float h = fadd(fsub(box.z, box.x), 1.f);
-          if ((w > A.min_size_p1) && (h > A.min_size_p1)) {
-            const unsigned long long key = ((unsigned long long)score_to_key(pr) << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)a);
-            const int pos = atomicAdd(&s_nkeys, 1);
-            if (pos < key_cap) keys[pos] = key;
-            else gkeys[pos] = key;
-          }
+    if (t >= 0 && rest + t < A.n) {
+      const float2 xx = make_float2(widen(x[2 * (rest + t)]), widen(x[2 * (rest + t) + 1]));
+      if (f2_maybe(A, xx.x, xx.y)) push(rest + t);
+    }
+  }
+  __syncthreads();
+  const int nmaybe = s_nmaybe;
+  for (int i0 = 0; i0 < nmaybe; i0 += kSortThreads) {
+    const int i = i0 + tid;
+    if (i < nmaybe) {
+      const int a = (i < kMaybeCap) ? s_maybe[i] : gmaybe[i];
+      const float2 xx = ld_pair(x + 2 * a);
+      // tf.nn.softmax: exp(x - max) * (1 / sum(exp(x - max))), sum in class order
+      const float mx = fmaxf(xx.x, xx.y);
+      const float e0 = cephes_expf(fsub(xx.x, mx));
+      const float e1 = cephes_expf(fsub(xx.y, mx));
+      const float pr = fmul(e1, fdiv(1.f, fadd(e0, e1)));
+      if (pr > A.select_thr) {                            // select_bboxes :24-36
+        const float4 box = pp_box<T>(A, b, a);
+        if (A.stash != nullptr) A.stash[(int64_t)b * A.n + a] = box;
+        const float w = fadd(fsub(box.w, box.y), 1.f);    // filter_bboxes :50-59
+        const float h = fadd(fsub(box.z, box.x), 1.f);
+        if ((w > A.min_size_p1) && (h > A.min_size_p1)) {
+          const unsigned long long key = ((unsigned long long)score_to_key(pr) << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)a);
+          const int pos = atomicAdd(&s_nkeys, 1);
+          if (pos < key_cap) keys[pos] = key;
+          else gkeys[pos] = key;
         }
       }
     }
-    __syncthreads();
-    cnt = s_nkeys;
-    if (cnt > kSortCap) {                                   // too many survivors for shared memory: the select runs on HBM
-      for (int i = tid; i < min(cnt, key_cap); i += kSortThreads) gkeys[i] = keys[i];
-      __syncthreads();
-    }
-  } else {
-    cnt = min(A.key_count[list], A.n);
   }
+  __syncthreads();
+  const int cnt = s_nkeys;
+  if (cnt > kSortCap) {                                   // too many survivors for shared memory: the select runs on HBM
+    for (int i = tid; i < min(cnt, key_cap); i += kSortThreads) gkeys[i] = keys[i];
+    __syncthreads();
+  }
+  return cnt;
+}
 
-  // ---- 1. top-k + sort
-  DAN_PHASE(8);
+// ---- 1. top-k + sort of the list's cnt keys; returns K, the number of candidates, and where their sorted keys are:
+// in shared memory, or at A.s_key + o for lists longer than kSortCap
+template <bool FILTER>
+DAN_D int top_k_sort(const PpArgs& A, int cnt, int64_t o, const unsigned long long* gkeys, unsigned long long* keys,
+                     unsigned char* dyn_smem, const unsigned long long*& sorted) {
+  __shared__ SortScratch sc;
   const int k_want = min(A.keep_topk, cnt);
-  int K;
-  const unsigned long long* sorted = keys;            // shared memory, or A.s_key for lists longer than kSortCap
+  sorted = keys;
   if (k_want <= kSortCap) {
     // a second key buffer behind the first one when the CTA's shared memory holds it (nothing else lives there yet)
-    unsigned long long* spare = ((size_t)A.sort_bytes + (size_t)min(cnt, kSortCap) * 8 <= (size_t)A.dyn_smem_bytes)
-                                    ? reinterpret_cast<unsigned long long*>(dyn_smem + A.sort_bytes) : nullptr;
-    K = min(select_and_sort(gkeys, cnt, k_want, keys, sc, FILTER, spare), A.keep_topk);
-  } else {
-    select_and_sort_large(gkeys, cnt, k_want, A.s_key + o, A.s_key2 + o, keys, sc);
-    sorted = A.s_key + o;
-    K = k_want;
+    unsigned long long* spare = ((size_t)A.plan.sort_bytes + (size_t)min(cnt, kSortCap) * 8 <= (size_t)A.plan.smem)
+                                    ? reinterpret_cast<unsigned long long*>(dyn_smem + A.plan.sort_bytes) : nullptr;
+    return min(select_and_sort(gkeys, cnt, k_want, keys, sc, FILTER, spare), A.keep_topk);
   }
-  DAN_PHASE(1);
+  select_and_sort_large(gkeys, cnt, k_want, A.s_key + o, A.s_key2 + o, keys, sc);
+  sorted = A.s_key + o;
+  return k_want;
+}
 
-  // ---- 2. decode + clip + normalise.  The candidate boxes (16 B) reuse the shared memory of the keys (8 B): the ranks
-  // are walked in DEscending batches of one key per thread, so a batch's boxes only overwrite key slots of ranks that
-  // are already done (box r covers key slots 2r and 2r+1 >= r); the barrier protects the batch's own keys.
+// ---- 2. decode + clip + normalise.  The candidate boxes (16 B) reuse the shared memory of the keys (8 B): the ranks
+// are walked in DEscending batches of one key per thread, so a batch's boxes only overwrite key slots of ranks that
+// are already done (box r covers key slots 2r and 2r+1 >= r); the barrier protects the batch's own keys.
+template <bool DECODE, typename T>
+DAN_D void decode_candidates(const PpArgs& A, int b, int64_t o, const unsigned long long* sorted, const float4* src_boxes,
+                             GreedyList& g) {
+  const int tid = threadIdx.x;
+  const int K = g.K;
   for (int r0 = K > 0 ? ((K - 1) / kSortThreads) * kSortThreads : -1; r0 >= 0; r0 -= kSortThreads) {
     const int r = r0 + tid;
     const unsigned long long key = (r < K) ? sorted[r] : 0ull;
@@ -734,33 +728,25 @@ __global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __
     if (r < K) {
       const uint32_t idx = key_index(key);
       const NmsBox nb = nms_norm(DECODE ? (A.stash != nullptr ? A.stash[(int64_t)b * A.n + idx] : pp_box<T>(A, b, (int)idx)) : src_boxes[idx]);
-      cbox[r] = make_float4(nb.y0, nb.x0, nb.y1, nb.x1);
-      carea[r] = nb.area;
+      g.cbox[r] = make_float4(nb.y0, nb.x0, nb.y1, nb.x1);
+      g.carea[r] = nb.area;
     }
   }
   __syncthreads();
-  DAN_PHASE(2);
+}
 
-  // ---- 3. greedy NMS, kChunk candidates per round
-#ifdef DAN_PHASE_TIMING
-  long long acc[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0}, t_a = 0, t_b = 0, n_sweeps = 0, n_surv = 0, n_chunks = 0;
-#define DAN_LAP(i) do { const long long now__ = clock64(); acc[i] += now__ - t_b; t_b = now__; } while (0)
-#define DAN_TICK() (t_a = clock64())
-#define DAN_TOCK(i) (acc[i] += clock64() - t_a)
-#else
-#define DAN_TICK() do { } while (0)
-#define DAN_TOCK(i) do { } while (0)
-#define DAN_LAP(i) do { } while (0)
-#endif
-  // Broad phase: the extent of the candidates is cut into 32 stripes per axis and every box carries the two 32-bit masks
-  // of the stripes it touches.  Boxes that intersect share a stripe on both axes, so a pair whose masks do not meet on
-  // either axis needs no exact test.
-  Stripes sg;
+// Broad phase: the extent of the candidates is cut into 32 stripes per axis and every box carries the two 32-bit masks
+// of the stripes it touches.  Boxes that intersect share a stripe on both axes, so a pair whose masks do not meet on
+// either axis needs no exact test.  Also empties the kept list's stripe bitsets and the hints.
+DAN_D void init_stripes(const PpArgs& A, GreedyList& g, RoundSmem& R) {
+  const int tid = threadIdx.x;
+  const int K = g.K;
+  Stripes& sg = g.sg;
   {
     float ylo = 3.0e38f, yhi = -3.0e38f, xlo = 3.0e38f, xhi = -3.0e38f;
     for (int r = tid; r < K; r += kSortThreads) {
-      const float4 bx = cbox[r];
-      if (carea[r] > 0.f && fabsf(bx.x) < 1e30f && fabsf(bx.y) < 1e30f && fabsf(bx.z) < 1e30f && fabsf(bx.w) < 1e30f) {
+      const float4 bx = g.cbox[r];
+      if (g.carea[r] > 0.f && fabsf(bx.x) < 1e30f && fabsf(bx.y) < 1e30f && fabsf(bx.z) < 1e30f && fabsf(bx.w) < 1e30f) {
         ylo = fminf(ylo, bx.x); yhi = fmaxf(yhi, bx.z);
         xlo = fminf(xlo, bx.y); xhi = fmaxf(xhi, bx.w);
       }
@@ -770,268 +756,278 @@ __global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __
     block_minmax(xlo, xhi, sg.xlo, ex);
     sg.yinv = (ey > sg.ylo) ? 32.f / (ey - sg.ylo) : 0.f;
     sg.xinv = (ex > sg.xlo) ? 32.f / (ex - sg.xlo) : 0.f;
-    sg.all = thr < 0.f;                                // a negative threshold: disjoint boxes suppress too
+    sg.all = A.nms_thr < 0.f;                          // a negative threshold: disjoint boxes suppress too
   }
-  for (int r = tid; r < K; r += kSortThreads) cmask[r] = sg.masks(cbox[r], carea[r]);
-  for (int i = tid; i < 64 * wcap; i += kSortThreads) stripes[i] = 0u;
-  for (int i = tid; i < 2 * kHintCells; i += kSortThreads) (&s_hint[0][0])[i] = 0x7fffffff;
-  if (tid < 2) s_next[tid] = 0;
-  if (tid == 0) s_nlist = 0;
+  for (int r = tid; r < K; r += kSortThreads) g.cmask[r] = sg.masks(g.cbox[r], g.carea[r]);
+  for (int i = tid; i < 64 * g.wcap; i += kSortThreads) g.xs[i] = 0u;
+  for (int i = tid; i < 2 * kHintCells; i += kSortThreads) (&R.hint[0][0])[i] = 0x7fffffff;
+  if (tid < 2) R.next[tid] = 0;
+  if (tid == 0) *R.nlist = 0;
   __syncthreads();
-  int L = 0;                                           // kept boxes so far (CTA-uniform)
-  int L_prev = 0;                                      // ... when the previous round tested its window
-  int w_end_prev = 0;                                  // end of the previous round's window: candidates below it carry state
-  for (int c0 = 0; c0 < K && L < A.nms_topk;) {
-    const int w_end = min(K, c0 + kWin);
-    DAN_TICK();
-    // a. window vs kept list.  Thread t owns candidate c0 + t.  A candidate that was in the previous window has met
-    // the first L_prev kept boxes already; a fresh one has met none.
-    const int my_r = c0 + tid;
-    const bool in_win = my_r < w_end;
-    {
-      bool alive = false, search = false;
-      int upto = 0;
-      if (in_win) {
-        const bool fresh = my_r >= w_end_prev;
-        alive = fresh ? true : (s_alive[my_r & (kWin - 1)] != 0);
-        upto = fresh ? 0 : L_prev;
-      }
-      if (alive && L > upto) {
-        const uint2 mm = cmask[my_r];
-        if (mm.x != 0u && mm.y != 0u) {                // (no area: no stripes, never suppressed)
-          // a1. the two hinted kept boxes of the cell of its centre: a member of a cluster of near duplicates dies here,
-          // after one or two exact tests by its own thread
-          const float4 me = cbox[my_r];
-          const float my_area = carea[my_r];
-          const int cl = sg.cell(me);
-          const int h0 = s_hint[0][cl], h1 = s_hint[1][cl];
-          bool dead = false;
-          if (h0 >= upto && h0 < L) dead = pair_suppresses(kbox[h0], karea[h0], me, my_area, thr);
-          if (!dead && h1 != h0 && h1 >= upto && h1 < L) dead = pair_suppresses(kbox[h1], karea[h1], me, my_area, thr);
-          alive = !dead;
-          search = !dead;
-        }
-      }
-      if (in_win) s_alive[my_r & (kWin - 1)] = alive ? 1 : 0;
-      const unsigned sm = __ballot_sync(0xffffffffu, search);
-      int base = 0;
-      if (lane == 0 && sm != 0u) base = atomicAdd(&s_nlist, __popc(sm));
-      base = __shfl_sync(0xffffffffu, base, 0);
-      if (search) s_list[base + __popc(sm & lt_mask)] = (unsigned short)tid;
-    }
-    __syncthreads();
-    // a2. the others against the kept list proper, which is indexed by stripe: bit j of xs[s] / ys[s] says that kept box j
-    // touches x / y stripe s.  The kept boxes a candidate can intersect are (OR of xs over its x stripes) AND (OR of ys
-    // over its y stripes): a group of G lanes owns one candidate, a lane one 32-bit word of the bitset, and only the set
-    // bits (beyond the boxes the candidate has met already) go through the exact test; the candidate leaves at the
-    // first suppressor, which becomes the cell's second hint.
-    const int nlist = s_nlist;
-    if (nlist > 0) {
-      const int W = (L + 31) >> 5;
-      const int G = W <= 8 ? 8 : (W <= 16 ? 16 : 32);        // lanes per candidate
-      const int cpw = 32 / G;                                // candidates per warp pass
-      const int gl = lane & (G - 1), sub = lane / G;
-      const unsigned gmask = (G == 32 ? 0xffffffffu : ((1u << G) - 1u)) << (sub * G);
-      while (true) {                                         // candidates are handed out dynamically: their cost varies a lot
-        int i0 = 0;
-        if (lane == 0) i0 = atomicAdd(&s_next[0], cpw);
-        i0 = __shfl_sync(0xffffffffu, i0, 0);
-        if (i0 >= nlist) break;
-        const bool have = i0 + sub < nlist;
-        const int r = c0 + (have ? (int)s_list[i0 + sub] : 0);
-        const float4 me = have ? cbox[r] : make_float4(0.f, 0.f, 0.f, 0.f);
-        const float my_area = have ? carea[r] : 0.f;
-        const uint2 mm = have ? cmask[r] : make_uint2(0u, 0u);
-        const int upto = (r >= w_end_prev) ? 0 : L_prev;
-        bool sup = false;
-        for (int wb = 0; wb < W; wb += G) {                  // one block of words unless the kept list is very long
-          const int w = wb + gl;
-          uint32_t poss = 0u;
-          if (w < W && w >= (upto >> 5) && mm.x != 0u && mm.y != 0u) {
-            // (the stripes of a box are a contiguous range: independent loads, no address chain)
-            uint32_t ax = 0u, ay = 0u;
-            const int xe = 31 - __clz(mm.x), ye = 31 - __clz(mm.y);
-#pragma unroll 2
-            for (int st = __ffs(mm.x) - 1; st <= xe; ++st) ax |= xs[st * wcap + w];
-#pragma unroll 2
-            for (int st = __ffs(mm.y) - 1; st <= ye; ++st) ay |= ys[st * wcap + w];
-            poss = ax & ay;
-            if (w == (upto >> 5)) poss &= ~((1u << (upto & 31)) - 1u);
-          }
-          while (__any_sync(0xffffffffu, poss != 0u && !sup)) {
-            bool t = false;
-            if (poss != 0u && !sup) {
-              const int j = (w << 5) + __ffs(poss) - 1;
-              poss &= poss - 1u;
-              t = pair_suppresses(kbox[j], karea[j], me, my_area, thr);
-              if (t) atomicExch(&s_hint[1][sg.cell(me)], j);
-            }
-            if ((__ballot_sync(0xffffffffu, t) & gmask) != 0u) sup = true;
-          }
-        }
-        if (have && gl == 0 && sup) s_alive[r & (kWin - 1)] = 0;
-      }
-    }
-    __syncthreads();
-    DAN_TOCK(0);
-    DAN_TICK();
-    // b. the first kSurv candidates of the window that are still alive, in rank order; the window of the next round
-    // starts behind the last of them
-    const bool f = in_win && s_alive[my_r & (kWin - 1)] != 0;
-    const unsigned fm = __ballot_sync(0xffffffffu, f);
-    if (lane == 0) s_wcnt[warp] = __popc(fm);
-    if (tid < kSurvWords) { s_keptm[tid] = 0u; s_supm[tid] = 0u; }
-    __syncthreads();
-    int total, ubase;
-    {
-      const int cw = (lane < kSortThreads / 32) ? s_wcnt[lane] : 0;
-      int incl = cw;
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) {
-        const int up = __shfl_up_sync(0xffffffffu, incl, d);
-        if (lane >= d) incl += up;
-      }
-      total = __shfl_sync(0xffffffffu, incl, 31);
-      ubase = __shfl_sync(0xffffffffu, incl - cw, warp & 31);
-    }
-    if (f) {
-      const int u = ubase + __popc(fm & lt_mask);
-      if (u < kSurv) {
-        s_surv[u] = my_r;
-        s_sbox[u] = cbox[my_r];
-        s_sarea[u] = carea[my_r];
-        s_smask[u] = cmask[my_r];
-        if (u == kSurv - 1) s_cnext = my_r + 1;
-      }
-    }
-    __syncthreads();
-    const int ns = min(total, kSurv);
-    const int c_next = (total >= kSurv) ? s_cnext : w_end;
-    DAN_TOCK(1);
-    DAN_TICK();
-    // c. suppression bits among the survivors: warp -> row v, lanes -> 32 earlier survivors per step
-    while (true) {                                           // rows handed out dynamically, the longest ones first
-      int vi = 0;
-      if (lane == 0) vi = atomicAdd(&s_next[1], 1);
-      vi = __shfl_sync(0xffffffffu, vi, 0);
-      if (vi >= ns) break;
-      const int v = ns - 1 - vi;
-      const float4 me = s_sbox[v];
-      const float my_area = s_sarea[v];
-      const uint2 mm = s_smask[v];
-      const int nw = (v + 31) >> 5;                    // words that hold some u < v
-      for (int w = 0; w < nw; ++w) {
-        const int u = (w << 5) + lane;
-        const uint2 um = s_smask[u];
-        const bool poss = (u < v) && (um.x & mm.x) != 0u && (um.y & mm.y) != 0u;
-        unsigned bits = 0u;
-        if (__any_sync(0xffffffffu, poss)) {
-          const bool t = poss && pair_suppresses(s_sbox[u], s_sarea[u], me, my_area, thr);
-          bits = __ballot_sync(0xffffffffu, t);
-        }
-        if (lane == 0) s_T[v][w] = bits;
-      }
-    }
-    __syncthreads();
-    DAN_TOCK(2);
-    DAN_TICK();
-    // d. relaxation: thread v owns survivor v (the first kSurv threads)
-    int sweeps = 0;
-    if (tid < kSurv) {
-      uint32_t trow[kSurvWords];
-      const int vw = tid >> 5;
-      const uint32_t vbit = 1u << (tid & 31);
-      const bool mine = tid < ns;
-#pragma unroll
-      for (int w = 0; w < kSurvWords; ++w) trow[w] = (mine && (w << 5) < tid) ? s_T[tid][w] : 0u;
-      bool decided = !mine;
-      bool open = true;
-      while (open && sweeps < kMaxSweeps) {
-        uint32_t hitm = 0u, pendm = 0u;
-        if (!decided) {
-#pragma unroll
-          for (int w = 0; w < kSurvWords; ++w) {
-            const uint32_t kw = s_keptm[w], sw = s_supm[w];
-            hitm |= trow[w] & kw;
-            pendm |= trow[w] & ~(kw | sw);
-          }
-        }
-        bar_sync_chunk();                              // every thread has read the masks of the previous sweep
-        if (!decided) {
-          if (hitm != 0u) { atomicOr(&s_supm[vw], vbit); decided = true; }
-          else if (pendm == 0u) { atomicOr(&s_keptm[vw], vbit); decided = true; }
-        }
-        open = bar_or_chunk(!decided);
-        ++sweeps;
-      }
-      if (open) {
-        if (warp == 0) resolve_chunk_serially(&s_T[0][0], s_keptm, s_supm, ns);
-        bar_sync_chunk();
-      }
-      DAN_TOCK(3);
-    }
-    __syncthreads();
-    DAN_TICK();
-    // e. append the kept survivors in rank order; a kept box becomes the first hint of its cell unless an earlier
-    // (higher scoring) one is centred there.  ALL threads take part: kEntryThreads threads share one survivor, each
-    // enters the kept box into every kEntryThreads-th stripe of both axes (a big box touches 2 x 20 stripes: in the hands
-    // of the survivor's own thread alone this was the longest serial piece of a round).
-    {
-      constexpr int kEntryThreads = kSortThreads / kSurv;
-      const int v = tid / kEntryThreads, part = tid % kEntryThreads;
-      const int vw = v >> 5;
-      const uint32_t vbit = 1u << (v & 31);
-      if (tid < 2) s_next[tid] = 0;
-      if (tid == 2) s_nlist = 0;
-      if (v < ns && (s_keptm[vw] & vbit)) {
-        int before = 0;
-#pragma unroll
-        for (int w = 0; w < kSurvWords; ++w)
-          if (w < vw) before += __popc(s_keptm[w]);
-        const int pos = L + before + __popc(s_keptm[vw] & (vbit - 1u));
-        if (pos < A.nms_topk) {
-          const uint2 sm = s_smask[v];
-          const uint32_t bit = 1u << (pos & 31);
-          if (part == 0) {
-            const float4 bx = s_sbox[v];
-            kbox[pos] = bx;
-            karea[pos] = s_sarea[v];
-            krank[pos] = s_surv[v];
-            if (sm.x != 0u) atomicMin(&s_hint[0][sg.cell(bx)], pos);
-          }
-          for (int st = part; st < 32; st += kEntryThreads) {
-            if ((sm.x >> st) & 1u) atomicOr(&xs[st * wcap + (pos >> 5)], bit);
-            if ((sm.y >> st) & 1u) atomicOr(&ys[st * wcap + (pos >> 5)], bit);
-          }
-        }
-      }
-    }
-    __syncthreads();
-    {
-      int nk = 0;
-#pragma unroll
-      for (int w = 0; w < kSurvWords; ++w) nk += __popc(s_keptm[w]);
-      L_prev = L;
-      L = min(L + nk, A.nms_topk);
-    }
-    w_end_prev = w_end;
-    c0 = c_next;
-#ifdef DAN_PHASE_TIMING
-    DAN_TOCK(4);
-    n_sweeps += sweeps; n_surv += ns; ++n_chunks;
-#endif
-  }
-  const int kept_n = L;
-  DAN_PHASE(3);
-#ifdef DAN_PHASE_TIMING
-  if (threadIdx.x == 0 && blockIdx.x == 0) {
-    for (int i = 0; i < 5; ++i) g_phase[10 + i] = acc[i];
-    for (int i = 5; i < 12; ++i) g_phase[15 + i] = acc[i];
-    g_phase[15] = n_sweeps; g_phase[16] = n_surv; g_phase[17] = n_chunks; g_phase[18] = K; g_phase[19] = kept_n;
-  }
-#endif
+}
 
-  // ---- 4. outputs, zero padded to nms_topk; with a peer exchange every slab row also goes to the other ranks
+// ---- a. window vs kept list.  Thread t owns candidate c0 + t.  A candidate that was in the previous window has met
+// the first L_prev kept boxes already; a fresh one has met none.
+DAN_D void test_window(const PpArgs& A, const GreedyList& g, RoundSmem& R, int w_end) {
+  const int tid = threadIdx.x;
+  const int lane = tid & 31;
+  const unsigned lt_mask = (1u << lane) - 1u;
+  const float thr = A.nms_thr;
+  const int L = g.L, L_prev = g.L_prev, w_end_prev = g.w_end_prev, c0 = g.c0;
+  const int my_r = c0 + tid;
+  const bool in_win = my_r < w_end;
+  {
+    bool alive = false, search = false;
+    int upto = 0;
+    if (in_win) {
+      const bool fresh = my_r >= w_end_prev;
+      alive = fresh ? true : (R.alive[my_r & (kWin - 1)] != 0);
+      upto = fresh ? 0 : L_prev;
+    }
+    if (alive && L > upto) {
+      const uint2 mm = g.cmask[my_r];
+      if (mm.x != 0u && mm.y != 0u) {                  // (no area: no stripes, never suppressed)
+        // a1. the two hinted kept boxes of the cell of its centre: a member of a cluster of near duplicates dies here,
+        // after one or two exact tests by its own thread
+        const float4 me = g.cbox[my_r];
+        const float my_area = g.carea[my_r];
+        const int cl = g.sg.cell(me);
+        const int h0 = R.hint[0][cl], h1 = R.hint[1][cl];
+        bool dead = false;
+        if (h0 >= upto && h0 < L) dead = pair_suppresses(g.kbox[h0], g.karea[h0], me, my_area, thr);
+        if (!dead && h1 != h0 && h1 >= upto && h1 < L) dead = pair_suppresses(g.kbox[h1], g.karea[h1], me, my_area, thr);
+        alive = !dead;
+        search = !dead;
+      }
+    }
+    if (in_win) R.alive[my_r & (kWin - 1)] = alive ? 1 : 0;
+    const unsigned sm = __ballot_sync(0xffffffffu, search);
+    int base = 0;
+    if (lane == 0 && sm != 0u) base = atomicAdd(R.nlist, __popc(sm));
+    base = __shfl_sync(0xffffffffu, base, 0);
+    if (search) R.list[base + __popc(sm & lt_mask)] = (unsigned short)tid;
+  }
+  __syncthreads();
+  // a2. the others against the kept list proper, which is indexed by stripe: bit j of xs[s] / ys[s] says that kept box j
+  // touches x / y stripe s.  The kept boxes a candidate can intersect are (OR of xs over its x stripes) AND (OR of ys
+  // over its y stripes): a group of G lanes owns one candidate, a lane one 32-bit word of the bitset, and only the set
+  // bits (beyond the boxes the candidate has met already) go through the exact test; the candidate leaves at the
+  // first suppressor, which becomes the cell's second hint.
+  const int nlist = *R.nlist;
+  if (nlist > 0) {
+    const int wcap = g.wcap;
+    const int W = (L + 31) >> 5;
+    const int G = W <= 8 ? 8 : (W <= 16 ? 16 : 32);        // lanes per candidate
+    const int cpw = 32 / G;                                // candidates per warp pass
+    const int gl = lane & (G - 1), sub = lane / G;
+    const unsigned gmask = (G == 32 ? 0xffffffffu : ((1u << G) - 1u)) << (sub * G);
+    while (true) {                                         // candidates are handed out dynamically: their cost varies a lot
+      int i0 = 0;
+      if (lane == 0) i0 = atomicAdd(&R.next[0], cpw);
+      i0 = __shfl_sync(0xffffffffu, i0, 0);
+      if (i0 >= nlist) break;
+      const bool have = i0 + sub < nlist;
+      const int r = c0 + (have ? (int)R.list[i0 + sub] : 0);
+      const float4 me = have ? g.cbox[r] : make_float4(0.f, 0.f, 0.f, 0.f);
+      const float my_area = have ? g.carea[r] : 0.f;
+      const uint2 mm = have ? g.cmask[r] : make_uint2(0u, 0u);
+      const int upto = (r >= w_end_prev) ? 0 : L_prev;
+      bool sup = false;
+      for (int wb = 0; wb < W; wb += G) {                  // one block of words unless the kept list is very long
+        const int w = wb + gl;
+        uint32_t poss = 0u;
+        if (w < W && w >= (upto >> 5) && mm.x != 0u && mm.y != 0u) {
+          // (the stripes of a box are a contiguous range: independent loads, no address chain)
+          uint32_t ax = 0u, ay = 0u;
+          const int xe = 31 - __clz(mm.x), ye = 31 - __clz(mm.y);
+#pragma unroll 2
+          for (int st = __ffs(mm.x) - 1; st <= xe; ++st) ax |= g.xs[st * wcap + w];
+#pragma unroll 2
+          for (int st = __ffs(mm.y) - 1; st <= ye; ++st) ay |= g.ys[st * wcap + w];
+          poss = ax & ay;
+          if (w == (upto >> 5)) poss &= ~((1u << (upto & 31)) - 1u);
+        }
+        while (__any_sync(0xffffffffu, poss != 0u && !sup)) {
+          bool t = false;
+          if (poss != 0u && !sup) {
+            const int j = (w << 5) + __ffs(poss) - 1;
+            poss &= poss - 1u;
+            t = pair_suppresses(g.kbox[j], g.karea[j], me, my_area, thr);
+            if (t) atomicExch(&R.hint[1][g.sg.cell(me)], j);
+          }
+          if ((__ballot_sync(0xffffffffu, t) & gmask) != 0u) sup = true;
+        }
+      }
+      if (have && gl == 0 && sup) R.alive[r & (kWin - 1)] = 0;
+    }
+  }
+  __syncthreads();
+}
+
+// ---- b. the first kSurv candidates of the window that are still alive, in rank order; returns how many (ns) and sets
+// c_next, the start of the next round's window: behind the last of them
+DAN_D int compact_survivors(const GreedyList& g, RoundSmem& R, int w_end, int& c_next) {
+  __shared__ int s_wcnt[kSortThreads / 32];
+  __shared__ int s_cnext;
+  const int tid = threadIdx.x;
+  const int lane = tid & 31;
+  const int warp = tid >> 5;
+  const unsigned lt_mask = (1u << lane) - 1u;
+  const int my_r = g.c0 + tid;
+  const bool in_win = my_r < w_end;
+  const bool f = in_win && R.alive[my_r & (kWin - 1)] != 0;
+  const unsigned fm = __ballot_sync(0xffffffffu, f);
+  if (lane == 0) s_wcnt[warp] = __popc(fm);
+  if (tid < kSurvWords) { R.keptm[tid] = 0u; R.supm[tid] = 0u; }
+  __syncthreads();
+  int total, ubase;
+  {
+    const int cw = (lane < kSortThreads / 32) ? s_wcnt[lane] : 0;
+    int incl = cw;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const int up = __shfl_up_sync(0xffffffffu, incl, d);
+      if (lane >= d) incl += up;
+    }
+    total = __shfl_sync(0xffffffffu, incl, 31);
+    ubase = __shfl_sync(0xffffffffu, incl - cw, warp & 31);
+  }
+  if (f) {
+    const int u = ubase + __popc(fm & lt_mask);
+    if (u < kSurv) {
+      R.surv[u] = my_r;
+      R.sbox[u] = g.cbox[my_r];
+      R.sarea[u] = g.carea[my_r];
+      R.smask[u] = g.cmask[my_r];
+      if (u == kSurv - 1) s_cnext = my_r + 1;
+    }
+  }
+  __syncthreads();
+  c_next = (total >= kSurv) ? s_cnext : w_end;
+  return min(total, kSurv);
+}
+
+// ---- c. suppression bits among the ns survivors: warp -> row v, lanes -> 32 earlier survivors per step
+DAN_D void survivor_bits(const PpArgs& A, RoundSmem& R, int ns) {
+  const int lane = threadIdx.x & 31;
+  const float thr = A.nms_thr;
+  while (true) {                                           // rows handed out dynamically, the longest ones first
+    int vi = 0;
+    if (lane == 0) vi = atomicAdd(&R.next[1], 1);
+    vi = __shfl_sync(0xffffffffu, vi, 0);
+    if (vi >= ns) break;
+    const int v = ns - 1 - vi;
+    const float4 me = R.sbox[v];
+    const float my_area = R.sarea[v];
+    const uint2 mm = R.smask[v];
+    const int nw = (v + 31) >> 5;                    // words that hold some u < v
+    for (int w = 0; w < nw; ++w) {
+      const int u = (w << 5) + lane;
+      const uint2 um = R.smask[u];
+      const bool poss = (u < v) && (um.x & mm.x) != 0u && (um.y & mm.y) != 0u;
+      unsigned bits = 0u;
+      if (__any_sync(0xffffffffu, poss)) {
+        const bool t = poss && pair_suppresses(R.sbox[u], R.sarea[u], me, my_area, thr);
+        bits = __ballot_sync(0xffffffffu, t);
+      }
+      if (lane == 0) R.T[v][w] = bits;
+    }
+  }
+  __syncthreads();
+}
+
+// ---- d. relaxation, kept(v) = no kept u in T[v]: thread v owns survivor v (the first kSurv threads).  A survivor is
+// decided once one of its suppressors is known kept, or all are known suppressed; chains longer than kMaxSweeps are
+// finished by resolve_chunk_serially.
+DAN_D void relax_survivors(RoundSmem& R, int ns) {
+  const int tid = threadIdx.x;
+  const int warp = tid >> 5;
+  if (tid < kSurv) {
+    uint32_t trow[kSurvWords];
+    const int vw = tid >> 5;
+    const uint32_t vbit = 1u << (tid & 31);
+    const bool mine = tid < ns;
+#pragma unroll
+    for (int w = 0; w < kSurvWords; ++w) trow[w] = (mine && (w << 5) < tid) ? R.T[tid][w] : 0u;
+    bool decided = !mine;
+    bool open = true;
+    int sweeps = 0;
+    while (open && sweeps < kMaxSweeps) {
+      uint32_t hitm = 0u, pendm = 0u;
+      if (!decided) {
+#pragma unroll
+        for (int w = 0; w < kSurvWords; ++w) {
+          const uint32_t kw = R.keptm[w], sw = R.supm[w];
+          hitm |= trow[w] & kw;
+          pendm |= trow[w] & ~(kw | sw);
+        }
+      }
+      bar_sync_chunk();                              // every thread has read the masks of the previous sweep
+      if (!decided) {
+        if (hitm != 0u) { atomicOr(&R.supm[vw], vbit); decided = true; }
+        else if (pendm == 0u) { atomicOr(&R.keptm[vw], vbit); decided = true; }
+      }
+      open = bar_or_chunk(!decided);
+      ++sweeps;
+    }
+    if (open) {
+      if (warp == 0) resolve_chunk_serially(&R.T[0][0], R.keptm, R.supm, ns);
+      bar_sync_chunk();
+    }
+  }
+  __syncthreads();
+}
+
+// ---- e. append the kept survivors in rank order; a kept box becomes the first hint of its cell unless an earlier
+// (higher scoring) one is centred there.  ALL threads take part: kEntryThreads threads share one survivor, each
+// enters the kept box into every kEntryThreads-th stripe of both axes (a big box touches 2 x 20 stripes: in the hands
+// of the survivor's own thread alone this was the longest serial piece of a round).  Then L counts them.
+DAN_D void append_kept(const PpArgs& A, GreedyList& g, RoundSmem& R, int ns) {
+  const int tid = threadIdx.x;
+  const int L = g.L;
+  {
+    constexpr int kEntryThreads = kSortThreads / kSurv;
+    const int v = tid / kEntryThreads, part = tid % kEntryThreads;
+    const int vw = v >> 5;
+    const uint32_t vbit = 1u << (v & 31);
+    if (tid < 2) R.next[tid] = 0;
+    if (tid == 2) *R.nlist = 0;
+    if (v < ns && (R.keptm[vw] & vbit)) {
+      int before = 0;
+#pragma unroll
+      for (int w = 0; w < kSurvWords; ++w)
+        if (w < vw) before += __popc(R.keptm[w]);
+      const int pos = L + before + __popc(R.keptm[vw] & (vbit - 1u));
+      if (pos < A.nms_topk) {
+        const uint2 sm = R.smask[v];
+        const uint32_t bit = 1u << (pos & 31);
+        if (part == 0) {
+          const float4 bx = R.sbox[v];
+          g.kbox[pos] = bx;
+          g.karea[pos] = R.sarea[v];
+          g.krank[pos] = R.surv[v];
+          if (sm.x != 0u) atomicMin(&R.hint[0][g.sg.cell(bx)], pos);
+        }
+        for (int st = part; st < 32; st += kEntryThreads) {
+          if ((sm.x >> st) & 1u) atomicOr(&g.xs[st * g.wcap + (pos >> 5)], bit);
+          if ((sm.y >> st) & 1u) atomicOr(&g.ys[st * g.wcap + (pos >> 5)], bit);
+        }
+      }
+    }
+  }
+  __syncthreads();
+  int nk = 0;
+#pragma unroll
+  for (int w = 0; w < kSurvWords; ++w) nk += __popc(R.keptm[w]);
+  g.L_prev = L;
+  g.L = min(L + nk, A.nms_topk);
+}
+
+// ---- 4. outputs, zero padded to nms_topk; with a peer exchange every slab row also goes to the other ranks
+template <bool DECODE>
+DAN_D void write_outputs(const PpArgs& A, int list, int64_t o, const GreedyList& g, const float* src_scores, const float4* src_boxes) {
+  const int tid = threadIdx.x;
+  const int kept_n = g.L;
   auto put_score = [&](int64_t oo, float v) {
     A.out_scores[oo] = v;
     for (int q = 0; q < A.npeers; ++q) *reinterpret_cast<float*>(reinterpret_cast<char*>(A.out_scores + oo) + A.peer_delta[q]) = v;
@@ -1043,11 +1039,11 @@ __global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __
   for (int t = tid; t < A.nms_topk; t += kSortThreads) {
     const int64_t oo = (int64_t)list * A.nms_topk + t;
     if (t < kept_n) {
-      const int pos = krank[t];
+      const int pos = g.krank[t];
       const unsigned long long key = A.s_key[o + pos];
       const uint32_t idx = key_index(key);
       put_score(oo, DECODE ? key_to_score((uint32_t)(key >> 32)) : src_scores[idx]);
-      put_box(oo, DECODE ? kbox[t] : src_boxes[idx]);     // clipped boxes are already min/max ordered
+      put_box(oo, DECODE ? g.kbox[t] : src_boxes[idx]);     // clipped boxes are already min/max ordered
       if (A.out_index != nullptr) A.out_index[oo] = (int32_t)idx;
       if (A.out_keep != nullptr) A.out_keep[oo] = A.filler ? pos : (int32_t)idx;
     } else {
@@ -1057,7 +1053,7 @@ __global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __
       if (A.out_keep != nullptr) {
         // parse_by_class runs NMS on the zero padded top-k list: zero-area filler rows are never suppressed
         // and get selected until nms_topk is reached
-        const int fpos = K + (t - kept_n);
+        const int fpos = g.K + (t - kept_n);
         A.out_keep[oo] = (A.filler && fpos < A.keep_topk) ? fpos : -1;
       }
     }
@@ -1066,23 +1062,70 @@ __global__ void DAN_NMS_BOUNDS nms_greedy_kernel(const PpArgs A, const float* __
     A.out_counts[list] = kept_n;
     for (int q = 0; q < A.npeers; ++q) *reinterpret_cast<int32_t*>(reinterpret_cast<char*>(A.out_counts + list) + A.peer_delta[q]) = kept_n;
   }
-  if (A.npeers > 0) {
-    // release: this CTA's rows are visible system-wide before it counts itself done; the last CTA of the launch bumps the
-    // rank's step number and writes it into its flag slot in every destination (dan_wait_detections polls those)
-    __threadfence_system();
-    __syncthreads();
-    if (tid == 0) {
-      const int done = atomicAdd(A.peer_state, 1);
-      if (done == (int)gridDim.x - 1) {
-        A.peer_state[0] = 0;
-        const int seq = A.peer_state[1] + 1;
-        A.peer_state[1] = seq;
-        __threadfence_system();
-        for (int q = 0; q < A.npeers; ++q) *reinterpret_cast<volatile int32_t*>(A.peer_flag[q]) = seq;
-      }
+}
+
+// release (peer exchange): this CTA's rows are visible system-wide before it counts itself done; the last CTA of the
+// launch bumps the rank's step number and writes it into its flag slot in every destination (dan_wait_detections polls
+// those)
+DAN_D void release_peers(const PpArgs& A) {
+  __threadfence_system();
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    const int done = atomicAdd(A.peer_state, 1);
+    if (done == (int)gridDim.x - 1) {
+      A.peer_state[0] = 0;
+      const int seq = A.peer_state[1] + 1;
+      A.peer_state[1] = seq;
+      __threadfence_system();
+      for (int q = 0; q < A.npeers; ++q) *reinterpret_cast<volatile int32_t*>(A.peer_flag[q]) = seq;
     }
   }
-  DAN_PHASE(4);
+}
+
+// T: element type of the predictions (DECODE only; the standalone sort / NMS instantiations take fp32 scores and boxes)
+template <bool DECODE, int WHERE, bool FILTER, typename T>
+__global__ void __launch_bounds__(kSortThreads, 1) nms_greedy_kernel(const PpArgs A, const float* __restrict__ src_scores,
+                                                                     const float4* __restrict__ src_boxes) {
+  extern __shared__ __align__(16) unsigned char dyn_smem[];
+  // (separate arrays: one __shared__ RoundSmem-shaped struct would be padded, 16 B more static shared memory)
+  __shared__ unsigned char s_alive[kWin];
+  __shared__ unsigned short s_list[kWin];
+  __shared__ int s_surv[kSurv];
+  __shared__ float4 s_sbox[kSurv];
+  __shared__ float s_sarea[kSurv];
+  __shared__ uint32_t s_T[kSurv][kSurvWords];
+  __shared__ uint32_t s_keptm[kSurvWords], s_supm[kSurvWords];
+  __shared__ uint2 s_smask[kSurv];
+  __shared__ int s_hint[2][kHintCells];
+  __shared__ int s_next[2];
+  __shared__ int s_nlist;
+  RoundSmem R = {s_alive, s_list, s_surv, s_sbox, s_sarea, s_smask, s_T, s_keptm, s_supm, s_hint, s_next, &s_nlist};
+
+  const int list = blockIdx.x;
+  const int b = list / max(A.num_classes - 1, 1);
+  const int64_t o = (int64_t)list * A.plan.slots;
+  unsigned long long* keys = reinterpret_cast<unsigned long long*>(dyn_smem);
+  unsigned long long* gkeys = A.keys + (int64_t)list * A.n;
+  GreedyList g = carve<WHERE>(A, dyn_smem, list);
+
+  const int cnt = FILTER ? filter_image<T>(A, list, b, keys, gkeys) : min(A.key_count[list], A.n);
+  const unsigned long long* sorted;
+  g.K = top_k_sort<FILTER>(A, cnt, o, gkeys, keys, dyn_smem, sorted);
+  decode_candidates<DECODE, T>(A, b, o, sorted, src_boxes, g);
+  init_stripes(A, g, R);
+  while (g.c0 < g.K && g.L < A.nms_topk) {
+    const int w_end = min(g.K, g.c0 + kWin);
+    test_window(A, g, R, w_end);
+    int c_next;
+    const int ns = compact_survivors(g, R, w_end, c_next);
+    survivor_bits(A, R, ns);
+    relax_survivors(R, ns);
+    append_kept(A, g, R, ns);
+    g.w_end_prev = w_end;
+    g.c0 = c_next;
+  }
+  write_outputs<DECODE>(A, list, o, g, src_scores, src_boxes);
+  if (A.npeers > 0) release_peers(A);
 }
 
 // One warp polls the arrival flags of the `world` ranks in this rank's receive buffer until all have reached the step
@@ -1109,7 +1152,7 @@ static PpLayout pp_layout(int64_t n, int64_t lists, int64_t keep_topk, bool nms,
   PpLayout w;
   size_t off = 0;
   auto take = [&](size_t bytes) { const size_t at = off; off += align_up(bytes, 256); return at; };
-  const int64_t ks = keep_topk < n ? keep_topk : (n > 0 ? n : 1);      // kstride
+  const int64_t ks = cand_slots(n, keep_topk);
   w.key_count = take(lists * 4);
   w.keys = take(lists * n * 8);
   w.maybe = take(nms ? lists * n * 4 : 0);
@@ -1146,9 +1189,9 @@ static void pp_bind(PpArgs& A, void* ws, const PpLayout& w) {
 // opt-in to > 48 KB of dynamic shared memory; the attribute belongs to the (function, device) pair, so it is set on
 // every call (a few hundred ns of host time) rather than cached in a process-wide flag
 template <bool DECODE, int WHERE, bool FILTER, typename T>
-static int launch_greedy(const PpArgs& A, int lists, size_t smem, const float* src_scores, const float4* src_boxes, cudaStream_t st) {
-  DAN_CUDA(cudaFuncSetAttribute(nms_greedy_kernel<DECODE, WHERE, FILTER, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  nms_greedy_kernel<DECODE, WHERE, FILTER, T><<<lists, kSortThreads, smem, st>>>(A, src_scores, src_boxes);
+static int launch_greedy(const PpArgs& A, int lists, const float* src_scores, const float4* src_boxes, cudaStream_t st) {
+  DAN_CUDA(cudaFuncSetAttribute(nms_greedy_kernel<DECODE, WHERE, FILTER, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, A.plan.smem));
+  nms_greedy_kernel<DECODE, WHERE, FILTER, T><<<lists, kSortThreads, A.plan.smem, st>>>(A, src_scores, src_boxes);
   DAN_LAUNCH_CHECK("nms_greedy_kernel");
   return DAN_OK;
 }
@@ -1157,17 +1200,10 @@ static int launch_greedy(const PpArgs& A, int lists, size_t smem, const float* s
 template <bool DECODE, bool FILTER, typename T>
 static int run_sort_nms(const PpArgs& A_in, int lists, const float* src_scores, const float4* src_boxes, cudaStream_t st) {
   PpArgs A = A_in;
-  const GreedyPlan g = greedy_plan(A.n, A.keep_topk, A.nms_cap);
-  A.sort_bytes = g.sort_bytes;
-  A.kcap = g.kcap;
-  A.wcap = g.wcap;
-  A.kstride = g.kcap;
-  A.dyn_smem_bytes = (int)g.smem;
-  A.cand_global = g.cand_global;
-  A.kept_global = g.kept_global;
-  if (g.kept_global) return launch_greedy<DECODE, 2, FILTER, T>(A, lists, g.smem, src_scores, src_boxes, st);
-  if (g.cand_global) return launch_greedy<DECODE, 1, FILTER, T>(A, lists, g.smem, src_scores, src_boxes, st);
-  return launch_greedy<DECODE, 0, FILTER, T>(A, lists, g.smem, src_scores, src_boxes, st);
+  A.plan = greedy_plan(A.n, A.keep_topk, A.nms_cap);
+  if (A.plan.where == 2) return launch_greedy<DECODE, 2, FILTER, T>(A, lists, src_scores, src_boxes, st);
+  if (A.plan.where == 1) return launch_greedy<DECODE, 1, FILTER, T>(A, lists, src_scores, src_boxes, st);
+  return launch_greedy<DECODE, 0, FILTER, T>(A, lists, src_scores, src_boxes, st);
 }
 
 // the launches of one postprocess call: [filter kernel +] the per-list NMS kernel, with T the prediction type
@@ -1192,10 +1228,6 @@ static int postprocess_launch(const PpArgs& A, bool fused, int lists, cudaStream
 using namespace dan;
 
 extern "C" {
-
-#ifdef DAN_PHASE_TIMING
-int dan_debug_phases(long long* h_out32) { return cudaMemcpyFromSymbol(h_out32, g_phase, sizeof(long long) * 32) == cudaSuccess ? 0 : -3; }
-#endif
 
 size_t dan_postprocess_workspace_bytes(int32_t num_anchors, int32_t batch, int32_t num_classes, int32_t keep_topk) {
   if (num_anchors < 0 || batch < 0 || num_classes < 2 || keep_topk < 1) return 0;

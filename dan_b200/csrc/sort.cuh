@@ -1,17 +1,9 @@
 // Block-wide top-k + sort of 64-bit keys in shared memory (1024-thread CTAs), shared by the postprocess and the
-// evaluation-merge kernels.  Include it INSIDE `namespace dan { ... }` of a .cu file, after common.cuh (the optional
-// DAN_PHASE timing macro of the including file is used when it is defined).
+// evaluation-merge kernels.  Include it INSIDE `namespace dan { ... }` of a .cu file, after common.cuh.
 #pragma once
 
-#ifndef DAN_PHASE
-#define DAN_PHASE(slot) do { } while (0)
-#endif
-
 constexpr int kSortCap = 8192;      // keys sorted in shared memory (64 KB)
-#ifndef DAN_SORT_THREADS
-#define DAN_SORT_THREADS 1024          // threads per CTA of the including file's sort kernels (a power of two >= 256)
-#endif
-constexpr int kSortThreads = DAN_SORT_THREADS;
+constexpr int kSortThreads = 1024;  // threads per CTA of the sort kernels
 
 // order-preserving float <-> uint32 (descending key order = descending score)
 DAN_D uint32_t score_to_key(float s) { return (uint32_t)float_to_ordered(s) ^ 0x80000000u; }
@@ -119,15 +111,12 @@ DAN_D void sort_smem_keys(unsigned long long* s_keys, int m) {
   for (int i = m + tid; i < p2; i += kSortThreads) s_keys[i] = 0ull;
   __syncthreads();
   if (lp2 >= 5) {            // (at least one full warp of owners)
-    // keys per thread: the smallest power of two that lets kSortThreads threads own all 2^lp2 keys
-    constexpr int kLogThreads = kSortThreads == 1024 ? 10 : kSortThreads == 512 ? 9 : 8;
-    const int lk = lp2 > kLogThreads ? lp2 - kLogThreads : 0;
+    // keys per thread: the smallest power of two that lets the 1024 threads own all 2^lp2 <= kSortCap keys
+    const int lk = lp2 > 10 ? lp2 - 10 : 0;
     if (lk == 0) bitonic_sort_regs<1>(s_keys, lp2);
     else if (lk == 1) bitonic_sort_regs<2>(s_keys, lp2);
     else if (lk == 2) bitonic_sort_regs<4>(s_keys, lp2);
     else if (lk == 3) bitonic_sort_regs<8>(s_keys, lp2);
-    else if (lk == 4) { if constexpr (kSortThreads < 1024) bitonic_sort_regs<16>(s_keys, lp2); }
-    else { if constexpr (kSortThreads < 512) bitonic_sort_regs<32>(s_keys, lp2); }
     return;
   }
   // small lists: plain bitonic sort in shared memory, descending; strides are powers of two -> shifts only
@@ -266,10 +255,6 @@ DAN_D int select_and_sort(const unsigned long long* __restrict__ keys, int cnt, 
     }
     m = k;
   }
-  DAN_PHASE(8);
-#ifdef DAN_NO_MERGE_SORT
-  s_spare = nullptr;
-#endif
   if (s_spare != nullptr && m > 128) {
     __syncthreads();
     merge_sort_smem_keys(s_keys, s_spare, m);
