@@ -131,6 +131,9 @@ _SIGNATURES = {
                                                        c_vp, c_vp, c_vp, c_sz, c_vp]),
     "dan_detect_face_workspace_bytes": (c_sz, [c_i64]),
     "dan_detect_face_select": (ctypes.c_int, [c_vp, c_vp, c_i64, c_f32, c_i32, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "dan_detect_face_batch_workspace_bytes": (c_sz, [c_i64, c_i32]),
+    "dan_detect_face_batch": (ctypes.c_int, [c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i32, ctypes.POINTER(c_f32), c_f32,
+                                             c_i32, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "dan_bbox_vote": (ctypes.c_int, [c_vp, c_vp, c_i32, c_i32, c_f32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "dan_gt_handoff": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_f32, c_f32, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp,
                                       c_vp]),

@@ -164,6 +164,15 @@ DAN_D float cephes_logf(float x) {
   return m;
 }
 
+// tf.nn.softmax of two logits, column 1 (the face probability): exp(x - max) * (1 / sum(exp(x - max))), sum in class
+// order - bit for bit the column 1 of dan_softmax with two classes
+DAN_D float softmax2_face(float x0, float x1) {
+  const float mx = fmaxf(x0, x1);
+  const float e0 = cephes_expf(fsub(x0, mx));
+  const float e1 = cephes_expf(fsub(x1, mx));
+  return fmul(e1, fdiv(1.f, fadd(e0, e1)));
+}
+
 // decode one box, anchor_manipulator.py:399-408 / :417-424
 DAN_D float4 decode_box(float4 p, float ay0, float ax0, float ay1, float ax1, float ps0, float ps1,
                         float ps2, float ps3) {

@@ -665,11 +665,7 @@ DAN_D int filter_image(const PpArgs& A, int list, int b, unsigned long long* key
     if (i < nmaybe) {
       const int a = (i < kMaybeCap) ? s_maybe[i] : gmaybe[i];
       const float2 xx = ld_pair(x + 2 * a);
-      // tf.nn.softmax: exp(x - max) * (1 / sum(exp(x - max))), sum in class order
-      const float mx = fmaxf(xx.x, xx.y);
-      const float e0 = cephes_expf(fsub(xx.x, mx));
-      const float e1 = cephes_expf(fsub(xx.y, mx));
-      const float pr = fmul(e1, fdiv(1.f, fadd(e0, e1)));
+      const float pr = softmax2_face(xx.x, xx.y);
       if (pr > A.select_thr) {                            // select_bboxes :24-36
         const float4 box = pp_box<T>(A, b, a);
         if (A.stash != nullptr) A.stash[(int64_t)b * A.n + a] = box;

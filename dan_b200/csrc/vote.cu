@@ -430,43 +430,222 @@ __global__ void __launch_bounds__(kSortThreads, 1) bbox_vote_kernel(const VoteAr
   }
 }
 
-struct FaceArgs {
-  const float4* boxes;        // [n] (ymin, xmin, ymax, xmax)
-  const float* scores;        // [n]
-  int n;
-  float shrink;
-  int top;                    // int(1.5 * max_per_image)
-  unsigned long long* keys;   // [n] workspace
-  float* out;                 // [top, 5] zero padded
-  int32_t* out_index;         // [top] optional, -1 padded
-  int32_t* out_count;
-};
+// detect_face (eval_sfd.py:95-114) for B images of N anchors, in two kernels:
+//   face_key_kernel     grid-wide over B x N: key = score bits << 32 | anchor (equal scores: higher anchor first), and a
+//                       per-image histogram of the keys' face_bin() (shared-memory histogram per CTA, flushed with one
+//                       global atomic per non-empty bin)
+//   face_select_kernel  one CTA per image: the histogram gives the bin that holds the k-th key; one pass over the image's
+//                       keys compacts those in that bin or above into shared memory, where they are sorted.  Only the k
+//                       rows are read (or decoded from the offsets), divided by shrink and written.
+// The score comes from the scores of decoded boxes (dan_detect_face_select) or from the two logits (the softmax in
+// tf.nn.softmax's op order, dan_detect_face_batch); the box from a decoded row or from a decode of the offset row.
+constexpr int kFaceBins = 4096;             // histogram bins per image
+constexpr int kFaceKeyThreads = 512;
+constexpr int kFaceChunk = 8 * kFaceKeyThreads;   // anchors per CTA of the key kernel
 
-__global__ void __launch_bounds__(256) face_key_kernel(const FaceArgs A) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += gridDim.x * blockDim.x)
-    A.keys[i] = ((unsigned long long)score_to_key(A.scores[i]) << 32) | (unsigned long long)(uint32_t)i;
+// A monotone map of a key to [0, kFaceBins): keys in a higher bin are larger.  Half of the bins cut the probabilities
+// [0.5, 1) into steps of 2^-12 (confident detections crowd there), the other half cover [2^-17, 0.5) at 128 bins per
+// octave; smaller scores (and negative ones) share bin 0, larger ones (and NaN) the last bin.
+DAN_D int face_bin(unsigned long long key) {
+  const uint32_t x = (uint32_t)(key >> 32);
+  constexpr uint32_t kHalf = 0xBF000000u;                  // score_to_key(0.5f)
+  if (x >= kHalf) return kFaceBins / 2 + (int)min((x - kHalf) >> 12, (uint32_t)(kFaceBins / 2 - 1));
+  return max((int)(x >> 16) - (int)((kHalf >> 16) - kFaceBins / 2), 0);
 }
 
-// eval_sfd.py:101-112
-__global__ void __launch_bounds__(kSortThreads, 1) face_select_kernel(const FaceArgs A) {
-  extern __shared__ unsigned long long s_keys[];
+struct FaceScores {                         // scores of decoded boxes, [B, N] fp32
+  const float* s;
+  DAN_D float score(int64_t row) const { return s[row]; }
+};
+
+template <typename T> struct FaceLogits {   // two logits per anchor, [B, N, 2]
+  const T* x;
+  bool pair_aligned;                        // false: a pair is not aligned for one load (read as two scalars)
+  DAN_D float score(int64_t row) const {
+    const float2 v = pair_aligned ? ld_pair(x + 2 * row) : make_float2(widen(x[2 * row]), widen(x[2 * row + 1]));
+    return softmax2_face(v.x, v.y);
+  }
+};
+
+struct FaceBoxes {                          // decoded boxes, [B, N, 4] (ymin, xmin, ymax, xmax)
+  const float4* boxes;
+  DAN_D float4 box(int64_t row, int) const { return boxes[row]; }
+};
+
+template <typename T> struct FaceOffsets {  // offsets [B, N, 4] (cy, cx, h, w), decoded like dan_decode_batch
+  const typename PredRow<T>::type* loc;
+  const float *ay0, *ax0, *ay1, *ax1;
+  float ps0, ps1, ps2, ps3;
+  DAN_D float4 box(int64_t row, int a) const {
+    return decode_box(PredRow<T>::widen(loc[row]), ay0[a], ax0[a], ay1[a], ax1[a], ps0, ps1, ps2, ps3);
+  }
+};
+
+struct FaceArgs {
+  int n;                      // anchors per image
+  int chunks;                 // CTAs of the key kernel per image
+  float shrink;
+  int top;                    // int(1.5 * max_per_image)
+  int k;                      // rows per image: max(min(n - 1, top), 0)
+  unsigned long long* keys;   // [B, n] workspace
+  int* hist;                  // [B, kFaceBins] workspace, zeroed before the key kernel
+  float* out;                 // [B, top, 5] zero padded
+  int32_t* out_index;         // [B, top] optional, -1 padded
+  int32_t* out_count;         // [1] optional (the single-image entry point)
+};
+
+template <class Score>
+__global__ void __launch_bounds__(kFaceKeyThreads) face_key_kernel(const FaceArgs A, const Score S) {
+  __shared__ int s_hist[kFaceBins];
+  const int tid = threadIdx.x, lane = tid & 31;
+  const int b = blockIdx.x / A.chunks;
+  const int a0 = (blockIdx.x - b * A.chunks) * kFaceChunk;
+  for (int i = tid; i < kFaceBins; i += kFaceKeyThreads) s_hist[i] = 0;
+  __syncthreads();
+  const int64_t row0 = (int64_t)b * A.n;
+#pragma unroll 4
+  for (int j = 0; j < kFaceChunk / kFaceKeyThreads; ++j) {
+    const int a = a0 + j * kFaceKeyThreads + tid;
+    int bin = -1;
+    if (a < A.n) {
+      const unsigned long long key = ((unsigned long long)score_to_key(S.score(row0 + a)) << 32) | (unsigned long long)(uint32_t)a;
+      A.keys[row0 + a] = key;
+      bin = face_bin(key);
+    }
+    const unsigned same = __match_any_sync(0xffffffffu, bin);         // one shared atomic per bin and warp
+    if (bin >= 0 && lane == __ffs(same) - 1) atomicAdd(&s_hist[bin], __popc(same));
+  }
+  __syncthreads();
+  int* hist = A.hist + (int64_t)b * kFaceBins;
+  for (int i = tid; i < kFaceBins; i += kFaceKeyThreads)
+    if (s_hist[i] != 0) atomicAdd(&hist[i], s_hist[i]);
+}
+
+// eval_sfd.py:101-112, one CTA per image
+template <class Box>
+__global__ void __launch_bounds__(kSortThreads, 1) face_select_kernel(const FaceArgs A, const Box src) {
+  extern __shared__ unsigned long long s_keys[];           // [kSortCap] keys | [kSortCap] merge buffer
   __shared__ SortScratch sc;
-  const int tid = threadIdx.x;
-  const int k = max(min(A.n - 1, A.top), 0);          // N == 0: the reference slices [:-1] of an empty array
-  if (k > 0) select_and_sort(A.keys, A.n, k, s_keys, sc);
+  __shared__ int s_warp[kSortThreads / 32];
+  __shared__ int s_bin, s_ge;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int b = blockIdx.x;
+  const int k = A.k;
+  const unsigned long long* keys = A.keys + (int64_t)b * A.n;
+  if (k > 0) {
+    // the bin t of the k-th largest key: thread i holds bins 4i .. 4i + 3, `above` counts the keys in higher bins
+    constexpr int kPer = kFaceBins / kSortThreads;
+    const int* hist = A.hist + (int64_t)b * kFaceBins + kPer * tid;
+    const int hb[kPer] = {hist[0], hist[1], hist[2], hist[3]};
+    const int c = hb[0] + hb[1] + hb[2] + hb[3];
+    int incl = c;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const int v = __shfl_down_sync(0xffffffffu, incl, d);
+      if (lane + d < 32) incl += v;
+    }
+    if (lane == 0) s_warp[warp] = incl;
+    if (tid == 0) sc.fill = 0;
+    __syncthreads();
+    int above = incl - c;
+    for (int w = warp + 1; w < kSortThreads / 32; ++w) above += s_warp[w];
+    if (above < k && above + c >= k) {                     // exactly one thread: the bins hold all n > k keys
+      int cum = above, t = kPer * tid;
+      for (int j = kPer - 1; j >= 0; --j) {
+        cum += hb[j];
+        if (cum >= k) { t = kPer * tid + j; break; }
+      }
+      s_bin = t;
+      s_ge = cum;
+    }
+    __syncthreads();
+    const int t = s_bin, ge = s_ge;
+    if (ge <= kSortCap) {
+      // one pass: the ge keys in bin t or above (a superset of the top k) into shared memory, one atomic per warp
+      for (int i0 = 0; i0 < A.n; i0 += 4 * kSortThreads) {
+        unsigned long long q[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          const int i = i0 + u * kSortThreads + tid;
+          q[u] = i < A.n ? __ldcs(keys + i) : 0ull;
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          const bool keep = i0 + u * kSortThreads + tid < A.n && face_bin(q[u]) >= t;
+          const unsigned m = __ballot_sync(0xffffffffu, keep);
+          if (m != 0u) {
+            int base = 0;
+            if (lane == 0) base = atomicAdd(&sc.fill, __popc(m));
+            base = __shfl_sync(0xffffffffu, base, 0);
+            if (keep) s_keys[base + __popc(m & ((1u << lane) - 1u))] = q[u];
+          }
+        }
+      }
+      __syncthreads();
+      select_and_sort(keys, ge, k, s_keys, sc, true, s_keys + kSortCap);
+    } else {
+      // more keys share the k-th key's bin than shared memory holds: radix select over all of the image's keys
+      select_and_sort(keys, A.n, k, s_keys, sc, false, s_keys + kSortCap);
+    }
+  }
+  float* out = A.out + (int64_t)b * A.top * 5;
   for (int r = tid; r < A.top; r += kSortThreads) {
     float o0 = 0.f, o1 = 0.f, o2 = 0.f, o3 = 0.f, o4 = 0.f;
     int idx = -1;
     if (r < k) {
-      idx = (int)(uint32_t)(s_keys[r] & 0xFFFFFFFFull);
-      const float4 bx = A.boxes[idx];
+      const unsigned long long key = s_keys[r];
+      idx = (int)(uint32_t)(key & 0xFFFFFFFFull);
+      const float4 bx = src.box((int64_t)b * A.n + idx, idx);
       o0 = fdiv(bx.y, A.shrink); o1 = fdiv(bx.x, A.shrink); o2 = fdiv(bx.w, A.shrink); o3 = fdiv(bx.z, A.shrink);
-      o4 = A.scores[idx];
+      o4 = key_to_score((uint32_t)(key >> 32));           // the score's bits, NaN payloads included
     }
-    A.out[r * 5] = o0; A.out[r * 5 + 1] = o1; A.out[r * 5 + 2] = o2; A.out[r * 5 + 3] = o3; A.out[r * 5 + 4] = o4;
-    if (A.out_index) A.out_index[r] = idx;
+    out[r * 5] = o0; out[r * 5 + 1] = o1; out[r * 5 + 2] = o2; out[r * 5 + 3] = o3; out[r * 5 + 4] = o4;
+    if (A.out_index) A.out_index[(int64_t)b * A.top + r] = idx;
   }
-  if (tid == 0) A.out_count[0] = k;
+  if (tid == 0 && A.out_count) A.out_count[b] = k;
+}
+
+constexpr size_t kFaceSelectSmem = 2 * kSortCap * sizeof(unsigned long long);
+
+static size_t face_hist_bytes(int32_t batch) { return align_up((size_t)batch * kFaceBins * sizeof(int), 256); }
+
+template <class Score, class Box>
+static int face_launch(const Score& score, const Box& box, int64_t n, int32_t batch, float shrink, int32_t top, float* out_det,
+                       int32_t* out_index, int32_t* out_count, void* workspace, cudaStream_t st) {
+  FaceArgs A = {};
+  A.n = (int)n;
+  A.chunks = (int)((n + kFaceChunk - 1) / kFaceChunk);
+  A.shrink = shrink;
+  A.top = top;
+  A.k = (int)(n - 1 < top ? (n - 1 > 0 ? n - 1 : 0) : top);    // N == 0: the reference slices [:-1] of an empty array
+  A.hist = static_cast<int*>(workspace);
+  A.keys = reinterpret_cast<unsigned long long*>(static_cast<unsigned char*>(workspace) + face_hist_bytes(batch));
+  A.out = out_det;
+  A.out_index = out_index;
+  A.out_count = out_count;
+  if (A.k > 0) {
+    DAN_CUDA(cudaMemsetAsync(A.hist, 0, (size_t)batch * kFaceBins * sizeof(int), st));
+    face_key_kernel<Score><<<(unsigned)((int64_t)A.chunks * batch), kFaceKeyThreads, 0, st>>>(A, score);
+    DAN_LAUNCH_CHECK("face_key_kernel");
+  }
+  DAN_CUDA(cudaFuncSetAttribute(face_select_kernel<Box>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFaceSelectSmem));
+  face_select_kernel<Box><<<batch, kSortThreads, kFaceSelectSmem, st>>>(A, box);
+  DAN_LAUNCH_CHECK("face_select_kernel");
+  return DAN_OK;
+}
+
+template <typename T>
+static int face_batch_launch(const void* cls_pred, const void* loc_pred, const float* a_ymin, const float* a_xmin, const float* a_ymax,
+                             const float* a_xmax, int64_t n, int32_t batch, const float* ps, float shrink, int32_t top, float* out_det,
+                             int32_t* out_index, void* workspace, cudaStream_t st) {
+  FaceLogits<T> score;
+  score.x = static_cast<const T*>(cls_pred);
+  score.pair_aligned = (reinterpret_cast<uintptr_t>(cls_pred) & (2 * sizeof(T) - 1)) == 0;
+  FaceOffsets<T> box;
+  box.loc = static_cast<const typename PredRow<T>::type*>(loc_pred);
+  box.ay0 = a_ymin; box.ax0 = a_xmin; box.ay1 = a_ymax; box.ax1 = a_xmax;
+  box.ps0 = ps[0]; box.ps1 = ps[1]; box.ps2 = ps[2]; box.ps3 = ps[3];
+  return face_launch(score, box, n, batch, shrink, top, out_det, out_index, nullptr, workspace, st);
 }
 
 }  // namespace
@@ -477,7 +656,12 @@ using namespace dan;
 
 extern "C" {
 
-size_t dan_detect_face_workspace_bytes(int64_t n) { return n < 0 ? 0 : align_up((size_t)n * 8, 256); }
+size_t dan_detect_face_batch_workspace_bytes(int64_t num_anchors, int32_t batch) {
+  if (num_anchors < 0 || batch < 0) return 0;
+  return face_hist_bytes(batch) + align_up((size_t)num_anchors * (size_t)batch * 8, 256);
+}
+
+size_t dan_detect_face_workspace_bytes(int64_t n) { return dan_detect_face_batch_workspace_bytes(n, 1); }
 
 int dan_detect_face_select(const float* bboxes, const float* scores, int64_t n, float shrink, int32_t top, float* out_det,
                            int32_t* out_index, int32_t* out_count, void* workspace, size_t workspace_bytes, void* stream) {
@@ -488,25 +672,41 @@ int dan_detect_face_select(const float* bboxes, const float* scores, int64_t n, 
   const size_t need = dan_detect_face_workspace_bytes(n);
   DAN_REQUIRE(n == 0 || (workspace != nullptr && workspace_bytes >= need), DAN_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu",
               need, workspace_bytes);
+  FaceScores score = {scores};
+  FaceBoxes box = {reinterpret_cast<const float4*>(bboxes)};
+  return face_launch(score, box, n, 1, shrink, top, out_det, out_index, out_count, workspace, (cudaStream_t)stream);
+}
+
+int dan_detect_face_batch(int32_t pred_dtype, const void* cls_pred, const void* loc_pred, const float* a_ymin, const float* a_xmin,
+                          const float* a_ymax, const float* a_xmax, int64_t num_anchors, int32_t batch, const float* h_prior_scaling,
+                          float shrink, int32_t top, float* out_det, int32_t* out_index, void* workspace, size_t workspace_bytes,
+                          void* stream) {
+  const int esize = dtype_bytes(pred_dtype);
+  DAN_REQUIRE(esize != 0, DAN_ERR_INVALID_ARGUMENT, "unknown pred_dtype %d", pred_dtype);
+  DAN_REQUIRE(num_anchors >= 0 && num_anchors < ((int64_t)1 << 31) && batch >= 0, DAN_ERR_INVALID_ARGUMENT, "bad num_anchors / batch");
+  DAN_REQUIRE(top >= 1 && top <= kSortCap, DAN_ERR_UNSUPPORTED, "top must be in [1, %d]", kSortCap);
+  if (batch == 0) return DAN_OK;
+  DAN_REQUIRE(cls_pred && loc_pred && a_ymin && a_xmin && a_ymax && a_xmax && h_prior_scaling && out_det, DAN_ERR_INVALID_ARGUMENT,
+              "NULL pointer");
+  DAN_REQUIRE((reinterpret_cast<uintptr_t>(loc_pred) & (uintptr_t)(4 * esize - 1)) == 0, DAN_ERR_INVALID_ARGUMENT,
+              "loc_pred must be %d-byte aligned", 4 * esize);
+  const int64_t chunks = (num_anchors + kFaceChunk - 1) / kFaceChunk;
+  DAN_REQUIRE(chunks * batch < ((int64_t)1 << 31), DAN_ERR_UNSUPPORTED, "batch x num_anchors too large");
+  const size_t need = dan_detect_face_batch_workspace_bytes(num_anchors, batch);
+  DAN_REQUIRE(workspace != nullptr && workspace_bytes >= need, DAN_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need,
+              workspace_bytes);
   cudaStream_t st = (cudaStream_t)stream;
-  FaceArgs A = {};
-  A.boxes = reinterpret_cast<const float4*>(bboxes);
-  A.scores = scores;
-  A.n = (int)n;
-  A.shrink = shrink;
-  A.top = top;
-  A.keys = static_cast<unsigned long long*>(workspace);
-  A.out = out_det;
-  A.out_index = out_index;
-  A.out_count = out_count;
-  if (n > 0) {
-    face_key_kernel<<<grid_for(n), 256, 0, st>>>(A);
-    DAN_LAUNCH_CHECK("face_key_kernel");
+  switch (pred_dtype) {
+    case DAN_DTYPE_F16:
+      return face_batch_launch<__half>(cls_pred, loc_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling, shrink, top,
+                                       out_det, out_index, workspace, st);
+    case DAN_DTYPE_BF16:
+      return face_batch_launch<__nv_bfloat16>(cls_pred, loc_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling, shrink,
+                                              top, out_det, out_index, workspace, st);
+    default:
+      return face_batch_launch<float>(cls_pred, loc_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling, shrink, top,
+                                      out_det, out_index, workspace, st);
   }
-  DAN_CUDA(cudaFuncSetAttribute(face_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSortCap * 8));
-  face_select_kernel<<<1, kSortThreads, kSortCap * 8, st>>>(A);
-  DAN_LAUNCH_CHECK("face_select_kernel");
-  return DAN_OK;
 }
 
 int dan_bbox_vote(const float* det, const int32_t* counts, int32_t batch, int32_t capacity, float nms_threshold,

@@ -556,6 +556,40 @@ def detect_face_select(bboxes, scores, shrink, top):
     return det, idx, cnt
 
 
+def detect_face_batch(cls_pred, loc_pred, anchors, shrink, top, prior_scaling=(0.1, 0.1, 0.2, 0.2), workspace=None):
+    """dan_detect_face_batch: softmax + decode + detect_face of B images from the head's raw outputs, fused.
+    cls_pred [B, N, 2] logits and loc_pred [B, N, 4] offsets, one dtype out of fp32 / fp16 / bf16; anchors =
+    (ymin, xmin, ymax, xmax) [N] each.  -> (det [B, top, 5] zero padded, index int32 [B, top] (-1 padded), k) where
+    k = max(min(N - 1, top), 0) valid rows per image.  Nothing synchronises with the host."""
+    L.require_device()
+    cls_pred = cls_pred.contiguous()
+    loc_pred = loc_pred.contiguous()
+    dtype = L.pred_dtype(cls_pred, "cls_pred")
+    if loc_pred.dtype != cls_pred.dtype:
+        raise TypeError("cls_pred is %s but loc_pred is %s: the predictions must share one dtype" % (cls_pred.dtype, loc_pred.dtype))
+    if cls_pred.dim() != 3 or cls_pred.shape[2] != 2:
+        raise ValueError("cls_pred must be [batch, num_anchors, 2], got %s" % (tuple(cls_pred.shape),))
+    batch, n = int(cls_pred.shape[0]), int(cls_pred.shape[1])
+    if tuple(loc_pred.shape) != (batch, n, 4):
+        raise ValueError("loc_pred must be [%d, %d, 4], got %s" % (batch, n, tuple(loc_pred.shape)))
+    if any(a.numel() != n for a in anchors):
+        raise ValueError("cls_pred has %d anchors per image but there are %d anchors" % (n, anchors[0].numel()))
+    dev = _dev(cls_pred)
+    _dev(loc_pred)
+    top = int(top)
+    det = torch.empty((batch, top, 5), dtype=torch.float32, device=dev)
+    idx = torch.empty((batch, top), dtype=torch.int32, device=dev)
+    nbytes = L.lib().dan_detect_face_batch_workspace_bytes(n, batch)
+    ws = (workspace or _ws).get(nbytes, dev)
+    ps = (ctypes.c_float * 4)(*[float(v) for v in prior_scaling])
+    with torch.cuda.device(dev):
+        L.check(L.lib().dan_detect_face_batch(dtype, L.dev_ptr(cls_pred, cls_pred.dtype, "cls_pred"),
+                                              L.dev_ptr(loc_pred, cls_pred.dtype, "loc_pred"), *_anchor_ptrs(*anchors), n, batch,
+                                              ps, float(shrink), top, L.dev_ptr(det), L.dev_ptr(idx), L.dev_ptr(ws), nbytes,
+                                              L.stream_ptr()))
+    return det, idx, max(min(n - 1, top), 0)
+
+
 def bbox_vote_batch(det, counts, nms_threshold, max_per_image, details=False):
     """dan_bbox_vote: det [B, cap, 5], counts int32 [B] or None -> (out [B, max_per_image, 5], out_count int32 [B]
     [, order int32 [B, cap], assign int32 [B, cap]])."""

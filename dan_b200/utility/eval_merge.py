@@ -1,6 +1,7 @@
 """Drop-in for the detection merge of the reference's evaluation scripts (SURVEY.md 8(f2)).
 
     detect_face_select   the numpy part of detect_face, eval_sfd.py:101-112 (= eval_dan.py:101-118): after net.run
+    detect_face_batch    softmax + decode_anchors + detect_face of a batch, from the head's logits and offsets
     bbox_vote            eval_sfd.py:170-210 (= eval_dan.py:201-241)
 
 Detections are rows (xmin, ymin, xmax, ymax, score), float32, +1 pixel convention, like the reference's numpy arrays;
@@ -21,6 +22,17 @@ def detect_face_select(bboxes, scores, shrink, max_per_image=750):
     top = int(max_per_image * 1.5)
     det, _, cnt = F.detect_face_select(L.as_f32(bboxes), L.as_f32(scores), shrink, top)
     return det[:int(cnt)]
+
+
+def detect_face_batch(cls_pred, loc_pred, anchors, shrink, max_per_image=750, prior_scaling=(0.1, 0.1, 0.2, 0.2)):
+    """The evaluation scripts' whole per-pass chain - softmax (eval_sfd.py:279), decode_anchors (:283) and
+    detect_face (:95-114) - for a batch, from the head's raw outputs: cls_pred [B, N, 2] logits and loc_pred [B, N, 4]
+    offsets (fp32, fp16 or bf16, one dtype), anchors (ymin, xmin, ymax, xmax) -> det [B, k, 5] rows
+    (xmin, ymin, xmax, ymax, score) with k = min(N - 1, int(max_per_image * 1.5)), sorted by descending score (equal
+    scores: higher index first).  No host read: the passes of one batch (scales, flips) are stacked with
+    torch.cat(dim=1) and go straight into bbox_vote_batch(det, None)."""
+    det, _, k = F.detect_face_batch(cls_pred, loc_pred, anchors, shrink, int(max_per_image * 1.5), prior_scaling)
+    return det[:, :k]
 
 
 def bbox_vote(det, nms_threshold=0.3, max_per_image=750):

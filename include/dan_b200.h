@@ -357,6 +357,18 @@ int dan_dynamic_anchor_routing_eval(const dan_routing_layers* h_layers, const fl
  *   (xmin, ymin, xmax, ymax, score), the top min(n-1, top) by descending score
  *   (top = int(1.5 * max_per_image) = 1125); equal scores: higher index first.
  *   out_det [top,5] zero padded, out_index [top] (-1 padded, may be NULL), out_count [1].
+ * dan_detect_face_batch: the whole detect_face chain of the evaluation scripts
+ *   (softmax :279, decode_anchors :283, detect_face :95-114) for B images from the
+ *   head's raw outputs: cls_pred [B,N,2] logits, loc_pred [B,N,4] offsets (cy,cx,h,w),
+ *   one dtype for both (DAN_DTYPE_*), and the N anchors.  Every image gets
+ *   k = max(min(N - 1, top), 0) rows, which the caller knows without a host read:
+ *   out_det [B,top,5] (xmin, ymin, xmax, ymax, score) zero padded, out_index [B,top]
+ *   anchor index (-1 padded, may be NULL).  Bit-identical to dan_softmax column 1 ->
+ *   dan_decode_batch -> dan_detect_face_select per image; fp16 / bf16 predictions give
+ *   the results of the fp32 call on the widened values.  Only the k rows are decoded;
+ *   nothing N-sized but one 8-byte key per anchor reaches memory.  top in [1, 8192],
+ *   N < 2^31, loc_pred rows 16-byte (fp32) / 8-byte (fp16, bf16) aligned; cls_pred
+ *   needs no alignment beyond its element type.  batch == 0 enqueues nothing.
  * dan_bbox_vote: bbox_vote (eval_sfd.py:170-210 = eval_dan.py:201-241), batched:
  *   det [B, capacity, 5] rows (xmin, ymin, xmax, ymax, score), counts [B] valid rows
  *   per image (NULL = capacity); out_det [B, max_per_image, 5] zero padded,
@@ -368,6 +380,13 @@ size_t dan_detect_face_workspace_bytes(int64_t n);
 int dan_detect_face_select(const float* bboxes, const float* scores, int64_t n, float shrink,
                            int32_t top, float* out_det, int32_t* out_index, int32_t* out_count,
                            void* workspace, size_t workspace_bytes, void* stream);
+size_t dan_detect_face_batch_workspace_bytes(int64_t num_anchors, int32_t batch);
+int dan_detect_face_batch(int32_t pred_dtype, const void* cls_pred, const void* loc_pred,
+                          const float* a_ymin, const float* a_xmin, const float* a_ymax,
+                          const float* a_xmax, int64_t num_anchors, int32_t batch,
+                          const float* h_prior_scaling, float shrink, int32_t top,
+                          float* out_det, int32_t* out_index, void* workspace,
+                          size_t workspace_bytes, void* stream);
 int dan_bbox_vote(const float* det, const int32_t* counts, int32_t batch, int32_t capacity,
                   float nms_threshold, int32_t max_per_image, float* out_det, int32_t* out_count,
                   int32_t* out_order, int32_t* out_assign, void* stream);
