@@ -403,22 +403,6 @@ static GreedyPlan greedy_plan(int64_t n, int keep_topk, int nms_cap) {
   return g;
 }
 
-// block-wide min / max of a float over all threads (every thread gets the result)
-DAN_D void block_minmax(float lo, float hi, float& out_lo, float& out_hi) {
-  __shared__ int s_lo[kSortThreads / 32], s_hi[kSortThreads / 32];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int wl = __reduce_min_sync(0xffffffffu, float_to_ordered(lo));
-  const int wh = __reduce_max_sync(0xffffffffu, float_to_ordered(hi));
-  if (lane == 0) { s_lo[warp] = wl; s_hi[warp] = wh; }
-  __syncthreads();
-  int a = (lane < kSortThreads / 32) ? s_lo[lane] : 0x7fffffff, b = (lane < kSortThreads / 32) ? s_hi[lane] : (int)0x80000000;
-  a = __reduce_min_sync(0xffffffffu, a);
-  b = __reduce_max_sync(0xffffffffu, b);
-  out_lo = ordered_to_float(a);
-  out_hi = ordered_to_float(b);
-  __syncthreads();
-}
-
 // stripe masks of the broad phase (see init_stripes); monotone in the coordinate, so overlapping intervals share a bit
 struct Stripes {
   float ylo, yinv, xlo, xinv;

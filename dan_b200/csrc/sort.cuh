@@ -1,5 +1,6 @@
-// Block-wide top-k + sort of 64-bit keys in shared memory (1024-thread CTAs), shared by the postprocess and the
-// evaluation-merge kernels.  Include it INSIDE `namespace dan { ... }` of a .cu file, after common.cuh.
+// Block-wide helpers of the 1024-thread CTAs that the postprocess and the evaluation-merge kernels share: top-k + sort of
+// 64-bit keys in shared memory, and the min / max of a float over the CTA.  Include it INSIDE `namespace dan { ... }` of
+// a .cu file, after common.cuh.
 #pragma once
 
 constexpr int kSortCap = 8192;      // keys sorted in shared memory (64 KB)
@@ -8,6 +9,22 @@ constexpr int kSortThreads = 1024;  // threads per CTA of the sort kernels
 // order-preserving float <-> uint32 (descending key order = descending score)
 DAN_D uint32_t score_to_key(float s) { return (uint32_t)float_to_ordered(s) ^ 0x80000000u; }
 DAN_D float key_to_score(uint32_t k) { return ordered_to_float((int)(k ^ 0x80000000u)); }
+
+// block-wide min / max of a float over all threads (every thread gets the result)
+DAN_D void block_minmax(float lo, float hi, float& out_lo, float& out_hi) {
+  __shared__ int s_lo[kSortThreads / 32], s_hi[kSortThreads / 32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int wl = __reduce_min_sync(0xffffffffu, float_to_ordered(lo));
+  const int wh = __reduce_max_sync(0xffffffffu, float_to_ordered(hi));
+  if (lane == 0) { s_lo[warp] = wl; s_hi[warp] = wh; }
+  __syncthreads();
+  int a = (lane < kSortThreads / 32) ? s_lo[lane] : 0x7fffffff, b = (lane < kSortThreads / 32) ? s_hi[lane] : (int)0x80000000;
+  a = __reduce_min_sync(0xffffffffu, a);
+  b = __reduce_max_sync(0xffffffffu, b);
+  out_lo = ordered_to_float(a);
+  out_hi = ordered_to_float(b);
+  __syncthreads();
+}
 
 // ---------------------------------------------------------------------------
 // K4: per-list top-k (radix select when needed) + bitonic sort, all in shared memory.

@@ -9,14 +9,21 @@
 // bbox_vote without the shrinking array: in descending score order, a detection that no earlier HEAD overlaps with
 // IoU >= thr is a head, every other one joins the FIRST head that overlaps it (pinned against the reference's own
 // function, tests/golden/vote_reference.npz).  One 1024-thread CTA per image keeps the sorted detections in shared
-// memory:
-//   1. 64-bit keys (score bits << 32 | index), bitonic sort (sort.cuh); equal scores: higher index first, i.e.
-//      numpy's argsort(kind="stable")[::-1] (the reference's default quicksort leaves ties unspecified)
-//   2. heads, 32 candidates per round: the round's candidates are resolved against each other with 32x32 pair tests
-//      and bit masks, then every thread tests its own (register resident) detections against the round's heads
-//   3. the groups with >= 2 members are numbered in head order (block scan); thread q walks the members of group q in
-//      score order: box sums accumulate sequentially like np.sum(axis=0), the score sum reproduces numpy's pairwise
-//      summation (8 interleaved accumulators up to 128 elements, recursive halving beyond), all in fp32 without FMA.
+// memory (vote_plan); bbox_vote_kernel runs these steps (DESIGN.md §4e):
+//   1.  sort_and_gather  64-bit keys (score bits << 32 | index), bitonic sort (sort.cuh); equal scores: higher index
+//                        first, i.e. numpy's argsort(kind="stable")[::-1] (the reference's default quicksort leaves ties
+//                        unspecified).  Thread t keeps the score ranks t, t + 1024, ... in registers (VoteRegs).
+//       init_stripes     broad phase of step 2: a stripe grid over the detections' extent, each detection's stripes
+//   2.  heads in score order, 32 candidates per round (five barriers each):
+//   2a. list_candidates  warp 0 lists the next (up to) 32 unassigned positions = the round's candidates
+//   2b. candidate_masks  the candidates against each other: 32x32 pair tests -> one bit mask per candidate
+//   2c. resolve_heads    which candidates are heads, which join an earlier head of the round; the heads' stripes
+//   2d. join_heads       every thread tests its own live detections against the round's heads
+//   3.  number_groups    the groups with >= 2 members are numbered in head order (block scan)
+//       write_groups     one warp walks the members of a group in score order: box sums accumulate sequentially like
+//                        np.sum(axis=0), the score sum reproduces numpy's pairwise summation (8 interleaved accumulators
+//                        up to 128 elements, recursive halving beyond), all in fp32 without FMA
+//       write_assign     the head of every detection (optional output)
 #include "common.cuh"
 
 namespace dan {
@@ -28,12 +35,38 @@ namespace {
 constexpr uint16_t kFree = 0xFFFFu;      // not assigned yet
 constexpr uint16_t kGone = 0xFFFEu;      // a head that does not even match itself (NaN IoU): deleted alone
 
+// Dynamic shared memory of one bbox_vote_kernel launch (vote_plan).  Offsets are in bytes from the start of the dynamic
+// shared memory, where the sort keys start; the boxes overwrite the keys once they are consumed.
+struct VotePlan {
+  int score;                  // [cap] float, after max(keys, boxes)
+  int assign;                 // [cap] uint16: head position of each detection (kFree, kGone)
+  int count;                  // [cap] uint16: members of the group headed there (4-byte aligned: two per atomic word)
+  int qlist;                  // [cap] uint16: head position of group q
+  int smem;                   // dynamic shared memory of the launch
+};
+
+constexpr int kVoteSmemMax = 221 * 1024;  // dynamic part (the kernel has ~1 KB of static shared memory)
+
+static VotePlan vote_plan(int cap) {
+  int pad = 256;                          // the sort pads the keys to a power of two (here at least 256)
+  while (pad < cap) pad <<= 1;
+  const int u16 = (int)align_up((size_t)cap * 2, 16);
+  VotePlan p;
+  p.score = pad * 8 > cap * 16 ? pad * 8 : cap * 16;
+  p.assign = p.score + cap * 4;
+  p.count = p.assign + u16;
+  p.qlist = p.count + u16;
+  p.smem = p.qlist + u16;
+  return p;
+}
+
 struct VoteArgs {
   const float* det;           // [B, cap, 5] (xmin, ymin, xmax, ymax, score)
   const int32_t* counts;      // [B] valid rows of each image (NULL: all cap rows)
   int cap;
   float thr;
   int max_out;
+  VotePlan plan;              // shared-memory plan of the launch
   float* out;                 // [B, max_out, 5] zero padded
   int32_t* out_count;         // [B]
   int32_t* out_order;         // [B, cap] optional: sorted position -> input row
@@ -80,11 +113,16 @@ struct MemberIter {
   const uint16_t* assign;
   const float4* box;
   const float* score;
-  int pos, n;                           // next window of 32 positions to look at
-  int base;                             // first position of the window `pending` describes
-  unsigned pending;                     // members of the current window that have not been consumed
+  int n;
   uint16_t head;
-  float sx, sy, sz, sw, mx;             // sequential sums of box * score (np.sum(axis=0)), running max score
+  int pos;                              // next window of 32 positions to look at
+  int base = 0;                         // first position of the window `pending` describes
+  unsigned pending = 0u;                // members of the current window that have not been consumed
+  float sx = 0.f, sy = 0.f, sz = 0.f, sw = 0.f;            // sequential sums of box * score (np.sum(axis=0))
+  float mx = -INFINITY;                                     // running max score
+  // the head is the first member of its own group (a deleted head has count 0)
+  DAN_D MemberIter(const uint16_t* assign_, const float4* box_, const float* score_, int n_, uint16_t head_)
+      : assign(assign_), box(box_), score(score_), n(n_), head(head_), pos(head_) {}
   DAN_D float next() {                  // score of the next member; accumulates its weighted box (warp-uniform)
     const int lane = threadIdx.x & 31;
     while (pending == 0u) {             // (the caller asks for exactly count[head] members, so one more always exists)
@@ -157,229 +195,245 @@ DAN_D float numpy_pairwise(MemberIter& it, int m) {
   return ret;
 }
 
-static size_t vote_smem_bytes(int cap) {
-  const size_t pad = (size_t)1 << (32 - __builtin_clz((unsigned)(cap > 1 ? cap - 1 : 1)));     // next power of two >= cap
-  const size_t keys = (pad < 256 ? 256 : pad) * 8;
-  const size_t boxes = (size_t)cap * 16;
-  // [ boxes (aliases the sort keys) | score | assign | count | qlist ]
-  return (keys > boxes ? keys : boxes) + (size_t)cap * 4 + align_up((size_t)cap * 2, 16) * 3;
+// count[head] += 1.  Two uint16 counts share one 32-bit word (VotePlan::count is 4-byte aligned), and no count exceeds
+// the 8192 detections of an image, so the low half never carries into the high one.
+DAN_D void count_member(uint16_t* count, int head) {
+  atomicAdd(reinterpret_cast<unsigned int*>(count) + (head >> 1), 1u << ((head & 1) * 16));
 }
 
-__global__ void __launch_bounds__(kSortThreads, 1) bbox_vote_kernel(const VoteArgs A) {
-  extern __shared__ __align__(16) unsigned char dyn_smem[];
-  __shared__ int s_scan[kSortThreads / 32];
-  __shared__ int s_total;
-  const int b = blockIdx.x;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int n = A.counts ? min(max(A.counts[b], 0), A.cap) : A.cap;
-  const float* det = A.det + (int64_t)b * A.cap * 5;
+constexpr int kPer = kSortCap / kSortThreads;    // score ranks per thread: t, t + 1024, ...
 
-  size_t pad = 256;
-  while ((int)pad < A.cap) pad <<= 1;
-  const size_t front = (pad * 8 > (size_t)A.cap * 16) ? pad * 8 : (size_t)A.cap * 16;
-  unsigned long long* keys = reinterpret_cast<unsigned long long*>(dyn_smem);
-  float4* box = reinterpret_cast<float4*>(dyn_smem);                     // aliases the keys once they are consumed
-  float* score = reinterpret_cast<float*>(dyn_smem + front);
-  uint16_t* assign = reinterpret_cast<uint16_t*>(dyn_smem + front + (size_t)A.cap * 4);
-  const size_t u16_span = ((size_t)A.cap * 2 + 15) / 16 * 8;             // elements per 16-byte aligned uint16 array
-  uint16_t* count = assign + u16_span;
-  uint16_t* qlist = count + u16_span;
+// An image's detections in the launch's dynamic shared memory (vote_plan), indexed by score rank.
+struct VoteImage {
+  int b, n;                   // image, detections
+  unsigned long long* keys;   // step 1: the sort keys, ...
+  float4* box;                // ... which the boxes overwrite
+  float* score;
+  uint16_t* assign;
+  uint16_t* count;
+  uint16_t* qlist;
+};
 
-  // ---- 1. sort by descending score (:171-172)
-  for (int i = tid; i < n; i += kSortThreads)
-    keys[i] = ((unsigned long long)score_to_key(det[i * 5 + 4]) << 32) | (unsigned long long)(uint32_t)i;
+// The thread's detections (score ranks tid + e * kSortThreads), in registers: every index into the arrays is a
+// compile-time constant.
+struct VoteRegs {
+  float4 box[kPer];
+  int rank[kPer];             // -1: none
+  uint32_t range[kPer];       // packed stripe ranges (VoteStripes::range)
+  unsigned alive;             // bit e: rank[e] is not assigned yet
+};
+
+// the kernel's static shared memory that the steps of a round pass to each other
+struct VoteRound {
+  int* cand;                  // [32] step a: positions of the round's candidates
+  int* ncand;
+  unsigned* mask;             // [32] step b: bit m of mask[k] = candidate k overlaps the earlier candidate m
+  unsigned* selfok;           // step b: bit k = candidate k overlaps itself (not NaN)
+  unsigned* xs;               // [32] step c: bit m of xs[s] = the round's head m touches x stripe s
+  unsigned* ys;               // ... y stripe s
+};
+
+DAN_D VoteImage carve(const VoteArgs& A, unsigned char* dyn_smem) {
+  VoteImage im;
+  im.b = blockIdx.x;
+  im.n = A.counts ? min(max(A.counts[im.b], 0), A.cap) : A.cap;
+  im.keys = reinterpret_cast<unsigned long long*>(dyn_smem);
+  im.box = reinterpret_cast<float4*>(dyn_smem);
+  im.score = reinterpret_cast<float*>(dyn_smem + A.plan.score);
+  im.assign = reinterpret_cast<uint16_t*>(dyn_smem + A.plan.assign);
+  im.count = reinterpret_cast<uint16_t*>(dyn_smem + A.plan.count);
+  im.qlist = reinterpret_cast<uint16_t*>(dyn_smem + A.plan.qlist);
+  return im;
+}
+
+// ---- 1. sort by descending score (:171-172), then gather through registers (the boxes overwrite the key storage)
+DAN_D void sort_and_gather(const VoteArgs& A, const VoteImage& im, VoteRegs& R) {
+  const int tid = threadIdx.x;
+  const float* det = A.det + (int64_t)im.b * A.cap * 5;
+  for (int i = tid; i < im.n; i += kSortThreads)
+    im.keys[i] = ((unsigned long long)score_to_key(det[i * 5 + 4]) << 32) | (unsigned long long)(uint32_t)i;
   __syncthreads();
-  sort_smem_keys(keys, n);
-  // gather through registers (the boxes overwrite the key storage); thread t keeps the boxes of the score ranks
-  // t, t + 1024, ... in registers for the sweeps below
-  constexpr int kPer = kSortCap / kSortThreads;
-  float4 rb[kPer];
+  sort_smem_keys(im.keys, im.n);
   float rs[kPer];
-  int rr[kPer];                                            // score rank of the box in rb[e], -1 = none
 #pragma unroll
   for (int e = 0; e < kPer; ++e) {
     const int r = tid + e * kSortThreads;
-    rr[e] = -1;
-    if (r < n) {
-      const int i = (int)(uint32_t)(keys[r] & 0xFFFFFFFFull);
-      rr[e] = r;
-      rb[e] = make_float4(det[i * 5], det[i * 5 + 1], det[i * 5 + 2], det[i * 5 + 3]);
+    R.rank[e] = -1;
+    if (r < im.n) {
+      const int i = (int)(uint32_t)(im.keys[r] & 0xFFFFFFFFull);
+      R.rank[e] = r;
+      R.box[e] = make_float4(det[i * 5], det[i * 5 + 1], det[i * 5 + 2], det[i * 5 + 3]);
       rs[e] = det[i * 5 + 4];
-      if (A.out_order) A.out_order[(int64_t)b * A.cap + r] = i;
+      if (A.out_order) A.out_order[(int64_t)im.b * A.cap + r] = i;
     }
   }
   __syncthreads();
 #pragma unroll
   for (int e = 0; e < kPer; ++e) {
-    if (rr[e] >= 0) {
-      box[rr[e]] = rb[e];
-      score[rr[e]] = rs[e];
-      assign[rr[e]] = kFree;
-      count[rr[e]] = 0;
+    if (R.rank[e] >= 0) {
+      im.box[R.rank[e]] = R.box[e];
+      im.score[R.rank[e]] = rs[e];
+      im.assign[R.rank[e]] = kFree;
+      im.count[R.rank[e]] = 0;
     }
   }
   __syncthreads();
+}
 
-  // ---- 2. heads in score order (:173-190), 32 candidate heads per round.
-  // Thread t owns the score ranks t, t + 1024, ...: an `alive` bit and the packed stripe ranges of each in registers.
-  //   a. warp 0 lists the next (up to) 32 unassigned positions = the candidates of this round
-  //   b. thread (k = warp, m = lane) tests candidate k against the earlier candidate m  -> 32 row masks
-  //   c. every thread resolves the 32 candidates from the masks (bit operations): candidate k is a head unless an earlier
-  //      HEAD of the round overlaps it (then it joins the first such head); warp s publishes which of the round's heads
-  //      touch x / y stripe s (two ballots)
-  //   d. every thread looks its own alive boxes behind the last candidate up in that index - (OR over the box's x
-  //      stripes) AND (OR over its y stripes) = the round's heads it can overlap - and runs the exact test on those
-  //      only, in head order (the first hit is the head it joins)
-  // Four barriers per 32 heads.
-  __shared__ int s_cand[32];
-  __shared__ unsigned s_mask[32];
-  __shared__ unsigned s_selfok;
-  __shared__ int s_ncand;
-  __shared__ unsigned s_xs[32], s_ys[32];
-  __shared__ float s_ext[kSortThreads / 32][4];
+// The stripe grid over the extent of the detections with finite coordinates below 1e30, and the stripe range of each
+// of the thread's detections; all of them are alive.
+DAN_D VoteStripes init_stripes(const VoteArgs& A, VoteRegs& R) {
+  float x0 = 3.0e38f, x1 = -3.0e38f, y0 = 3.0e38f, y1 = -3.0e38f;
+#pragma unroll
+  for (int e = 0; e < kPer; ++e) {
+    const float4 bx = R.box[e];
+    if (R.rank[e] >= 0 && fabsf(bx.x) < 1e30f && fabsf(bx.y) < 1e30f && fabsf(bx.z) < 1e30f && fabsf(bx.w) < 1e30f) {
+      x0 = fminf(x0, bx.x); x1 = fmaxf(x1, fadd(bx.z, 1.f));
+      y0 = fminf(y0, bx.y); y1 = fmaxf(y1, fadd(bx.w, 1.f));
+    }
+  }
   VoteStripes sg;
-  {
-    float x0 = 3.0e38f, x1 = -3.0e38f, y0 = 3.0e38f, y1 = -3.0e38f;
-#pragma unroll
-    for (int e = 0; e < kPer; ++e) {
-      const float4 bx = rb[e];
-      if (rr[e] >= 0 && fabsf(bx.x) < 1e30f && fabsf(bx.y) < 1e30f && fabsf(bx.z) < 1e30f && fabsf(bx.w) < 1e30f) {
-        x0 = fminf(x0, bx.x); x1 = fmaxf(x1, fadd(bx.z, 1.f));
-        y0 = fminf(y0, bx.y); y1 = fmaxf(y1, fadd(bx.w, 1.f));
-      }
-    }
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      x0 = fminf(x0, __shfl_xor_sync(0xffffffffu, x0, d)); x1 = fmaxf(x1, __shfl_xor_sync(0xffffffffu, x1, d));
-      y0 = fminf(y0, __shfl_xor_sync(0xffffffffu, y0, d)); y1 = fmaxf(y1, __shfl_xor_sync(0xffffffffu, y1, d));
-    }
-    if (lane == 0) { s_ext[warp][0] = x0; s_ext[warp][1] = x1; s_ext[warp][2] = y0; s_ext[warp][3] = y1; }
-    __syncthreads();
-    for (int w = 0; w < kSortThreads / 32; ++w) {
-      x0 = fminf(x0, s_ext[w][0]); x1 = fmaxf(x1, s_ext[w][1]);
-      y0 = fminf(y0, s_ext[w][2]); y1 = fmaxf(y1, s_ext[w][3]);
-    }
-    sg.xlo = x0; sg.ylo = y0;
-    sg.xinv = (x1 > x0) ? fdiv(32.f, fsub(x1, x0)) : 0.f;
-    sg.yinv = (y1 > y0) ? fdiv(32.f, fsub(y1, y0)) : 0.f;
-    sg.all = !(A.thr > 0.f);
-  }
-  uint32_t rq[kPer];                                       // packed stripe ranges of the thread's boxes
-  unsigned alive = 0;
+  float ex, ey;
+  block_minmax(x0, x1, sg.xlo, ex);
+  block_minmax(y0, y1, sg.ylo, ey);
+  sg.xinv = (ex > sg.xlo) ? fdiv(32.f, fsub(ex, sg.xlo)) : 0.f;
+  sg.yinv = (ey > sg.ylo) ? fdiv(32.f, fsub(ey, sg.ylo)) : 0.f;
+  sg.all = !(A.thr > 0.f);
+  R.alive = 0u;
 #pragma unroll
   for (int e = 0; e < kPer; ++e) {
-    alive |= (rr[e] >= 0) ? (1u << e) : 0u;
-    rq[e] = (rr[e] >= 0) ? sg.range(rb[e]) : 0u;
+    R.alive |= (R.rank[e] >= 0) ? (1u << e) : 0u;
+    R.range[e] = (R.rank[e] >= 0) ? sg.range(R.box[e]) : 0u;
   }
-  auto add_count = [&](int head, unsigned k) {
-    atomicAdd(reinterpret_cast<unsigned int*>(count) + (head >> 1), k << ((head & 1) * 16));
-  };
-  int cur = 0;
-  while (true) {
-    if (warp == 0) {                                       // a.
-      int have = 0, p = cur;
-      while (p < n && have < 32) {
-        const bool un = (p + lane < n) && assign[p + lane] == kFree;
-        const unsigned m = __ballot_sync(0xffffffffu, un);
-        const int rank = have + __popc(m & ((1u << lane) - 1u));
-        if (un && rank < 32) s_cand[rank] = p + lane;
-        have += __popc(m);
-        p += 32;
-      }
-      if (lane == 0) s_ncand = min(have, 32);
+  return sg;
+}
+
+// ---- 2. heads in score order (:173-190), 32 candidate heads per round.
+// a. warp 0 lists the next (up to) 32 unassigned positions from `cur` on; returns their number (CTA-uniform)
+DAN_D int list_candidates(const VoteImage& im, const VoteRound& S, int cur) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (warp == 0) {
+    int have = 0, p = cur;
+    while (p < im.n && have < 32) {
+      const bool un = (p + lane < im.n) && im.assign[p + lane] == kFree;
+      const unsigned m = __ballot_sync(0xffffffffu, un);
+      const int rank = have + __popc(m & ((1u << lane) - 1u));
+      if (un && rank < 32) S.cand[rank] = p + lane;
+      have += __popc(m);
+      p += 32;
     }
-    __syncthreads();
-    const int ncand = s_ncand;
-    if (ncand == 0) break;
-    const int last = s_cand[ncand - 1];
-    {                                                      // b.
-      const int k = warp, m = lane;
-      bool ov = false, self_ok = false;
-      if (k < ncand && m <= k && m < ncand) {
-        const float4 bm = box[s_cand[m]];
-        const bool hit = vote_overlaps(bm, vote_area(bm), box[s_cand[k]], A.thr);
-        ov = hit && m < k;
-        self_ok = hit && m == k;
-      }
-      const unsigned row = __ballot_sync(0xffffffffu, ov);
-      const unsigned so = __ballot_sync(0xffffffffu, self_ok);
-      if (lane == 0) s_mask[k] = row;
-      if (lane == 0 && k == 0) s_selfok = 0u;
-      __syncthreads();
-      if (lane == 0 && so) atomicOr(&s_selfok, 1u << k);
-    }
-    __syncthreads();
-    unsigned heads = 0u;                                   // c. (redundantly in every thread)
-    int joined = -1;                                       // lane k of warp 0 applies candidate k
-    for (int k = 0; k < ncand; ++k) {
-      const unsigned mk = s_mask[k] & heads;
-      if (mk == 0u) heads |= 1u << k;
-      if (warp == 0 && lane == k) joined = mk ? __ffs(mk) - 1 : -1;
-    }
-    if (warp == 0 && lane < ncand) {
-      const int pos = s_cand[lane];
-      if (joined >= 0) {
-        assign[pos] = (uint16_t)s_cand[joined];
-        add_count(s_cand[joined], 1u);
-      } else if ((s_selfok >> lane) & 1u) {
-        assign[pos] = (uint16_t)pos;
-        add_count(pos, 1u);
-      } else {
-        assign[pos] = kGone;                               // NaN self IoU: deleted alone (:189-190)
-      }
-    }
-    {                                                      // warp s: the round's heads that touch x / y stripe s
-      uint32_t q = 0u;
-      const bool is_head = lane < ncand && ((heads >> lane) & 1u);
-      if (is_head) q = sg.range(box[s_cand[lane]]);
-      const bool every = (q & kEverywhere) != 0u;
-      const unsigned hx = __ballot_sync(0xffffffffu, is_head && (every || ((stripe_span(q & 31u, (q >> 5) & 31u) >> warp) & 1u)));
-      const unsigned hy = __ballot_sync(0xffffffffu, is_head && (every || ((stripe_span((q >> 10) & 31u, (q >> 15) & 31u) >> warp) & 1u)));
-      if (lane == 0) { s_xs[warp] = hx; s_ys[warp] = hy; }
-    }
-#pragma unroll
-    for (int e = 0; e < kPer; ++e)                         // the candidates themselves are settled
-      if (tid + e * kSortThreads <= last) alive &= ~(1u << e);
-    __syncthreads();
-#pragma unroll
-    for (int e = 0; e < kPer; ++e) {                       // d.
-      if ((alive >> e) & 1u) {
-        const uint32_t q = rq[e];
-        unsigned poss = heads;
-        if (!(q & kEverywhere)) {
-          unsigned ax = 0u, ay = 0u;
-          for (uint32_t st = q & 31u; st <= ((q >> 5) & 31u); ++st) ax |= s_xs[st];
-          for (uint32_t st = (q >> 10) & 31u; st <= ((q >> 15) & 31u); ++st) ay |= s_ys[st];
-          poss = ax & ay;
-        }
-        const int r = tid + e * kSortThreads;              // (the box itself stays in shared memory: it is needed rarely)
-        const float4 me = poss ? box[r] : make_float4(0.f, 0.f, 0.f, 0.f);
-        while (poss) {                                     // ascending = head order: the first hit is the head it joins
-          const int m = __ffs(poss) - 1;
-          poss &= poss - 1u;
-          const int hp = s_cand[m];
-          const float4 h = box[hp];
-          if (vote_overlaps(h, vote_area(h), me, A.thr)) {
-            assign[r] = (uint16_t)hp;
-            alive &= ~(1u << e);
-            add_count(hp, 1u);
-            poss = 0u;                                     // (no `break`: the lanes of the warp leave the loop together,
-                                                           // racecheck saw them reach the barrier apart otherwise)
-          }
-        }
-      }
-    }
-    cur = last + 1;
-    __syncthreads();
+    if (lane == 0) *S.ncand = min(have, 32);
   }
   __syncthreads();
+  return *S.ncand;
+}
 
-  // ---- 3. groups with at least two members, numbered in head order (:191-197, :205)
-  const int E = (n + kSortThreads - 1) / kSortThreads;
+// b. thread (k = warp, m = lane) tests candidate k against the earlier candidate m -> 32 row masks, and candidate k
+// against itself
+DAN_D void candidate_masks(const VoteArgs& A, const VoteImage& im, const VoteRound& S, int ncand) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int k = warp, m = lane;
+  bool ov = false, self_ok = false;
+  if (k < ncand && m <= k && m < ncand) {
+    const float4 bm = im.box[S.cand[m]];
+    const bool hit = vote_overlaps(bm, vote_area(bm), im.box[S.cand[k]], A.thr);
+    ov = hit && m < k;
+    self_ok = hit && m == k;
+  }
+  const unsigned row = __ballot_sync(0xffffffffu, ov);
+  const unsigned so = __ballot_sync(0xffffffffu, self_ok);
+  if (lane == 0) S.mask[k] = row;
+  if (lane == 0 && k == 0) *S.selfok = 0u;
+  __syncthreads();
+  if (lane == 0 && so) atomicOr(S.selfok, 1u << k);
+  __syncthreads();
+}
+
+// c. every thread resolves the candidates from the masks (bit operations): candidate k is a head unless an earlier HEAD
+// of the round overlaps it, then it joins the first such head; lane k of warp 0 writes candidate k's assign and count.
+// Warp s publishes which of the round's heads touch x / y stripe s (two ballots).  Returns the heads (bit k: candidate k).
+DAN_D unsigned resolve_heads(const VoteImage& im, const VoteRound& S, const VoteStripes& sg, int ncand) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  unsigned heads = 0u;
+  int joined = -1;
+  for (int k = 0; k < ncand; ++k) {
+    const unsigned mk = S.mask[k] & heads;
+    if (mk == 0u) heads |= 1u << k;
+    if (warp == 0 && lane == k) joined = mk ? __ffs(mk) - 1 : -1;
+  }
+  if (warp == 0 && lane < ncand) {
+    const int pos = S.cand[lane];
+    if (joined >= 0) {
+      im.assign[pos] = (uint16_t)S.cand[joined];
+      count_member(im.count, S.cand[joined]);
+    } else if ((*S.selfok >> lane) & 1u) {
+      im.assign[pos] = (uint16_t)pos;
+      count_member(im.count, pos);
+    } else {
+      im.assign[pos] = kGone;                              // NaN self IoU: deleted alone (:189-190)
+    }
+  }
+  uint32_t q = 0u;
+  const bool is_head = lane < ncand && ((heads >> lane) & 1u);
+  if (is_head) q = sg.range(im.box[S.cand[lane]]);
+  const bool every = (q & kEverywhere) != 0u;
+  const unsigned hx = __ballot_sync(0xffffffffu, is_head && (every || ((stripe_span(q & 31u, (q >> 5) & 31u) >> warp) & 1u)));
+  const unsigned hy = __ballot_sync(0xffffffffu, is_head && (every || ((stripe_span((q >> 10) & 31u, (q >> 15) & 31u) >> warp) & 1u)));
+  if (lane == 0) { S.xs[warp] = hx; S.ys[warp] = hy; }
+  __syncthreads();
+  return heads;
+}
+
+// d. every thread looks its own alive detections behind the round's last candidate up in the stripe index - (OR over
+// the detection's x stripes) AND (OR over its y stripes) = the round's heads it can overlap - and runs the exact test on
+// those only, in head order: the first hit is the head it joins
+DAN_D void join_heads(const VoteArgs& A, const VoteImage& im, const VoteRound& S, VoteRegs& R, unsigned heads, int last) {
+  const int tid = threadIdx.x;
+#pragma unroll
+  for (int e = 0; e < kPer; ++e)                           // the candidates themselves are settled
+    if (tid + e * kSortThreads <= last) R.alive &= ~(1u << e);
+#pragma unroll
+  for (int e = 0; e < kPer; ++e) {
+    if ((R.alive >> e) & 1u) {
+      const uint32_t q = R.range[e];
+      unsigned poss = heads;
+      if (!(q & kEverywhere)) {
+        unsigned ax = 0u, ay = 0u;
+        for (uint32_t st = q & 31u; st <= ((q >> 5) & 31u); ++st) ax |= S.xs[st];
+        for (uint32_t st = (q >> 10) & 31u; st <= ((q >> 15) & 31u); ++st) ay |= S.ys[st];
+        poss = ax & ay;
+      }
+      const int r = tid + e * kSortThreads;                // (the box itself stays in shared memory: it is needed rarely)
+      const float4 me = poss ? im.box[r] : make_float4(0.f, 0.f, 0.f, 0.f);
+      while (poss) {                                       // ascending = head order: the first hit is the head it joins
+        const int m = __ffs(poss) - 1;
+        poss &= poss - 1u;
+        const int hp = S.cand[m];
+        const float4 h = im.box[hp];
+        if (vote_overlaps(h, vote_area(h), me, A.thr)) {
+          im.assign[r] = (uint16_t)hp;
+          R.alive &= ~(1u << e);
+          count_member(im.count, hp);
+          poss = 0u;                                       // (no `break`: the lanes of the warp leave the loop together,
+                                                           // racecheck saw them reach the barrier apart otherwise)
+        }
+      }
+    }
+  }
+  __syncthreads();
+}
+
+// ---- 3. groups with at least two members, numbered in head order (:191-197, :205): qlist[q] = head of group q.
+// Returns the number of groups written (at most max_out).
+DAN_D int number_groups(const VoteArgs& A, const VoteImage& im) {
+  __shared__ int s_scan[kSortThreads / 32];
+  __shared__ int s_total;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int E = (im.n + kSortThreads - 1) / kSortThreads;
   int mine_cnt = 0;
   for (int e = 0; e < E; ++e) {
     const int r = tid * E + e;
-    if (r < n && count[r] >= 2) ++mine_cnt;
+    if (r < im.n && im.count[r] >= 2) ++mine_cnt;
   }
   int incl = mine_cnt;
 #pragma unroll
@@ -397,37 +451,61 @@ __global__ void __launch_bounds__(kSortThreads, 1) bbox_vote_kernel(const VoteAr
   int q = before + incl - mine_cnt;
   for (int e = 0; e < E; ++e) {
     const int r = tid * E + e;
-    if (r < n && count[r] >= 2) {
-      if (q < A.max_out) qlist[q] = (uint16_t)r;
+    if (r < im.n && im.count[r] >= 2) {
+      if (q < A.max_out) im.qlist[q] = (uint16_t)r;
       ++q;
     }
   }
   if (tid == 0) s_total = min(total, A.max_out);
   __syncthreads();
-  const int groups = s_total;
-  float* out = A.out + (int64_t)b * A.max_out * 5;
-  for (int g = warp; g < A.max_out; g += kSortThreads / 32) {          // one warp per group (warp-uniform control flow)
+  return s_total;
+}
+
+// one warp per group (warp-uniform control flow): the score-weighted mean box and the max score (:198-203)
+DAN_D void write_groups(const VoteArgs& A, const VoteImage& im, int groups) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  float* out = A.out + (int64_t)im.b * A.max_out * 5;
+  for (int g = warp; g < A.max_out; g += kSortThreads / 32) {
     float o0 = 0.f, o1 = 0.f, o2 = 0.f, o3 = 0.f, o4 = 0.f;
     if (g < groups) {
-      MemberIter it;
-      it.assign = assign; it.box = box; it.score = score; it.n = n;
-      it.head = qlist[g];
-      it.pos = it.head;                 // the head is the first member of its own group (a deleted head has count 0)
-      it.base = 0;
-      it.pending = 0u;
-      it.sx = it.sy = it.sz = it.sw = 0.f;
-      it.mx = __int_as_float(0xff800000);
-      const float ssum = numpy_pairwise(it, (int)count[it.head]);       // :199-201
+      MemberIter it(im.assign, im.box, im.score, im.n, im.qlist[g]);
+      const float ssum = numpy_pairwise(it, (int)im.count[it.head]);    // :199-201
       o0 = fdiv(it.sx, ssum); o1 = fdiv(it.sy, ssum); o2 = fdiv(it.sz, ssum); o3 = fdiv(it.sw, ssum);
       o4 = it.mx;                                                       // :200,202
     }
     if (lane == 0) { out[g * 5] = o0; out[g * 5 + 1] = o1; out[g * 5 + 2] = o2; out[g * 5 + 3] = o3; out[g * 5 + 4] = o4; }
   }
-  if (tid == 0) A.out_count[b] = groups;
-  if (A.out_assign) {
-    for (int r = tid; r < n; r += kSortThreads)
-      A.out_assign[(int64_t)b * A.cap + r] = assign[r] == kGone ? -2 : (int)assign[r];
+  if (tid == 0) A.out_count[im.b] = groups;
+}
+
+DAN_D void write_assign(const VoteArgs& A, const VoteImage& im) {
+  for (int r = threadIdx.x; r < im.n; r += kSortThreads)
+    A.out_assign[(int64_t)im.b * A.cap + r] = im.assign[r] == kGone ? -2 : (int)im.assign[r];
+}
+
+__global__ void __launch_bounds__(kSortThreads, 1) bbox_vote_kernel(const VoteArgs A) {
+  extern __shared__ __align__(16) unsigned char dyn_smem[];
+  __shared__ int s_cand[32];
+  __shared__ int s_ncand;
+  __shared__ unsigned s_mask[32], s_selfok, s_xs[32], s_ys[32];
+  const VoteRound S = {s_cand, &s_ncand, s_mask, &s_selfok, s_xs, s_ys};
+  const VoteImage im = carve(A, dyn_smem);
+  VoteRegs R;
+  sort_and_gather(A, im, R);
+  const VoteStripes sg = init_stripes(A, R);
+  int cur = 0;
+  while (true) {
+    const int ncand = list_candidates(im, S, cur);
+    if (ncand == 0) break;
+    const int last = S.cand[ncand - 1];
+    candidate_masks(A, im, S, ncand);
+    const unsigned heads = resolve_heads(im, S, sg, ncand);
+    join_heads(A, im, S, R, heads, last);
+    cur = last + 1;
   }
+  __syncthreads();
+  write_groups(A, im, number_groups(A, im));
+  if (A.out_assign) write_assign(A, im);
 }
 
 // detect_face (eval_sfd.py:95-114) for B images of N anchors, in two kernels:
@@ -727,10 +805,10 @@ int dan_bbox_vote(const float* det, const int32_t* counts, int32_t batch, int32_
   A.out_count = out_count;
   A.out_order = out_order;
   A.out_assign = out_assign;
-  const size_t smem = vote_smem_bytes(capacity);
-  DAN_REQUIRE(smem <= 221 * 1024, DAN_ERR_UNSUPPORTED, "capacity %d needs %zu bytes of shared memory", capacity, smem);
-  DAN_CUDA(cudaFuncSetAttribute(bbox_vote_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 221 * 1024));
-  bbox_vote_kernel<<<batch, kSortThreads, smem, (cudaStream_t)stream>>>(A);
+  A.plan = vote_plan(capacity);
+  DAN_REQUIRE(A.plan.smem <= kVoteSmemMax, DAN_ERR_UNSUPPORTED, "capacity %d needs %d bytes of shared memory", capacity, A.plan.smem);
+  DAN_CUDA(cudaFuncSetAttribute(bbox_vote_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kVoteSmemMax));
+  bbox_vote_kernel<<<batch, kSortThreads, A.plan.smem, (cudaStream_t)stream>>>(A);
   DAN_LAUNCH_CHECK("bbox_vote_kernel");
   return DAN_OK;
 }
