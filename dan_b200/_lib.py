@@ -135,6 +135,8 @@ _SIGNATURES = {
     "dan_detect_face_batch": (ctypes.c_int, [c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i32, ctypes.POINTER(c_f32), c_f32,
                                              c_i32, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "dan_bbox_vote": (ctypes.c_int, [c_vp, c_vp, c_i32, c_i32, c_f32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "dan_bbox_vote_workspace_bytes": (c_sz, [c_i32, c_i32]),
+    "dan_bbox_vote_ws": (ctypes.c_int, [c_vp, c_vp, c_i32, c_i32, c_f32, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "dan_gt_handoff": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_f32, c_f32, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp,
                                       c_vp]),
     "dan_peer_alloc": (ctypes.c_int, [c_sz, ctypes.POINTER(c_vp), c_vp]),

@@ -590,9 +590,10 @@ def detect_face_batch(cls_pred, loc_pred, anchors, shrink, top, prior_scaling=(0
     return det, idx, max(min(n - 1, top), 0)
 
 
-def bbox_vote_batch(det, counts, nms_threshold, max_per_image, details=False):
-    """dan_bbox_vote: det [B, cap, 5], counts int32 [B] or None -> (out [B, max_per_image, 5], out_count int32 [B]
-    [, order int32 [B, cap], assign int32 [B, cap]])."""
+def bbox_vote_batch(det, counts, nms_threshold, max_per_image, details=False, workspace=None):
+    """dan_bbox_vote_ws: det [B, cap, 5], counts int32 [B] or None -> (out [B, max_per_image, 5], out_count int32 [B]
+    [, order int32 [B, cap], assign int32 [B, cap]]).  cap <= 2^20; above 8192 the scratch comes from `workspace` (or
+    the per-stream default), nothing is allocated for cap <= 8192."""
     L.require_device()
     dev = _dev(det)
     d = det.contiguous()
@@ -604,10 +605,12 @@ def bbox_vote_batch(det, counts, nms_threshold, max_per_image, details=False):
     order = torch.full((batch, cap), -1, dtype=torch.int32, device=dev) if details else None
     assign = torch.full((batch, cap), -1, dtype=torch.int32, device=dev) if details else None
     c = counts.contiguous() if counts is not None else None
+    nbytes = L.lib().dan_bbox_vote_workspace_bytes(batch, cap)
+    ws = (workspace or _ws).get(nbytes, dev) if nbytes > 0 else None
     with torch.cuda.device(dev):
-        L.check(L.lib().dan_bbox_vote(L.dev_ptr(d, torch.float32, "det"), L.dev_ptr(c, torch.int32, "counts"), batch, cap,
-                                      float(nms_threshold), int(max_per_image), L.dev_ptr(out), L.dev_ptr(cnt),
-                                      L.dev_ptr(order), L.dev_ptr(assign), L.stream_ptr()))
+        L.check(L.lib().dan_bbox_vote_ws(L.dev_ptr(d, torch.float32, "det"), L.dev_ptr(c, torch.int32, "counts"), batch, cap,
+                                         float(nms_threshold), int(max_per_image), L.dev_ptr(out), L.dev_ptr(cnt),
+                                         L.dev_ptr(order), L.dev_ptr(assign), L.dev_ptr(ws), nbytes, L.stream_ptr()))
     return (out, cnt, order, assign) if details else (out, cnt)
 
 

@@ -36,7 +36,8 @@ def detect_face_batch(cls_pred, loc_pred, anchors, shrink, max_per_image=750, pr
 
 
 def bbox_vote(det, nms_threshold=0.3, max_per_image=750):
-    """det [n, 5] -> merged detections [m, 5] (m <= max_per_image).  One host read (m)."""
+    """det [n, 5] -> merged detections [m, 5] (m <= max_per_image).  n <= 2^20: a stack of any number of passes of
+    detect_face (1125 rows each at the default max_per_image).  One host read (m)."""
     det = L.as_f32(det)
     if det.shape[0] == 0:
         return det.new_zeros((0, 5))
@@ -46,5 +47,6 @@ def bbox_vote(det, nms_threshold=0.3, max_per_image=750):
 
 def bbox_vote_batch(det, counts, nms_threshold=0.3, max_per_image=750):
     """Many images at once, nothing synchronises: det [B, capacity, 5] (rows beyond counts[b] are ignored), counts
-    int32 [B] -> (out [B, max_per_image, 5] zero padded, out_count int32 [B])."""
+    int32 [B] or None -> (out [B, max_per_image, 5] zero padded, out_count int32 [B]).  capacity <= 2^20; above 8192
+    the call uses a device workspace of dan_bbox_vote_workspace_bytes(B, capacity) bytes (about 44 bytes per row)."""
     return F.bbox_vote_batch(L.as_f32(det), None if counts is None else counts.to(torch.int32), nms_threshold, max_per_image)

@@ -374,7 +374,19 @@ int dan_dynamic_anchor_routing_eval(const dan_routing_layers* h_layers, const fl
  *   per image (NULL = capacity); out_det [B, max_per_image, 5] zero padded,
  *   out_count [B]; optional out_order / out_assign [B, capacity]: sorted position ->
  *   input row / head position (-2 = head deleted alone), for inspection.
- *   capacity <= 8192 (the stack of multi-scale detections is <= 6 x 1125).
+ *   capacity <= 8192.  A stack of P passes (scales, flips) of 1.5 * max_per_image
+ *   rows each has 1125 P rows at the default 750: the recipe's 4 to 10 passes per
+ *   image give up to 11 250, so dan_bbox_vote_ws is the entry point for stacks.
+ * dan_bbox_vote_ws: dan_bbox_vote with the same arguments and results for
+ *   capacity <= 1048576 (2^20) rows per image; larger capacities are refused with
+ *   DAN_ERR_UNSUPPORTED.  capacity <= 8192 runs the same kernel as dan_bbox_vote and
+ *   needs no workspace (dan_bbox_vote_workspace_bytes returns 0, workspace may be
+ *   NULL).  Above 8192 the detections of each image are sorted and merged in the
+ *   workspace (16-byte aligned, at least dan_bbox_vote_workspace_bytes(batch,
+ *   capacity) bytes, else DAN_ERR_WORKSPACE); the results are the same bits.  The
+ *   path is chosen from capacity alone.  Every check happens before anything is
+ *   enqueued; nothing synchronises, and the call can be captured in a CUDA graph.
+ * dan_bbox_vote_workspace_bytes: bytes for capacity in (8192, 2^20], else 0.
  * ------------------------------------------------------------------------- */
 size_t dan_detect_face_workspace_bytes(int64_t n);
 int dan_detect_face_select(const float* bboxes, const float* scores, int64_t n, float shrink,
@@ -390,6 +402,11 @@ int dan_detect_face_batch(int32_t pred_dtype, const void* cls_pred, const void* 
 int dan_bbox_vote(const float* det, const int32_t* counts, int32_t batch, int32_t capacity,
                   float nms_threshold, int32_t max_per_image, float* out_det, int32_t* out_count,
                   int32_t* out_order, int32_t* out_assign, void* stream);
+size_t dan_bbox_vote_workspace_bytes(int32_t batch, int32_t capacity);
+int dan_bbox_vote_ws(const float* det, const int32_t* counts, int32_t batch, int32_t capacity,
+                     float nms_threshold, int32_t max_per_image, float* out_det,
+                     int32_t* out_count, int32_t* out_order, int32_t* out_assign,
+                     void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------- *
  * (f4, SURVEY.md 8f) input hand-off: the deterministic tail of the training
