@@ -743,6 +743,8 @@ __global__ void __launch_bounds__(kSortThreads, 1) bbox_vote_large_kernel(const 
 //   face_select_kernel  one CTA per image: the histogram gives the bin that holds the k-th key; one pass over the image's
 //                       keys compacts those in that bin or above into shared memory, where they are sorted.  Only the k
 //                       rows are read (or decoded from the offsets), divided by shrink and written.
+//   face_select_large_kernel  the same steps for k > kSortCap (up to kVoteLargeCap): the candidates are compacted into
+//                       the workspace and sorted there with select_and_sort_large (face_large_plan).
 // The score comes from the scores of decoded boxes (dan_detect_face_select) or from the two logits (the softmax in
 // tf.nn.softmax's op order, dan_detect_face_batch); the box from a decoded row or from a decode of the offset row.
 constexpr int kFaceBins = 4096;             // histogram bins per image
@@ -827,79 +829,81 @@ __global__ void __launch_bounds__(kFaceKeyThreads) face_key_kernel(const FaceArg
     if (s_hist[i] != 0) atomicAdd(&hist[i], s_hist[i]);
 }
 
-// eval_sfd.py:101-112, one CTA per image
-template <class Box>
-__global__ void __launch_bounds__(kSortThreads, 1) face_select_kernel(const FaceArgs A, const Box src) {
-  extern __shared__ unsigned long long s_keys[];           // [kSortCap] keys | [kSortCap] merge buffer
-  __shared__ SortScratch sc;
-  __shared__ int s_warp[kSortThreads / 32];
-  __shared__ int s_bin, s_ge;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int b = blockIdx.x;
+// eval_sfd.py:101-112, one CTA per image, in the steps below (both select kernels run them).
+struct FaceBin {
+  int t;                      // the bin of the k-th largest key
+  int ge;                     // keys in bin t or above (>= k)
+};
+
+// 1. the bin t of image b's k-th largest key (k = A.k > 0) and the keys in bin t or above, from the image's histogram:
+// thread i holds bins 4i .. 4i + 3, `above` counts the keys in higher bins.  Also zeroes sc.fill for step 2.
+// s_warp [32], s_bin and s_ge are the kernel's shared memory.  (The steps take the thread, lane and warp index from
+// the kernel, which computes them first: face_select_kernel then compiles to the instructions it had as one function.)
+DAN_D FaceBin face_kth_bin(const FaceArgs& A, int b, int tid, int lane, int warp, SortScratch& sc, int* s_warp, int& s_bin,
+                           int& s_ge) {
   const int k = A.k;
-  const unsigned long long* keys = A.keys + (int64_t)b * A.n;
-  if (k > 0) {
-    // the bin t of the k-th largest key: thread i holds bins 4i .. 4i + 3, `above` counts the keys in higher bins
-    constexpr int kPer = kFaceBins / kSortThreads;
-    const int* hist = A.hist + (int64_t)b * kFaceBins + kPer * tid;
-    const int hb[kPer] = {hist[0], hist[1], hist[2], hist[3]};
-    const int c = hb[0] + hb[1] + hb[2] + hb[3];
-    int incl = c;
+  constexpr int kPer = kFaceBins / kSortThreads;
+  const int* hist = A.hist + (int64_t)b * kFaceBins + kPer * tid;
+  const int hb[kPer] = {hist[0], hist[1], hist[2], hist[3]};
+  const int c = hb[0] + hb[1] + hb[2] + hb[3];
+  int incl = c;
 #pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const int v = __shfl_down_sync(0xffffffffu, incl, d);
-      if (lane + d < 32) incl += v;
+  for (int d = 1; d < 32; d <<= 1) {
+    const int v = __shfl_down_sync(0xffffffffu, incl, d);
+    if (lane + d < 32) incl += v;
+  }
+  if (lane == 0) s_warp[warp] = incl;
+  if (tid == 0) sc.fill = 0;
+  __syncthreads();
+  int above = incl - c;
+  for (int w = warp + 1; w < kSortThreads / 32; ++w) above += s_warp[w];
+  if (above < k && above + c >= k) {                       // exactly one thread: the bins hold all n > k keys
+    int cum = above, t = kPer * tid;
+    for (int j = kPer - 1; j >= 0; --j) {
+      cum += hb[j];
+      if (cum >= k) { t = kPer * tid + j; break; }
     }
-    if (lane == 0) s_warp[warp] = incl;
-    if (tid == 0) sc.fill = 0;
-    __syncthreads();
-    int above = incl - c;
-    for (int w = warp + 1; w < kSortThreads / 32; ++w) above += s_warp[w];
-    if (above < k && above + c >= k) {                     // exactly one thread: the bins hold all n > k keys
-      int cum = above, t = kPer * tid;
-      for (int j = kPer - 1; j >= 0; --j) {
-        cum += hb[j];
-        if (cum >= k) { t = kPer * tid + j; break; }
-      }
-      s_bin = t;
-      s_ge = cum;
+    s_bin = t;
+    s_ge = cum;
+  }
+  __syncthreads();
+  return {s_bin, s_ge};
+}
+
+// 2. one pass over the image's n keys: the ge keys in bin t or above (a superset of the top k) into dst[0, ge) (shared
+// memory or the workspace), in no particular order, one atomic on sc.fill per warp
+DAN_D void face_compact(const unsigned long long* keys, int n, int t, unsigned long long* dst, int tid, int lane, SortScratch& sc) {
+  for (int i0 = 0; i0 < n; i0 += 4 * kSortThreads) {
+    unsigned long long q[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int i = i0 + u * kSortThreads + tid;
+      q[u] = i < n ? __ldcs(keys + i) : 0ull;
     }
-    __syncthreads();
-    const int t = s_bin, ge = s_ge;
-    if (ge <= kSortCap) {
-      // one pass: the ge keys in bin t or above (a superset of the top k) into shared memory, one atomic per warp
-      for (int i0 = 0; i0 < A.n; i0 += 4 * kSortThreads) {
-        unsigned long long q[4];
 #pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const int i = i0 + u * kSortThreads + tid;
-          q[u] = i < A.n ? __ldcs(keys + i) : 0ull;
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const bool keep = i0 + u * kSortThreads + tid < A.n && face_bin(q[u]) >= t;
-          const unsigned m = __ballot_sync(0xffffffffu, keep);
-          if (m != 0u) {
-            int base = 0;
-            if (lane == 0) base = atomicAdd(&sc.fill, __popc(m));
-            base = __shfl_sync(0xffffffffu, base, 0);
-            if (keep) s_keys[base + __popc(m & ((1u << lane) - 1u))] = q[u];
-          }
-        }
+    for (int u = 0; u < 4; ++u) {
+      const bool keep = i0 + u * kSortThreads + tid < n && face_bin(q[u]) >= t;
+      const unsigned m = __ballot_sync(0xffffffffu, keep);
+      if (m != 0u) {
+        int base = 0;
+        if (lane == 0) base = atomicAdd(&sc.fill, __popc(m));
+        base = __shfl_sync(0xffffffffu, base, 0);
+        if (keep) dst[base + __popc(m & ((1u << lane) - 1u))] = q[u];
       }
-      __syncthreads();
-      select_and_sort(keys, ge, k, s_keys, sc, true, s_keys + kSortCap);
-    } else {
-      // more keys share the k-th key's bin than shared memory holds: radix select over all of the image's keys
-      select_and_sort(keys, A.n, k, s_keys, sc, false, s_keys + kSortCap);
     }
   }
+}
+
+// 4. the top rows of image b from its k sorted keys (shared memory or the workspace): the box read or decoded, / shrink,
+// columns (xmin, ymin, xmax, ymax, score); rows k .. top - 1 zero with index -1
+template <class Box>
+DAN_D void face_write_rows(const FaceArgs& A, const Box& src, int b, int k, const unsigned long long* sorted, int tid) {
   float* out = A.out + (int64_t)b * A.top * 5;
   for (int r = tid; r < A.top; r += kSortThreads) {
     float o0 = 0.f, o1 = 0.f, o2 = 0.f, o3 = 0.f, o4 = 0.f;
     int idx = -1;
     if (r < k) {
-      const unsigned long long key = s_keys[r];
+      const unsigned long long key = sorted[r];
       idx = (int)(uint32_t)(key & 0xFFFFFFFFull);
       const float4 bx = src.box((int64_t)b * A.n + idx, idx);
       o0 = fdiv(bx.y, A.shrink); o1 = fdiv(bx.x, A.shrink); o2 = fdiv(bx.w, A.shrink); o3 = fdiv(bx.z, A.shrink);
@@ -911,9 +915,102 @@ __global__ void __launch_bounds__(kSortThreads, 1) face_select_kernel(const Face
   if (tid == 0 && A.out_count) A.out_count[b] = k;
 }
 
+// k <= kSortCap: steps 2 and 3 in shared memory
+template <class Box>
+__global__ void __launch_bounds__(kSortThreads, 1) face_select_kernel(const FaceArgs A, const Box src) {
+  extern __shared__ unsigned long long s_keys[];           // [kSortCap] keys | [kSortCap] merge buffer
+  __shared__ SortScratch sc;
+  __shared__ int s_warp[kSortThreads / 32];
+  __shared__ int s_bin, s_ge;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int b = blockIdx.x;
+  const int k = A.k;
+  const unsigned long long* keys = A.keys + (int64_t)b * A.n;
+  if (k > 0) {
+    const FaceBin fb = face_kth_bin(A, b, tid, lane, warp, sc, s_warp, s_bin, s_ge);
+    if (fb.ge <= kSortCap) {
+      face_compact(keys, A.n, fb.t, s_keys, tid, lane, sc);
+      __syncthreads();
+      select_and_sort(keys, fb.ge, k, s_keys, sc, true, s_keys + kSortCap);     // 3. (the keys are staged)
+    } else {
+      // more keys share the k-th key's bin than shared memory holds: radix select over all of the image's keys
+      select_and_sort(keys, A.n, k, s_keys, sc, false, s_keys + kSortCap);
+    }
+  }
+  face_write_rows(A, src, b, k, s_keys, tid);
+}
+
 constexpr size_t kFaceSelectSmem = 2 * kSortCap * sizeof(unsigned long long);
 
 static size_t face_hist_bytes(int32_t batch) { return align_up((size_t)batch * kFaceBins * sizeof(int), 256); }
+
+// Workspace of face_select_large_kernel (k > kSortCap): one slice per image behind the histograms and the keys.  Offsets
+// of the arrays are in bytes from the start of an image's slice (image * `image`); every array is 256-byte aligned.
+struct FaceLargePlan {
+  size_t region;              // start of the slices in the workspace (= dan_detect_face_batch_workspace_bytes(n, B))
+  size_t image;               // workspace bytes per image
+  size_t sorted;              // [k] u64: the top k keys, sorted (select_and_sort_large's buf_a)
+  size_t topk;                // [k] u64: the top k keys as selected, unsorted (the sort's input)
+  size_t cand;                // [cand_cap] u64: the keys in the k-th key's bin or above (step 2), then the sort's
+                              //   merge buffer (buf_b, k keys)
+  int cand_cap;               // 2k: more candidates (ties in one bin) select over all n keys instead
+};
+
+static FaceLargePlan face_large_plan(int64_t n, int32_t batch, int k) {
+  FaceLargePlan p = {};
+  p.region = face_hist_bytes(batch) + align_up((size_t)n * (size_t)batch * 8, 256);
+  p.cand_cap = 2 * k;
+  size_t off = 0;
+  auto take = [&](size_t bytes) { const size_t at = off; off += align_up(bytes, 256); return at; };
+  p.sorted = take((size_t)k * 8);
+  p.topk = take((size_t)k * 8);
+  p.cand = take((size_t)p.cand_cap * 8);
+  p.image = off;
+  return p;
+}
+
+// k > kSortCap: the candidates are compacted into the workspace and sorted there (runs of kSortCap keys in shared
+// memory, merged in the workspace); ws is the start of the plan's slices
+template <class Box>
+__global__ void __launch_bounds__(kSortThreads, 1) face_select_large_kernel(const FaceArgs A, const Box src, const FaceLargePlan P,
+                                                                            unsigned char* ws) {
+  extern __shared__ unsigned long long s_keys[];           // [kSortCap] the runs of the sort
+  __shared__ SortScratch sc;
+  __shared__ int s_warp[kSortThreads / 32];
+  __shared__ int s_bin, s_ge;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int b = blockIdx.x;
+  const int k = A.k;
+  const unsigned long long* keys = A.keys + (int64_t)b * A.n;
+  unsigned char* slice = ws + (size_t)b * P.image;
+  unsigned long long* sorted = reinterpret_cast<unsigned long long*>(slice + P.sorted);
+  unsigned long long* topk = reinterpret_cast<unsigned long long*>(slice + P.topk);
+  unsigned long long* cand = reinterpret_cast<unsigned long long*>(slice + P.cand);
+  const FaceBin fb = face_kth_bin(A, b, tid, lane, warp, sc, s_warp, s_bin, s_ge);
+  // 3. the k largest of the candidates (or, with more keys in the k-th key's bin than the candidate area holds, of all
+  // n keys) into `topk`, then sorted into `sorted`.  (select_and_sort_large is called with cnt == k, as
+  // bbox_vote_large_kernel calls it: a call with cnt > k in this file changes the instructions of that kernel.)
+  const unsigned long long* from = keys;
+  int cnt = A.n;
+  if (fb.ge <= P.cand_cap) {
+    face_compact(keys, A.n, fb.t, cand, tid, lane, sc);
+    __syncthreads();
+    from = cand;
+    cnt = fb.ge;
+  }
+  const unsigned long long kth = radix_select_kth(from, cnt, k, sc);
+  if (tid == 0) sc.fill = 0;
+  __syncthreads();
+  for (int i = tid; i < cnt; i += kSortThreads) {
+    const unsigned long long key = from[i];
+    if (key >= kth) topk[atomicAdd(&sc.fill, 1)] = key;   // exactly k keys (keys are unique)
+  }
+  __syncthreads();
+  select_and_sort_large(topk, k, k, sorted, cand, s_keys, sc);
+  face_write_rows(A, src, b, k, sorted, tid);
+}
+
+constexpr int kFaceLargeSmem = kSortCap * sizeof(unsigned long long);
 
 template <class Score, class Box>
 static int face_launch(const Score& score, const Box& box, int64_t n, int32_t batch, float shrink, int32_t top, float* out_det,
@@ -933,6 +1030,13 @@ static int face_launch(const Score& score, const Box& box, int64_t n, int32_t ba
     DAN_CUDA(cudaMemsetAsync(A.hist, 0, (size_t)batch * kFaceBins * sizeof(int), st));
     face_key_kernel<Score><<<(unsigned)((int64_t)A.chunks * batch), kFaceKeyThreads, 0, st>>>(A, score);
     DAN_LAUNCH_CHECK("face_key_kernel");
+  }
+  if (A.k > kSortCap) {
+    const FaceLargePlan P = face_large_plan(n, batch, A.k);
+    DAN_CUDA(cudaFuncSetAttribute(face_select_large_kernel<Box>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFaceLargeSmem));
+    face_select_large_kernel<Box><<<batch, kSortThreads, kFaceLargeSmem, st>>>(A, box, P, static_cast<unsigned char*>(workspace) + P.region);
+    DAN_LAUNCH_CHECK("face_select_large_kernel");
+    return DAN_OK;
   }
   DAN_CUDA(cudaFuncSetAttribute(face_select_kernel<Box>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFaceSelectSmem));
   face_select_kernel<Box><<<batch, kSortThreads, kFaceSelectSmem, st>>>(A, box);
@@ -954,6 +1058,54 @@ static int face_batch_launch(const void* cls_pred, const void* loc_pred, const f
   return face_launch(score, box, n, batch, shrink, top, out_det, out_index, nullptr, workspace, st);
 }
 
+// dan_detect_face_select and dan_detect_face_select_top: the same checks, top in [1, top_cap]
+static int face_select_checked(const float* bboxes, const float* scores, int64_t n, float shrink, int32_t top, int32_t top_cap,
+                        float* out_det, int32_t* out_index, int32_t* out_count, void* workspace, size_t workspace_bytes, void* stream) {
+  DAN_REQUIRE(n >= 0 && n < ((int64_t)1 << 31), DAN_ERR_INVALID_ARGUMENT, "bad n");
+  DAN_REQUIRE(top >= 1 && top <= top_cap, DAN_ERR_UNSUPPORTED, "top must be in [1, %d]", top_cap);
+  DAN_REQUIRE(out_det && out_count, DAN_ERR_INVALID_ARGUMENT, "NULL output");
+  DAN_REQUIRE(n == 0 || (bboxes && scores && aligned16(bboxes)), DAN_ERR_INVALID_ARGUMENT, "NULL / misaligned input");
+  const size_t need = dan_detect_face_top_workspace_bytes(n, 1, top);
+  DAN_REQUIRE(n == 0 || (workspace != nullptr && workspace_bytes >= need), DAN_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu",
+              need, workspace_bytes);
+  FaceScores score = {scores};
+  FaceBoxes box = {reinterpret_cast<const float4*>(bboxes)};
+  return face_launch(score, box, n, 1, shrink, top, out_det, out_index, out_count, workspace, (cudaStream_t)stream);
+}
+
+// dan_detect_face_batch and dan_detect_face_batch_top: the same checks, top in [1, top_cap]
+static int face_batch_checked(int32_t pred_dtype, const void* cls_pred, const void* loc_pred, const float* a_ymin, const float* a_xmin,
+                       const float* a_ymax, const float* a_xmax, int64_t num_anchors, int32_t batch, const float* h_prior_scaling,
+                       float shrink, int32_t top, int32_t top_cap, float* out_det, int32_t* out_index, void* workspace,
+                       size_t workspace_bytes, void* stream) {
+  const int esize = dtype_bytes(pred_dtype);
+  DAN_REQUIRE(esize != 0, DAN_ERR_INVALID_ARGUMENT, "unknown pred_dtype %d", pred_dtype);
+  DAN_REQUIRE(num_anchors >= 0 && num_anchors < ((int64_t)1 << 31) && batch >= 0, DAN_ERR_INVALID_ARGUMENT, "bad num_anchors / batch");
+  DAN_REQUIRE(top >= 1 && top <= top_cap, DAN_ERR_UNSUPPORTED, "top must be in [1, %d]", top_cap);
+  if (batch == 0) return DAN_OK;
+  DAN_REQUIRE(cls_pred && loc_pred && a_ymin && a_xmin && a_ymax && a_xmax && h_prior_scaling && out_det, DAN_ERR_INVALID_ARGUMENT,
+              "NULL pointer");
+  DAN_REQUIRE((reinterpret_cast<uintptr_t>(loc_pred) & (uintptr_t)(4 * esize - 1)) == 0, DAN_ERR_INVALID_ARGUMENT,
+              "loc_pred must be %d-byte aligned", 4 * esize);
+  const int64_t chunks = (num_anchors + kFaceChunk - 1) / kFaceChunk;
+  DAN_REQUIRE(chunks * batch < ((int64_t)1 << 31), DAN_ERR_UNSUPPORTED, "batch x num_anchors too large");
+  const size_t need = dan_detect_face_top_workspace_bytes(num_anchors, batch, top);
+  DAN_REQUIRE(workspace != nullptr && workspace_bytes >= need, DAN_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need,
+              workspace_bytes);
+  cudaStream_t st = (cudaStream_t)stream;
+  switch (pred_dtype) {
+    case DAN_DTYPE_F16:
+      return face_batch_launch<__half>(cls_pred, loc_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling, shrink, top,
+                                       out_det, out_index, workspace, st);
+    case DAN_DTYPE_BF16:
+      return face_batch_launch<__nv_bfloat16>(cls_pred, loc_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling, shrink,
+                                              top, out_det, out_index, workspace, st);
+    default:
+      return face_batch_launch<float>(cls_pred, loc_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling, shrink, top,
+                                      out_det, out_index, workspace, st);
+  }
+}
+
 }  // namespace
 
 }  // namespace dan
@@ -969,50 +1121,41 @@ size_t dan_detect_face_batch_workspace_bytes(int64_t num_anchors, int32_t batch)
 
 size_t dan_detect_face_workspace_bytes(int64_t n) { return dan_detect_face_batch_workspace_bytes(n, 1); }
 
+size_t dan_detect_face_top_workspace_bytes(int64_t num_anchors, int32_t batch, int32_t top) {
+  if (num_anchors < 0 || batch < 0) return 0;
+  const int64_t k = num_anchors - 1 < top ? (num_anchors - 1 > 0 ? num_anchors - 1 : 0) : top;
+  const size_t base = dan_detect_face_batch_workspace_bytes(num_anchors, batch);
+  if (top > kVoteLargeCap) return 0;
+  if (k <= kSortCap) return base;
+  return base + (size_t)batch * face_large_plan(num_anchors, batch, (int)k).image;
+}
+
 int dan_detect_face_select(const float* bboxes, const float* scores, int64_t n, float shrink, int32_t top, float* out_det,
                            int32_t* out_index, int32_t* out_count, void* workspace, size_t workspace_bytes, void* stream) {
-  DAN_REQUIRE(n >= 0 && n < ((int64_t)1 << 31), DAN_ERR_INVALID_ARGUMENT, "bad n");
-  DAN_REQUIRE(top >= 1 && top <= kSortCap, DAN_ERR_UNSUPPORTED, "top must be in [1, %d]", kSortCap);
-  DAN_REQUIRE(out_det && out_count, DAN_ERR_INVALID_ARGUMENT, "NULL output");
-  DAN_REQUIRE(n == 0 || (bboxes && scores && aligned16(bboxes)), DAN_ERR_INVALID_ARGUMENT, "NULL / misaligned input");
-  const size_t need = dan_detect_face_workspace_bytes(n);
-  DAN_REQUIRE(n == 0 || (workspace != nullptr && workspace_bytes >= need), DAN_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu",
-              need, workspace_bytes);
-  FaceScores score = {scores};
-  FaceBoxes box = {reinterpret_cast<const float4*>(bboxes)};
-  return face_launch(score, box, n, 1, shrink, top, out_det, out_index, out_count, workspace, (cudaStream_t)stream);
+  return face_select_checked(bboxes, scores, n, shrink, top, kSortCap, out_det, out_index, out_count, workspace, workspace_bytes,
+                             stream);
+}
+
+int dan_detect_face_select_top(const float* bboxes, const float* scores, int64_t n, float shrink, int32_t top, float* out_det,
+                               int32_t* out_index, int32_t* out_count, void* workspace, size_t workspace_bytes, void* stream) {
+  return face_select_checked(bboxes, scores, n, shrink, top, kVoteLargeCap, out_det, out_index, out_count, workspace,
+                             workspace_bytes, stream);
 }
 
 int dan_detect_face_batch(int32_t pred_dtype, const void* cls_pred, const void* loc_pred, const float* a_ymin, const float* a_xmin,
                           const float* a_ymax, const float* a_xmax, int64_t num_anchors, int32_t batch, const float* h_prior_scaling,
                           float shrink, int32_t top, float* out_det, int32_t* out_index, void* workspace, size_t workspace_bytes,
                           void* stream) {
-  const int esize = dtype_bytes(pred_dtype);
-  DAN_REQUIRE(esize != 0, DAN_ERR_INVALID_ARGUMENT, "unknown pred_dtype %d", pred_dtype);
-  DAN_REQUIRE(num_anchors >= 0 && num_anchors < ((int64_t)1 << 31) && batch >= 0, DAN_ERR_INVALID_ARGUMENT, "bad num_anchors / batch");
-  DAN_REQUIRE(top >= 1 && top <= kSortCap, DAN_ERR_UNSUPPORTED, "top must be in [1, %d]", kSortCap);
-  if (batch == 0) return DAN_OK;
-  DAN_REQUIRE(cls_pred && loc_pred && a_ymin && a_xmin && a_ymax && a_xmax && h_prior_scaling && out_det, DAN_ERR_INVALID_ARGUMENT,
-              "NULL pointer");
-  DAN_REQUIRE((reinterpret_cast<uintptr_t>(loc_pred) & (uintptr_t)(4 * esize - 1)) == 0, DAN_ERR_INVALID_ARGUMENT,
-              "loc_pred must be %d-byte aligned", 4 * esize);
-  const int64_t chunks = (num_anchors + kFaceChunk - 1) / kFaceChunk;
-  DAN_REQUIRE(chunks * batch < ((int64_t)1 << 31), DAN_ERR_UNSUPPORTED, "batch x num_anchors too large");
-  const size_t need = dan_detect_face_batch_workspace_bytes(num_anchors, batch);
-  DAN_REQUIRE(workspace != nullptr && workspace_bytes >= need, DAN_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", need,
-              workspace_bytes);
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (pred_dtype) {
-    case DAN_DTYPE_F16:
-      return face_batch_launch<__half>(cls_pred, loc_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling, shrink, top,
-                                       out_det, out_index, workspace, st);
-    case DAN_DTYPE_BF16:
-      return face_batch_launch<__nv_bfloat16>(cls_pred, loc_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling, shrink,
-                                              top, out_det, out_index, workspace, st);
-    default:
-      return face_batch_launch<float>(cls_pred, loc_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling, shrink, top,
-                                      out_det, out_index, workspace, st);
-  }
+  return face_batch_checked(pred_dtype, cls_pred, loc_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling,
+                            shrink, top, kSortCap, out_det, out_index, workspace, workspace_bytes, stream);
+}
+
+int dan_detect_face_batch_top(int32_t pred_dtype, const void* cls_pred, const void* loc_pred, const float* a_ymin,
+                              const float* a_xmin, const float* a_ymax, const float* a_xmax, int64_t num_anchors, int32_t batch,
+                              const float* h_prior_scaling, float shrink, int32_t top, float* out_det, int32_t* out_index,
+                              void* workspace, size_t workspace_bytes, void* stream) {
+  return face_batch_checked(pred_dtype, cls_pred, loc_pred, a_ymin, a_xmin, a_ymax, a_xmax, num_anchors, batch, h_prior_scaling,
+                            shrink, top, kVoteLargeCap, out_det, out_index, workspace, workspace_bytes, stream);
 }
 
 size_t dan_bbox_vote_workspace_bytes(int32_t batch, int32_t capacity) {

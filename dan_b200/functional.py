@@ -538,7 +538,8 @@ def dynamic_anchor_routing_eval(layers, anchors, gt_targets, labels, mask_in, wo
 # evaluation merge: detect_face top-k + bbox_vote (SURVEY.md 8(f2))
 # ----------------------------------------------------------------------------------
 def detect_face_select(bboxes, scores, shrink, top):
-    """dan_detect_face_select -> (det [top, 5] zero padded, index int32 [top] (-1 padded), count int32 [1])."""
+    """dan_detect_face_select_top -> (det [top, 5] zero padded, index int32 [top] (-1 padded), count int32 [1]).
+    top <= 2^20; above 8192 rows the sort runs in a larger workspace."""
     L.require_device()
     dev = _dev(bboxes)
     b = bboxes.contiguous()
@@ -547,12 +548,12 @@ def detect_face_select(bboxes, scores, shrink, top):
     det = torch.empty((top, 5), dtype=torch.float32, device=dev)
     idx = torch.empty(top, dtype=torch.int32, device=dev)
     cnt = torch.empty(1, dtype=torch.int32, device=dev)
-    nbytes = L.lib().dan_detect_face_workspace_bytes(n)
+    nbytes = L.lib().dan_detect_face_top_workspace_bytes(n, 1, int(top))
     ws = _ws.get(nbytes, dev)
     with torch.cuda.device(dev):
-        L.check(L.lib().dan_detect_face_select(L.dev_ptr(b, torch.float32, "bboxes"), L.dev_ptr(s, torch.float32, "scores"), n,
-                                               float(shrink), int(top), L.dev_ptr(det), L.dev_ptr(idx), L.dev_ptr(cnt),
-                                               L.dev_ptr(ws), nbytes, L.stream_ptr()))
+        L.check(L.lib().dan_detect_face_select_top(L.dev_ptr(b, torch.float32, "bboxes"), L.dev_ptr(s, torch.float32, "scores"), n,
+                                                   float(shrink), int(top), L.dev_ptr(det), L.dev_ptr(idx), L.dev_ptr(cnt),
+                                                   L.dev_ptr(ws), nbytes, L.stream_ptr()))
     return det, idx, cnt
 
 
@@ -560,7 +561,8 @@ def detect_face_batch(cls_pred, loc_pred, anchors, shrink, top, prior_scaling=(0
     """dan_detect_face_batch: softmax + decode + detect_face of B images from the head's raw outputs, fused.
     cls_pred [B, N, 2] logits and loc_pred [B, N, 4] offsets, one dtype out of fp32 / fp16 / bf16; anchors =
     (ymin, xmin, ymax, xmax) [N] each.  -> (det [B, top, 5] zero padded, index int32 [B, top] (-1 padded), k) where
-    k = max(min(N - 1, top), 0) valid rows per image.  Nothing synchronises with the host."""
+    k = max(min(N - 1, top), 0) valid rows per image.  top <= 2^20 (dan_detect_face_batch_top; above 8192 rows the
+    workspace holds each image's sort).  Nothing synchronises with the host."""
     L.require_device()
     cls_pred = cls_pred.contiguous()
     loc_pred = loc_pred.contiguous()
@@ -579,14 +581,14 @@ def detect_face_batch(cls_pred, loc_pred, anchors, shrink, top, prior_scaling=(0
     top = int(top)
     det = torch.empty((batch, top, 5), dtype=torch.float32, device=dev)
     idx = torch.empty((batch, top), dtype=torch.int32, device=dev)
-    nbytes = L.lib().dan_detect_face_batch_workspace_bytes(n, batch)
+    nbytes = L.lib().dan_detect_face_top_workspace_bytes(n, batch, top)
     ws = (workspace or _ws).get(nbytes, dev)
     ps = (ctypes.c_float * 4)(*[float(v) for v in prior_scaling])
     with torch.cuda.device(dev):
-        L.check(L.lib().dan_detect_face_batch(dtype, L.dev_ptr(cls_pred, cls_pred.dtype, "cls_pred"),
-                                              L.dev_ptr(loc_pred, cls_pred.dtype, "loc_pred"), *_anchor_ptrs(*anchors), n, batch,
-                                              ps, float(shrink), top, L.dev_ptr(det), L.dev_ptr(idx), L.dev_ptr(ws), nbytes,
-                                              L.stream_ptr()))
+        L.check(L.lib().dan_detect_face_batch_top(dtype, L.dev_ptr(cls_pred, cls_pred.dtype, "cls_pred"),
+                                                  L.dev_ptr(loc_pred, cls_pred.dtype, "loc_pred"), *_anchor_ptrs(*anchors), n, batch,
+                                                  ps, float(shrink), top, L.dev_ptr(det), L.dev_ptr(idx), L.dev_ptr(ws), nbytes,
+                                                  L.stream_ptr()))
     return det, idx, max(min(n - 1, top), 0)
 
 

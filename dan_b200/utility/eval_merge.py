@@ -18,7 +18,8 @@ from .. import functional as F
 def detect_face_select(bboxes, scores, shrink, max_per_image=750):
     """bboxes [n, 4] (ymin, xmin, ymax, xmax) and scores [n] as returned by the network -> det [k, 5] with
     k = min(n - 1, int(max_per_image * 1.5)), sorted by descending score (equal scores: higher index first; the
-    reference's default argsort leaves ties unspecified).  One host read (k)."""
+    reference's default argsort leaves ties unspecified).  max_per_image <= 65535, bbox_vote's own limit (k <= 98302).
+    One host read (k)."""
     top = int(max_per_image * 1.5)
     det, _, cnt = F.detect_face_select(L.as_f32(bboxes), L.as_f32(scores), shrink, top)
     return det[:int(cnt)]
@@ -29,8 +30,9 @@ def detect_face_batch(cls_pred, loc_pred, anchors, shrink, max_per_image=750, pr
     detect_face (:95-114) - for a batch, from the head's raw outputs: cls_pred [B, N, 2] logits and loc_pred [B, N, 4]
     offsets (fp32, fp16 or bf16, one dtype), anchors (ymin, xmin, ymax, xmax) -> det [B, k, 5] rows
     (xmin, ymin, xmax, ymax, score) with k = min(N - 1, int(max_per_image * 1.5)), sorted by descending score (equal
-    scores: higher index first).  No host read: the passes of one batch (scales, flips) are stacked with
-    torch.cat(dim=1) and go straight into bbox_vote_batch(det, None)."""
+    scores: higher index first).  max_per_image <= 65535, bbox_vote's own limit (k <= 98302; above 8192 rows the
+    workspace holds each image's sort, about 32 bytes per row).  No host read: the passes of one batch (scales, flips)
+    are stacked with torch.cat(dim=1) and go straight into bbox_vote_batch(det, None)."""
     det, _, k = F.detect_face_batch(cls_pred, loc_pred, anchors, shrink, int(max_per_image * 1.5), prior_scaling)
     return det[:, :k]
 

@@ -369,6 +369,24 @@ int dan_dynamic_anchor_routing_eval(const dan_routing_layers* h_layers, const fl
  *   nothing N-sized but one 8-byte key per anchor reaches memory.  top in [1, 8192],
  *   N < 2^31, loc_pred rows 16-byte (fp32) / 8-byte (fp16, bf16) aligned; cls_pred
  *   needs no alignment beyond its element type.  batch == 0 enqueues nothing.
+ * dan_detect_face_batch_top / dan_detect_face_select_top: dan_detect_face_batch /
+ *   dan_detect_face_select with the same arguments, checks and results for top in
+ *   [1, 1048576] (2^20, the most rows per image dan_bbox_vote_ws merges; larger or
+ *   smaller top: DAN_ERR_UNSUPPORTED), e.g. top 98 302 for max_per_image 65 535.
+ *   Every image still gets k = max(min(N - 1, top), 0) rows.  k <= 8192 runs the
+ *   same kernels as the calls without _top; above 8192 the candidates of each image
+ *   are selected and sorted in the workspace, with the same bits.  The path is
+ *   chosen from k alone.  Workspace: dan_detect_face_top_workspace_bytes(N, B, top)
+ *   (B = 1 for _select_top), else DAN_ERR_WORKSPACE.  Every check happens before
+ *   anything is enqueued; nothing synchronises, the calls can be captured in a CUDA
+ *   graph, and batch == 0 enqueues nothing.  Output offsets are 64-bit, so B x top
+ *   needs no bound of its own.
+ * dan_detect_face_top_workspace_bytes: for k <= 8192 the same as
+ *   dan_detect_face_batch_workspace_bytes(N, B); for k > 8192 that plus
+ *   B x (align256(8 k) sorted keys + align256(8 k) selected keys + align256(16 k)
+ *   candidates, which the sort reuses as its merge buffer), where align256 rounds up
+ *   to a multiple of 256: about 32 bytes per row of k, never O(N).  0 for top > 2^20
+ *   or N, B < 0.
  * dan_bbox_vote: bbox_vote (eval_sfd.py:170-210 = eval_dan.py:201-241), batched:
  *   det [B, capacity, 5] rows (xmin, ymin, xmax, ymax, score), counts [B] valid rows
  *   per image (NULL = capacity); out_det [B, max_per_image, 5] zero padded,
@@ -399,6 +417,17 @@ int dan_detect_face_batch(int32_t pred_dtype, const void* cls_pred, const void* 
                           const float* h_prior_scaling, float shrink, int32_t top,
                           float* out_det, int32_t* out_index, void* workspace,
                           size_t workspace_bytes, void* stream);
+size_t dan_detect_face_top_workspace_bytes(int64_t num_anchors, int32_t batch, int32_t top);
+int dan_detect_face_batch_top(int32_t pred_dtype, const void* cls_pred, const void* loc_pred,
+                              const float* a_ymin, const float* a_xmin, const float* a_ymax,
+                              const float* a_xmax, int64_t num_anchors, int32_t batch,
+                              const float* h_prior_scaling, float shrink, int32_t top,
+                              float* out_det, int32_t* out_index, void* workspace,
+                              size_t workspace_bytes, void* stream);
+int dan_detect_face_select_top(const float* bboxes, const float* scores, int64_t n, float shrink,
+                               int32_t top, float* out_det, int32_t* out_index,
+                               int32_t* out_count, void* workspace, size_t workspace_bytes,
+                               void* stream);
 int dan_bbox_vote(const float* det, const int32_t* counts, int32_t batch, int32_t capacity,
                   float nms_threshold, int32_t max_per_image, float* out_det, int32_t* out_count,
                   int32_t* out_order, int32_t* out_assign, void* stream);
