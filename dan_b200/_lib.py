@@ -11,7 +11,7 @@ import os
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# DAN_B200_LIB: an alternative build of the same library (tuning experiments, tools/variant.sh)
+# DAN_B200_LIB: load another build of the same library instead (A/B runs of two builds, e.g. a change against its parent)
 LIB_PATH = os.environ.get("DAN_B200_LIB") or os.path.join(_HERE, "libdan_b200.so")
 
 DAN_MAX_LAYERS = 16

@@ -6,16 +6,20 @@
 //     pass 1  enc_pass1_fused_kernel: everything that depends on ONE anchor - row maximum / argmax, stage 1 of the
 //             matcher, labels, encode, ALL outputs (44 B/anchor) - plus the per-GT column maxima (atomicMax on fp32
 //             bit patterns), the per-GT match counts and, mining, the stage-3 candidates in per-GT buckets
+//             (pass1_task: a CTA's chunk of anchors and images; load_warp_anchors: its anchors and warp box)
 //     pass 2  enc_pass2_find_kernel + enc_pass2_apply_kernel: stage 2 (mining) / the GT-side claim (dual) as a patch
-//             of the few anchors whose overlap reaches a GT's column maximum
+//             of the few anchors whose overlap reaches a GT's column maximum (DESIGN.md §4a).  Find: summarize_columns,
+//             list_reaching_warps (level 1), flag_box_hits (level 2), enqueue_flagged; apply: walk_gts twice, stage2_match
 //   dense path  (dan_small_mining_match / dan_dual_max_match): the literal custom op boundary, the overlaps [N,M] of
-//               one image given in HBM and read in 32 x 32 tiles transposed through shared memory:
+//               one image given in HBM and read in 32 x 32 tiles transposed through shared memory (load_tile):
 //     pass 1  dense_pass1_kernel: per-GT column maxima (dual with gt_max_first = 0: which GTs have an anchor-side
 //             positive)
 //     pass 2  dense_pass2_kernel: per anchor, stage 1 from the row maximum, stage 2 / the claim against the column
-//             maxima, match and score; mining: the anchors still unmatched push their candidates to per-GT buckets
+//             maxima (stage2_match), match and score; mining: the anchors still unmatched push their candidates to
+//             per-GT buckets
 //   pass 3  (mining only, both paths) stage 3 "hard face compensation": one CTA per image walks the GTs in ascending
 //           order (the stage is order dependent, small_mining_match.cc:199-222) and patches the few affected anchors
+//           (list_needy; per window window_end, load_window, resolve_window, apply_window; or rescan_overflowed)
 //
 // Culling (fused path): a warp owns 32 consecutive anchors; it reduces their
 // bounding box with redux.sync and tests 32 GT boxes per ballot against it.  Only
@@ -238,11 +242,38 @@ DAN_D int stage1_match(const EncArgs& A, float best, int best_gt) {
   return match;
 }
 
+// stage 1, then stage 2 of the mining matcher (small_mining_match.cc:178-186: the last tied GT wins) / the GT-side claim
+// of the dual matcher (anchor_manipulator.py:95-104: argmax over overlap * claim mask; GT 0 if claimed only through
+// zero-overlap ties) for the row in `s`: the match, and its score in `score`
+template <bool MINING>
+DAN_D int stage2_match(const EncArgs& A, const RowState& s, float& score) {
+  int match = stage1_match<MINING>(A, s.best, s.best_gt);
+  score = s.best;
+  if (MINING) {
+    if (s.owner >= 0) { match = s.owner; score = s.owner_ov; }
+  } else if (s.claimed) {
+    if (s.cbest > 0.f) { match = s.cbest_gt; score = s.cbest; }
+    else { match = 0; score = s.ov0; }
+  }
+  return match;
+}
+
 // ---------------------------------------------------------------------------
 // dense path, passes 1 and 2, on the overlaps [n, m_dense] of one image.  A warp owns 32 consecutive anchors (rows)
 // and reads the matrix in 32 x 32 tiles through shared memory (row stride 33: conflict-free both ways), so that a lane
 // holds a column for the column maxima and a row for the row maxima.
 // ---------------------------------------------------------------------------
+// the warp's tile of rows [row0, row0 + 32) and columns [j0, j0 + 32) of the [A.n, m] matrix, zero outside it: lane l
+// loads column j0 + l of every row
+DAN_D void load_tile(const EncArgs& A, int m, float* tile, int row0, int j0, int lane) {
+  const int jc = j0 + lane;
+  for (int r = 0; r < 32; ++r) {
+    const int row = row0 + r;
+    tile[r * 33 + lane] = (row < A.n && jc < m) ? A.overlaps[(int64_t)row * m + jc] : 0.f;
+  }
+  __syncwarp();
+}
+
 template <bool NEED_ROW>
 __global__ void __launch_bounds__(kEncThreads) dense_pass1_kernel(const EncArgs A) {
   __shared__ float s_tile[(kEncThreads / 32) * 32 * 33];
@@ -258,12 +289,8 @@ __global__ void __launch_bounds__(kEncThreads) dense_pass1_kernel(const EncArgs 
   float best = 0.f;
   int best_gt = 0;
   for (int j0 = 0; j0 < m; j0 += 32) {
+    load_tile(A, m, tile, row0, j0, lane);
     const int jc = j0 + lane;
-    for (int r = 0; r < 32; ++r) {
-      const int row = row0 + r;
-      tile[r * 33 + lane] = (row < A.n && jc < m) ? A.overlaps[(int64_t)row * m + jc] : 0.f;
-    }
-    __syncwarp();
     // column maximum of the 32x32 tile: lane == column
     float cmx = 0.f;
     for (int r = 0; r < 32; ++r) cmx = fmaxf(cmx, tile[r * 33 + lane]);
@@ -308,12 +335,7 @@ __global__ void __launch_bounds__(kEncThreads) dense_pass2_kernel(const EncArgs 
   for (int round = 0; round < 2; ++round) {
     if (row0 < A.n && (round == 0 || warp_push)) {
       for (int j0 = 0; j0 < m; j0 += 32) {
-        const int jc = j0 + lane;
-        for (int r = 0; r < 32; ++r) {
-          const int row = row0 + r;
-          tile[r * 33 + lane] = (row < A.n && jc < m) ? A.overlaps[(int64_t)row * m + jc] : 0.f;
-        }
-        __syncwarp();
+        load_tile(A, m, tile, row0, j0, lane);
         const int lim = min(32, m - j0);
         for (int jj = 0; jj < lim; ++jj) {
           const int j = j0 + jj;
@@ -334,17 +356,10 @@ __global__ void __launch_bounds__(kEncThreads) dense_pass2_kernel(const EncArgs 
     if (round == 1) break;
 
     // ---- resolve this anchor (end of round 0)
-    match = stage1_match<MINING>(A, s.best, s.best_gt);
-    score = s.best;
+    match = stage2_match<MINING>(A, s, score);
     if (MINING) {
-      // stage 2, small_mining_match.cc:178-186
-      if (s.owner >= 0) { match = s.owner; score = s.owner_ov; }
       if (valid && match >= 0) atomicAdd(A.cnt + match, 1);
       push_round = valid && match < 0 && s.best > A.stop;
-    } else if (s.claimed) {
-      // anchor_manipulator.py:95-104 GT-side claim has priority; argmax over (overlap * claim mask)
-      if (s.cbest > 0.f) { match = s.cbest_gt; score = s.cbest; }
-      else { match = 0; score = s.ov0; }
     }
     // round 1 runs only in CTAs with a pushing anchor, and there only in the warps that hold one
     if (!MINING || !__syncthreads_or(push_round ? 1 : 0)) break;
@@ -395,33 +410,12 @@ DAN_D bool may_hit(const WarpBox& wb, float4 g) {
 // ---------------------------------------------------------------------------
 constexpr int kFusedThreads = 128;
 
-// Timeline of fused pass 1, for tools/pass1_timeline.py: with -DDAN_PASS1_TIMELINE lane 0 of every warp writes the
-// global timer (ns) at its start and end and the number of images it walked; otherwise the macros are empty.
-#ifdef DAN_PASS1_TIMELINE
-constexpr int kTimelineWarps = 1 << 16;
-__device__ unsigned long long g_p1_timeline[3 * kTimelineWarps];
-DAN_D unsigned long long global_ns() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-#define DAN_P1_MARK(slot, value)                                                          \
-  do {                                                                                    \
-    const unsigned w__ = blockIdx.x * (kFusedThreads / 32) + (threadIdx.x >> 5);        \
-    if ((threadIdx.x & 31) == 0 && w__ < kTimelineWarps) g_p1_timeline[3 * w__ + (slot)] = (value); \
-  } while (0)
-#else
-#define DAN_P1_MARK(slot, value) do { } while (0)
-#endif
 // Images per CTA of pass 1 on the fine levels.  A warp there meets ~2 GTs per image (~150 warp instructions) against
 // ~350 instructions of per-(warp, image) bookkeeping, so it walks several images; a warp of a coarse level meets every
 // GT of the image and keeps one, so that it does not become the tail of the launch (profiles/r03_pass1_breakdown.md).
 // Measured on B200 at batch 32: 2 images give back 3.5 % of the rate with steps in flight, 8 add 1 % to it but make a
 // lone pass 1 30 % longer.
-#ifndef DAN_ENC_FINE_IMAGES
-#define DAN_ENC_FINE_IMAGES 4
-#endif
-constexpr int kFineImages = DAN_ENC_FINE_IMAGES;
+constexpr int kFineImages = 4;
 // a hinted level of at least this many cells (32 warps) counts as fine: at 640^2 the 160^2 / 80^2 / 40^2 levels
 // (2.1 / 2.7 / 4.4 culled GTs per warp and image), not the 20^2 one (11.8)
 constexpr int kFineMinCells = 1024;
@@ -489,28 +483,17 @@ DAN_D void write_negative(const EncArgs& A, int64_t row, const AnchorCtr& ac, Ra
   if (A.match32 != nullptr) __stcs(A.match32 + row, match);
 }
 
-// pass 1 (fused path): everything that depends on ONE anchor only - row maximum / argmax, stage 1 of the matcher,
-// labels, encode, ALL outputs - plus the two cross-anchor quantities the later passes need: the per-GT column maxima
-// (atomicMax) and, for the mining matcher, the stage-3 candidates (overlap > stop_positive_thres) and the per-GT
-// match counts.  What stage 2 / the GT-side claim of the dual matcher changes afterwards is a handful of anchors per
-// GT; pass 2 finds and patches them.
-// TILED: the warps hold the tiles of the layout hint (A.warp_map != NULL); a separate instantiation because the kernel
-// sits on its register cap and the strip version can derive everything from threadIdx
-#ifndef DAN_ENC_TILED_BLOCKS
-#define DAN_ENC_TILED_BLOCKS 6   // 40 registers: no spills (A/B on B200: +1 % over the 32-register build)
-#endif
-template <bool NEED_ROW, bool MINING, bool TILED>
-__global__ void __launch_bounds__(kEncThreads, TILED ? DAN_ENC_TILED_BLOCKS : 6)
-enc_pass1_fused_kernel(const EncArgs A, int batch, int coarse_chunks) {
-  DAN_P1_MARK(0, global_ns());
-  const int lane = threadIdx.x & 31;
-  const int nwarps = (A.n + 31) >> 5;
-  const int nchunks = (A.n + kFusedThreads - 1) / kFusedThreads;
-  // CTA -> (anchor chunk, images [b0, b_end)).  The chunks are walked from the END of the anchor array: the coarse
-  // pyramid levels live there, their warps see every GT and run the longest, so they must not be the tail of the
-  // launch.  The last `coarse_chunks` chunks come first, one CTA per image, all images of a chunk next to each other;
-  // then the fine chunks, one CTA per group of kFineImages images.  Fine chunks exist only with the layout hint, i.e. in
-  // the TILED instantiation.
+// CTA -> (anchor chunk, images [b0, b_end)) of pass 1.  The chunks are walked from the END of the anchor array: the
+// coarse pyramid levels live there, their warps see every GT and run the longest, so they must not be the tail of the
+// launch.  The last `coarse_chunks` chunks come first, one CTA per image, all images of a chunk next to each other; then
+// the fine chunks, one CTA per group of kFineImages images.  Fine chunks exist only with the layout hint, i.e. in the
+// TILED instantiation.  pass1_grid() is the host's count of these CTAs.
+struct Pass1Task {
+  int from_end, b0, b_end;    // the anchor chunk, counted from the end of the anchor array; the images of the CTA
+};
+
+template <bool TILED>
+DAN_D Pass1Task pass1_task(int batch, int coarse_chunks) {
   int from_end, b0, b_end;
   const int coarse_ctas = coarse_chunks * batch;
   if (!TILED || (int)blockIdx.x < coarse_ctas) {
@@ -525,20 +508,56 @@ enc_pass1_fused_kernel(const EncArgs A, int batch, int coarse_chunks) {
     b0 = (j - c * groups) * kFineImages;
     b_end = min(batch, b0 + kFineImages);
   }
-  // the warp's index (wbest / wbox / queue entries are per warp) and its anchors
-  const int wid = (nchunks - 1 - from_end) * (kFusedThreads / 32) + (threadIdx.x >> 5);
-  const int a = TILED ? ((wid < nwarps) ? warp_anchor(A, wid, lane) : A.n) : wid * 32 + lane;
-  const bool valid = a < A.n;
-  AnchorBox ab = {};
-  AnchorCtr ac = {};
-  bool active = false;
+  return {from_end, b0, b_end};
+}
+
+static int pass1_grid(int batch, int coarse_chunks, int fine_chunks) {
+  return coarse_chunks * batch + fine_chunks * ((batch + kFineImages - 1) / kFineImages);
+}
+
+// The anchor a of this lane of pass 1 (valid: a < A.n) in its matching and centre forms and whether the mask keeps it,
+// loaded once for all the images of the CTA, and the bounding box of the warp's active anchors, which the CTA of image 0
+// stores for pass 2
+DAN_D void load_warp_anchors(const EncArgs& A, int a, bool valid, int wid, int nwarps, int b0, int lane, AnchorBox& ab,
+                             AnchorCtr& ac, bool& active, WarpBox& wb) {
+  ab = {};
+  ac = {};
+  active = false;
   if (valid) {
     ab = load_anchor(A, a);
     ac = anchor_ctr(ab.y0, ab.x0, ab.y1, ab.x1);
     active = (A.mask == nullptr) || (A.mask[a] != 0);
   }
-  const WarpBox wb = warp_bbox(active, ab);
+  wb = warp_bbox(active, ab);
   if (b0 == 0 && lane == 0 && wid < nwarps) A.wbox[wid] = make_float4(wb.y0, wb.x0, wb.y1, wb.x1);
+}
+
+// pass 1 (fused path): everything that depends on ONE anchor only - row maximum / argmax, stage 1 of the matcher,
+// labels, encode, ALL outputs - plus the two cross-anchor quantities the later passes need: the per-GT column maxima
+// (atomicMax) and, for the mining matcher, the stage-3 candidates (overlap > stop_positive_thres) and the per-GT
+// match counts.  What stage 2 / the GT-side claim of the dual matcher changes afterwards is a handful of anchors per
+// GT; pass 2 finds and patches them.
+// TILED: the warps hold the tiles of the layout hint (A.warp_map != NULL); a separate instantiation because the kernel
+// sits on its register cap and the strip version can derive everything from threadIdx.  The cap is 40 registers: every
+// instantiation uses all 40 without spilling, and on B200 this build was 1 % faster than one capped at 32.  The culled
+// GT walk of an image and the row's end stay inline: as functions they reorder the front end's output, and ptxas then
+// allocates this register-capped kernel differently.
+template <bool NEED_ROW, bool MINING, bool TILED>
+__global__ void __maxnreg__(40) enc_pass1_fused_kernel(const EncArgs A, int batch, int coarse_chunks) {
+  const int lane = threadIdx.x & 31;
+  const int nwarps = (A.n + 31) >> 5;
+  const int nchunks = (A.n + kFusedThreads - 1) / kFusedThreads;
+  const Pass1Task t = pass1_task<TILED>(batch, coarse_chunks);
+  const int b0 = t.b0, b_end = t.b_end;
+  // the warp's index (wbest / wbox / queue entries are per warp) and its anchors
+  const int wid = (nchunks - 1 - t.from_end) * (kFusedThreads / 32) + (threadIdx.x >> 5);
+  const int a = TILED ? ((wid < nwarps) ? warp_anchor(A, wid, lane) : A.n) : wid * 32 + lane;
+  const bool valid = a < A.n;
+  AnchorBox ab;
+  AnchorCtr ac;
+  bool active;
+  WarpBox wb;
+  load_warp_anchors(A, a, valid, wid, nwarps, b0, lane, ab, ac, active, wb);
   const auto raw = [&] { return raw_anchor(A.ay0, A.ax0, A.ay1, A.ax1, a); };
   for (int b = b0; b < b_end; ++b) {
     const ImageGt ig = image_gt<false>(A, b);
@@ -590,8 +609,6 @@ enc_pass1_fused_kernel(const EncArgs A, int batch, int coarse_chunks) {
       }
     }
   }
-  DAN_P1_MARK(1, global_ns());
-  DAN_P1_MARK(2, (unsigned long long)(b_end - b0) | ((unsigned long long)from_end << 32));
 }
 
 // pass 2 (fused path): stage 2 of the mining matcher (small_mining_match.cc:160-197) / the GT-side claim of the dual
@@ -604,6 +621,146 @@ enc_pass1_fused_kernel(const EncArgs A, int batch, int coarse_chunks) {
 constexpr int kPatchThreads = 128;
 constexpr int kPatchGt = 1024;        // GT boxes staged in shared memory at a time
 
+// A warp's walk over the GTs of image `ig`, 32 per ballot: each GT k for which test(wide, column maximum, box) holds on
+// its lane (wide: see the file header) is broadcast, and every lane runs visit(k, its overlap (0 if inactive), col. max)
+template <bool MINING, typename Test, typename Visit>
+DAN_D void walk_gts(const EncArgs& A, const ImageGt& ig, int lane, bool active, const AnchorBox& ab, Test test,
+                    Visit visit) {
+  for (int k0 = 0; k0 < ig.m_eff; k0 += 32) {
+    const int k = k0 + lane;
+    bool t = false;
+    float cmk = 0.f;                                   // GT k's column maximum and box
+    float4 gk = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (k < ig.m_eff) {
+      cmk = __uint_as_float(__ldg(A.colmax + ig.slot0 + k));
+      gk = gt_box(A, ig, k);
+      t = test(MINING ? (cmk < FLT_EPSILON) : (cmk == 0.f), cmk, gk);
+    }
+    unsigned hits = __ballot_sync(0xffffffffu, t);
+    while (hits) {
+      const int kl = __ffs(hits) - 1;
+      hits &= hits - 1;
+      const float4 g = make_float4(__shfl_sync(0xffffffffu, gk.x, kl), __shfl_sync(0xffffffffu, gk.y, kl),
+                                   __shfl_sync(0xffffffffu, gk.z, kl), __shfl_sync(0xffffffffu, gk.w, kl));
+      const float cm = __shfl_sync(0xffffffffu, cmk, kl);
+      bool hit = false;
+      float ov = 0.f;
+      if (active) ov = pair_iou(ab.my0, ab.mx0, ab.my1, ab.mx1, ab.marea, g.x, g.y, g.z, g.w, box_area(g.x, g.y, g.z, g.w), hit);
+      visit(k0 + kl, ov, cm);
+    }
+  }
+}
+
+// Shared arrays of enc_pass2_find_kernel: staged GT boxes and column maxima, the warps level 1 lists (reach, box, flag).
+// Separate __shared__ arrays behind pointers: as one __shared__ struct they cost the kernel two more registers.
+struct FindSmem {
+  int* list;        // [kPatchThreads]: the listed warps of pass 1 ...
+  float* reach;     //   ... their reach (wbest, widened by the mining tie band) ...
+  float4* wbox;     //   ... their bounding box ...
+  int* flag;        //   ... and whether they go to the queue
+  float4* box;      // [kPatchGt]: staged GT boxes ...
+  float* cm;        //   ... and column maxima
+  int& n;           // listed warps
+  float* cmin;      // [kPatchThreads / 32]: per-warp partial minimum column maximum ...
+  int* wide;        //   ... and "wide" flag
+};
+
+// The smallest column maximum of image `ig` and whether a GT ties with zero-overlap anchors (wide), over the CTA; with
+// `staged` the GT boxes and column maxima are staged in S on the way.  Ends with a barrier.
+template <bool MINING>
+DAN_D void summarize_columns(const EncArgs& A, const ImageGt& ig, bool staged, const FindSmem& S, float& cmin,
+                             bool& wide) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  cmin = 3.0e38f;
+  wide = false;
+  for (int k = tid; k < ig.m_eff; k += kPatchThreads) {
+    const float cm = __uint_as_float(A.colmax[ig.slot0 + k]);
+    if (staged) {
+      S.cm[k] = cm;
+      S.box[k] = gt_box(A, ig, k);
+    }
+    wide |= MINING ? (cm < FLT_EPSILON) : (cm == 0.f);
+    cmin = fminf(cmin, cm);
+  }
+  cmin = warp_min_f(cmin);
+  wide = __any_sync(0xffffffffu, wide);
+  if (lane == 0) { S.cmin[warp] = cmin; S.wide[warp] = wide ? 1 : 0; }
+  if (tid == 0) S.n = 0;
+  __syncthreads();
+#pragma unroll
+  for (int w = 0; w < kPatchThreads / 32; ++w) { cmin = fminf(cmin, S.cmin[w]); wide |= S.wide[w] != 0; }
+}
+
+// Level 1, a thread per warp of pass 1: can the warp reach the smallest column maximum at all?  Lists those that can in
+// S (flagged at once when the image is wide) and returns their number, after a barrier.
+template <bool MINING>
+DAN_D int list_reaching_warps(const EncArgs& A, int b, float cmin, bool wide, const FindSmem& S) {
+  const int nwarps = (A.n + 31) >> 5;
+  const int wr = blockIdx.y * kPatchThreads + threadIdx.x;
+  bool cand = false;
+  float my_reach = 0.f;
+  if (wr < nwarps) {
+    const float wb = A.wbest[(int64_t)b * nwarps + wr];
+    my_reach = MINING ? fadd(wb, 2.f * FLT_EPSILON) : wb;
+    cand = wide || (my_reach >= cmin);
+  }
+  if (cand) {
+    const int pos = atomicAdd(&S.n, 1);
+    S.list[pos] = wr;
+    S.reach[pos] = my_reach;
+    S.wbox[pos] = A.wbox[wr];                                 // (all candidates of the CTA in one round trip)
+    S.flag[pos] = wide ? 1 : 0;
+  }
+  __syncthreads();
+  return S.n;
+}
+
+// Level 2, still without touching the anchors: flag a listed warp if some GT's column maximum is within its reach AND the
+// GT's box meets its bounding box; a warp tests 32 GTs per step for each of its list entries.  Ends with a barrier.
+DAN_D void flag_box_hits(const EncArgs& A, const ImageGt& ig, bool staged, int n_list, const FindSmem& S) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  for (int c0 = 0; c0 < ig.m_eff; c0 += kPatchGt) {
+    const int mc = min(kPatchGt, ig.m_eff - c0);
+    if (!staged) {
+      __syncthreads();
+      for (int k = tid; k < mc; k += kPatchThreads) {
+        S.box[k] = gt_box(A, ig, c0 + k);
+        S.cm[k] = __uint_as_float(A.colmax[ig.slot0 + c0 + k]);
+      }
+      __syncthreads();
+    }
+    for (int i = warp; i < n_list; i += kPatchThreads / 32) {
+      if (S.flag[i]) continue;                               // (warp-uniform)
+      const float reach_w = S.reach[i];
+      const float4 wq = S.wbox[i];
+      const WarpBox wrec = {wq.x, wq.y, wq.z, wq.w};
+      bool any = false;
+      for (int k0 = 0; k0 < mc && !any; k0 += 32) {
+        const int k = k0 + lane;
+        any = __any_sync(0xffffffffu, (k < mc) && (S.cm[k] <= reach_w) && may_hit(wrec, S.box[k]));
+      }
+      if (any && lane == 0) S.flag[i] = 1;
+      __syncwarp();
+    }
+  }
+  __syncthreads();
+}
+
+// The flagged warps go to the batch-wide queue of enc_pass2_apply_kernel: they cluster in a few CTAs (the coarse levels
+// meet every GT), and each costs a chain of dependent loads, so they are spread over the whole GPU
+DAN_D void enqueue_flagged(const EncArgs& A, int b, int n_list, const FindSmem& S) {
+  const int tid = threadIdx.x, lane = tid & 31;
+  const bool flagged = tid < n_list && S.flag[tid] != 0;
+  const unsigned fm = __ballot_sync(0xffffffffu, flagged);
+  if (fm != 0u) {
+    int base = 0;
+    if (lane == 0) base = atomicAdd(A.queue_n, __popc(fm));
+    base = __shfl_sync(0xffffffffu, base, 0);
+    if (flagged) A.queue[base + __popc(fm & ((1u << lane) - 1u))] = make_int2(b, S.list[tid]);
+  }
+}
+
+// first and second level of pass 2, one CTA per (image, 128 warps of pass 1)
 template <bool MINING>
 __global__ void __launch_bounds__(kPatchThreads) enc_pass2_find_kernel(const EncArgs A) {
   __shared__ int s_list[kPatchThreads];
@@ -615,95 +772,18 @@ __global__ void __launch_bounds__(kPatchThreads) enc_pass2_find_kernel(const Enc
   __shared__ int s_n;
   __shared__ float s_cmin[kPatchThreads / 32];
   __shared__ int s_wide[kPatchThreads / 32];
+  const FindSmem S = {s_list, s_reach, s_wbox, s_flag, s_box, s_cm, s_n, s_cmin, s_wide};
   const int b = blockIdx.x;
-  const int tid = threadIdx.x;
-  const int lane = tid & 31;
-  const int warp = tid >> 5;
-  const int nwarps = (A.n + 31) >> 5;
   const ImageGt ig = image_gt<false>(A, b);
-  const bool need_haspos = !MINING && !A.gt_max_first;
   // the usual case: all GT boxes and column maxima of the image fit the staging arrays and stay there
   const bool staged = ig.m_eff <= kPatchGt;
-
-  // smallest column maximum of the image; does any GT tie with zero-overlap anchors?
-  float cmin = 3.0e38f;
-  bool wide = false;
-  for (int k = tid; k < ig.m_eff; k += kPatchThreads) {
-    const float cm = __uint_as_float(A.colmax[ig.slot0 + k]);
-    if (staged) {
-      s_cm[k] = cm;
-      s_box[k] = gt_box(A, ig, k);
-    }
-    wide |= MINING ? (cm < FLT_EPSILON) : (cm == 0.f);
-    cmin = fminf(cmin, cm);
-  }
-  cmin = warp_min_f(cmin);
-  wide = __any_sync(0xffffffffu, wide);
-  if (lane == 0) { s_cmin[warp] = cmin; s_wide[warp] = wide ? 1 : 0; }
-  if (tid == 0) s_n = 0;
-  __syncthreads();
-#pragma unroll
-  for (int w = 0; w < kPatchThreads / 32; ++w) { cmin = fminf(cmin, s_cmin[w]); wide |= s_wide[w] != 0; }
-
-  // first level, one thread per warp of pass 1: can the warp reach the smallest column maximum at all?
-  const int wr = blockIdx.y * kPatchThreads + tid;
-  bool cand = false;
-  float my_reach = 0.f;
-  if (wr < nwarps) {
-    const float wb = A.wbest[(int64_t)b * nwarps + wr];
-    my_reach = MINING ? fadd(wb, 2.f * FLT_EPSILON) : wb;
-    cand = wide || (my_reach >= cmin);
-  }
-  if (cand) {
-    const int pos = atomicAdd(&s_n, 1);
-    s_list[pos] = wr;
-    s_reach[pos] = my_reach;
-    s_wbox[pos] = A.wbox[wr];                                 // (all candidates of the CTA in one round trip)
-    s_flag[pos] = wide ? 1 : 0;
-  }
-  __syncthreads();
-  const int n_list = s_n;
+  float cmin;
+  bool wide;
+  summarize_columns<MINING>(A, ig, staged, S, cmin, wide);
+  const int n_list = list_reaching_warps<MINING>(A, b, cmin, wide, S);
   if (n_list == 0) return;                                   // (CTA-uniform)
-
-  // second level, still without touching the anchors: is there a GT whose column maximum the warp can reach AND whose
-  // box meets the warp's bounding box?  A warp tests 32 GTs per step for each of its list entries.
-  if (!wide) {
-    for (int c0 = 0; c0 < ig.m_eff; c0 += kPatchGt) {
-      const int mc = min(kPatchGt, ig.m_eff - c0);
-      if (!staged) {
-        __syncthreads();
-        for (int k = tid; k < mc; k += kPatchThreads) {
-          s_box[k] = gt_box(A, ig, c0 + k);
-          s_cm[k] = __uint_as_float(A.colmax[ig.slot0 + c0 + k]);
-        }
-        __syncthreads();
-      }
-      for (int i = warp; i < n_list; i += kPatchThreads / 32) {
-        if (s_flag[i]) continue;                             // (warp-uniform)
-        const float reach_w = s_reach[i];
-        const float4 wq = s_wbox[i];
-        const WarpBox wrec = {wq.x, wq.y, wq.z, wq.w};
-        bool any = false;
-        for (int k0 = 0; k0 < mc && !any; k0 += 32) {
-          const int k = k0 + lane;
-          any = __any_sync(0xffffffffu, (k < mc) && (s_cm[k] <= reach_w) && may_hit(wrec, s_box[k]));
-        }
-        if (any && lane == 0) s_flag[i] = 1;
-        __syncwarp();
-      }
-    }
-    __syncthreads();
-  }
-  // the flagged warps go to the batch-wide work queue of enc_pass2_apply_kernel: they cluster in a few CTAs (the coarse
-  // pyramid levels meet every GT), and each costs a chain of dependent loads, so they are spread over the whole GPU
-  const bool flagged = tid < n_list && s_flag[tid] != 0;
-  const unsigned fm = __ballot_sync(0xffffffffu, flagged);
-  if (fm != 0u) {
-    int base = 0;
-    if (lane == 0) base = atomicAdd(A.queue_n, __popc(fm));
-    base = __shfl_sync(0xffffffffu, base, 0);
-    if (flagged) A.queue[base + __popc(fm & ((1u << lane) - 1u))] = make_int2(b, s_list[tid]);
-  }
+  if (!wide) flag_box_hits(A, ig, staged, n_list, S);
+  enqueue_flagged(A, b, n_list, S);
 }
 
 // third level of pass 2: one warp per queued (image, warp of pass 1): load the anchors, evaluate the GTs the warp can
@@ -720,8 +800,6 @@ __global__ void __launch_bounds__(kPatchThreads) enc_pass2_apply_kernel(const En
     const int2 q = A.queue[e];
     const int b = q.x;
     const ImageGt ig = image_gt<false>(A, b);
-    auto box_at = [&](int k) { return gt_box(A, ig, k); };
-    auto cm_at = [&](int k) { return __uint_as_float(__ldg(A.colmax + ig.slot0 + k)); };
     const int a = warp_anchor(A, q.y, lane);
     const bool valid = a < A.n;
     const float wb = A.wbest[(int64_t)b * nwarps + q.y];
@@ -735,79 +813,29 @@ __global__ void __launch_bounds__(kPatchThreads) enc_pass2_apply_kernel(const En
     const WarpBox wbx = warp_bbox(active, ab);
     // the GTs the warp can reach: does any anchor really tie with / get claimed by one?
     bool tie = false;
-    for (int k0 = 0; k0 < ig.m_eff; k0 += 32) {
-      const int k = k0 + lane;
-      bool test = false;
-      float cmk = 0.f;
-      float4 gk = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (k < ig.m_eff) {
-        cmk = cm_at(k);
-        gk = box_at(k);
-        const bool widek = MINING ? (cmk < FLT_EPSILON) : (cmk == 0.f);
-        test = widek || (cmk <= reach_w && may_hit(wbx, gk));
-      }
-      unsigned hits = __ballot_sync(0xffffffffu, test);
-      while (hits) {
-        const int kl = __ffs(hits) - 1;
-        const int kk = k0 + kl;
-        hits &= hits - 1;
-        const float4 g = make_float4(__shfl_sync(0xffffffffu, gk.x, kl), __shfl_sync(0xffffffffu, gk.y, kl),
-                                     __shfl_sync(0xffffffffu, gk.z, kl), __shfl_sync(0xffffffffu, gk.w, kl));
-        const float cm = __shfl_sync(0xffffffffu, cmk, kl);
-        bool hit = false;
-        float ov = 0.f;
-        if (active) ov = pair_iou(ab.my0, ab.mx0, ab.my1, ab.mx1, ab.marea, g.x, g.y, g.z, g.w, box_area(g.x, g.y, g.z, g.w), hit);
-        if (MINING) tie |= fabsf(fsub(ov, cm)) < FLT_EPSILON;
-        else tie |= (ov == cm) && (!need_haspos || A.haspos[ig.slot0 + kk] == 0);
-      }
-    }
+    walk_gts<MINING>(A, ig, lane, active, ab,
+                     [&](bool widek, float cmk, float4 gk) { return widek || (cmk <= reach_w && may_hit(wbx, gk)); },
+                     [&](int kk, float ov, float cm) {
+                       if (MINING) tie |= fabsf(fsub(ov, cm)) < FLT_EPSILON;
+                       else tie |= (ov == cm) && (!need_haspos || A.haspos[ig.slot0 + kk] == 0);
+                     });
     if (!__any_sync(0xffffffffu, tie && valid)) continue;
     // the full row again, then the patch
     RowState s;
-    for (int k0 = 0; k0 < ig.m_eff; k0 += 32) {
-      const int k = k0 + lane;
-      bool test = false;
-      float cmk = 0.f;
-      float4 gk = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (k < ig.m_eff) {
-        cmk = cm_at(k);
-        gk = box_at(k);
-        const bool widek = MINING ? (cmk < FLT_EPSILON) : (cmk == 0.f);
-        test = may_hit(wbx, gk) || widek;
-      }
-      unsigned hits = __ballot_sync(0xffffffffu, test);
-      while (hits) {
-        const int kl = __ffs(hits) - 1;
-        const int kk = k0 + kl;
-        hits &= hits - 1;
-        const float4 g = make_float4(__shfl_sync(0xffffffffu, gk.x, kl), __shfl_sync(0xffffffffu, gk.y, kl),
-                                     __shfl_sync(0xffffffffu, gk.z, kl), __shfl_sync(0xffffffffu, gk.w, kl));
-        const float cm = __shfl_sync(0xffffffffu, cmk, kl);
-        bool hit = false;
-        float ov = 0.f;
-        if (active) ov = pair_iou(ab.my0, ab.mx0, ab.my1, ab.mx1, ab.marea, g.x, g.y, g.z, g.w, box_area(g.x, g.y, g.z, g.w), hit);
-        const bool claimable = !need_haspos || A.haspos[ig.slot0 + kk] == 0;
-        row_update<MINING>(s, kk, ov, cm, claimable);
-      }
-    }
+    walk_gts<MINING>(A, ig, lane, active, ab, [&](bool widek, float, float4 gk) { return may_hit(wbx, gk) || widek; },
+                     [&](int kk, float ov, float cm) {
+                       row_update<MINING>(s, kk, ov, cm, !need_haspos || A.haspos[ig.slot0 + kk] == 0);
+                     });
     if (!valid) continue;
     const int match1 = stage1_match<MINING>(A, s.best, s.best_gt);
-    int match = match1;
-    float score = s.best;
-    if (MINING) {
-      if (s.owner >= 0) { match = s.owner; score = s.owner_ov; }     // stage 2, :178-186 (the last tied GT wins)
-      if (match != match1) {
-        if (match1 >= 0) atomicSub(A.cnt + ig.slot0 + match1, 1);
-        atomicAdd(A.cnt + ig.slot0 + match, 1);
-      }
-    } else if (s.claimed) {
-      // :95-104 GT-side claim has priority; argmax over (overlap * claim mask); claimed only through zero-overlap
-      // ties: the argmax of an all-zero row is GT 0, the score is its overlap
-      if (s.cbest > 0.f) { match = s.cbest_gt; score = s.cbest; }
-      else { match = 0; score = s.ov0; }
+    float score;
+    const int match = stage2_match<MINING>(A, s, score);
+    if (MINING && match != match1) {
+      if (match1 >= 0) atomicSub(A.cnt + ig.slot0 + match1, 1);
+      atomicAdd(A.cnt + ig.slot0 + match, 1);
     }
     if (match != match1 || score != s.best)
-      write_positive(A, (int64_t)b * A.n + a, ab, box_at(match), score, match);
+      write_positive(A, (int64_t)b * A.n + a, ab, gt_box(A, ig, match), score, match);
   }
 }
 
@@ -996,158 +1024,182 @@ struct P3Smem {
   int warp_cnt[kP3Warps];
 };
 
+// The GTs of [j0, j0 + kP3Range) short of min_match, ascending, with need and bucket fill into S.needy_*; their number
+DAN_D int list_needy(const EncArgs& A, const ImageGt& ig, int j0, P3Smem& S) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  int nneedy = 0;
+  for (int jb = 0; jb < kP3Range && j0 + jb < ig.m_eff; jb += kP3Threads) {
+    const int j = j0 + jb + tid;
+    int need = 0, fill = 0;
+    if (j < ig.m_eff) {
+      need = A.min_match - A.cnt[ig.slot0 + j];
+      fill = A.fill[ig.slot0 + j];
+    }
+    const unsigned m = __ballot_sync(0xffffffffu, need > 0);
+    if (lane == 0) S.warp_cnt[warp] = __popc(m);
+    __syncthreads();
+    int before = nneedy;
+    for (int w = 0; w < kP3Warps; ++w) {
+      if (w < warp) before += S.warp_cnt[w];
+      nneedy += S.warp_cnt[w];
+    }
+    if (need > 0) {
+      const int pos = before + __popc(m & ((1u << lane) - 1u));
+      S.needy_j[pos] = j;
+      S.needy_need[pos] = need;
+      S.needy_fill[pos] = fill;
+    }
+    __syncthreads();
+  }
+  return nneedy;
+}
+
+// Needy GT q, whose bucket overflowed, by one warp: rescan every anchor of the image in index order; everything before
+// this GT is already in the outputs, the GT is alone in its "window", and its patches are applied at once
+template <bool DENSE>
+DAN_D void rescan_overflowed(const EncArgs& A, const ImageGt& ig, int b, int q, const P3Smem& S) {
+  const int lane = threadIdx.x & 31;
+  const int gj = S.needy_j[q];
+  HeapItem* list = A.spill + (int64_t)b * 2 * A.n;   // then the heap of compensate_from_spill
+  int c = 0;
+  const float4 gb = DENSE ? make_float4(0.f, 0.f, 0.f, 0.f) : gt_box(A, ig, gj);
+  const float garea = box_area(gb.x, gb.y, gb.z, gb.w);
+  for (int a0 = 0; a0 < A.n; a0 += 32) {
+    const int a = a0 + lane;
+    bool ok = false;
+    float ov = 0.f;
+    if (a < A.n) {
+      if (DENSE) {
+        ov = A.overlaps[(int64_t)a * ig.m_eff + gj];
+      } else if (A.mask == nullptr || A.mask[a] != 0) {
+        const AnchorBox ab = load_anchor(A, a);
+        bool hit;
+        ov = pair_iou(ab.my0, ab.mx0, ab.my1, ab.mx1, ab.marea, gb.x, gb.y, gb.z, gb.w, garea, hit);
+      }
+      ok = (ov > A.stop) && still_unmatched<DENSE>(A, (int64_t)b * A.n + a);
+    }
+    const unsigned mm = __ballot_sync(0xffffffffu, ok);
+    if (ok) list[c + __popc(mm & ((1u << lane) - 1u))] = HeapItem{ov, a};
+    c += __popc(mm);
+  }
+  __threadfence_block();
+  __syncwarp();
+  compensate_from_spill<DENSE>(A, ig, b, gj, S.needy_need[q], list, c, list + A.n);
+}
+
+// the end q1 of the window [q0, q1): consecutive needy GTs with intact buckets, at most kP3Window, kP3SelCap selections
+DAN_D int window_end(const P3Smem& S, int q0, int nneedy) {
+  int q1 = q0, budget = 0;
+  while (q1 < nneedy && q1 - q0 < kP3Window && S.needy_fill[q1] <= kBucketCap) {
+    const int take = min(S.needy_need[q1], S.needy_fill[q1]);
+    if (q1 > q0 && budget + take > kP3SelCap) break;
+    budget += take;
+    ++q1;
+  }
+  return q1;
+}
+
+// The candidates of the window's nq GTs, and which of them are still unmatched after stage 2 and after the windows
+// before this one (already in HBM).  Ends with a barrier.
+template <bool DENSE>
+DAN_D void load_window(const EncArgs& A, const ImageGt& ig, int b, int q0, int nq, P3Smem& S) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int g = warp; g < nq; g += kP3Warps) {
+    const int gj = S.needy_j[q0 + g], gfill = S.needy_fill[q0 + g];
+    bool a0 = false, a1 = false;
+    if (lane < gfill) {
+      const HeapItem it = A.bucket[(int64_t)(ig.slot0 + gj) * kBucketCap + lane];
+      S.cand[g][lane] = it;
+      a0 = still_unmatched<DENSE>(A, (int64_t)b * A.n + it.id);
+    }
+    if (lane + 32 < gfill) {
+      const HeapItem it = A.bucket[(int64_t)(ig.slot0 + gj) * kBucketCap + lane + 32];
+      S.cand[g][lane + 32] = it;
+      a1 = still_unmatched<DENSE>(A, (int64_t)b * A.n + it.id);
+    }
+    const unsigned lo = __ballot_sync(0xffffffffu, a0), hi = __ballot_sync(0xffffffffu, a1);
+    if (lane == 0) {
+      S.alive[g] = ((unsigned long long)hi << 32) | lo;
+      S.blocked[g] = 0ull;
+      S.dirty[g] = 1;
+    }
+  }
+  __syncthreads();
+}
+
+// The fixed-point rounds of the window, until no blocked set changes; the selections are left in S.sel (CTA-uniform)
+DAN_D void resolve_window(int q0, int nq, P3Smem& S) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const P3Hash hash{S.hash_key, S.hash_val};
+  while (true) {
+    for (int g = warp; g < nq; g += kP3Warps) {
+      if (S.dirty[g] == 0) continue;                        // (warp-uniform: written by this warp in the last round)
+      const unsigned long long live = S.alive[g] & ~S.blocked[g];
+      const unsigned long long sel = select_from_bucket(S.cand[g], S.needy_fill[q0 + g], live, S.needy_need[q0 + g],
+                                                        S.sort_buf[warp], S.heap[warp], S.sort_slot[warp]);
+      if (lane == 0) S.sel[g] = sel;
+    }
+    for (int i = tid; i < kP3Hash; i += kP3Threads) { S.hash_key[i] = -1; S.hash_val[i] = 0x7fffffff; }
+    __syncthreads();
+    if (nq == 1) break;                                     // a lone GT has nobody to compete with
+    for (int g = warp; g < nq; g += kP3Warps) {
+      const unsigned long long sel = S.sel[g];
+      if ((sel >> lane) & 1ull) p3_hash_put(hash, S.cand[g][lane].id, g);
+      if ((sel >> (lane + 32)) & 1ull) p3_hash_put(hash, S.cand[g][lane + 32].id, g);
+    }
+    __syncthreads();
+    bool changed = false;
+    for (int g = warp; g < nq; g += kP3Warps) {
+      const unsigned long long alive = S.alive[g];
+      const bool b0 = ((alive >> lane) & 1ull) && p3_hash_get(hash, S.cand[g][lane].id) < g;
+      const bool b1 = ((alive >> (lane + 32)) & 1ull) && p3_hash_get(hash, S.cand[g][lane + 32].id) < g;
+      const unsigned lo = __ballot_sync(0xffffffffu, b0), hi = __ballot_sync(0xffffffffu, b1);
+      const unsigned long long blocked = ((unsigned long long)hi << 32) | lo;
+      const bool diff = blocked != S.blocked[g];
+      changed |= diff;
+      __syncwarp();
+      if (lane == 0) {
+        S.blocked[g] = blocked;
+        S.dirty[g] = diff ? 1 : 0;
+      }
+    }
+    if (!__syncthreads_or(changed ? 1 : 0)) break;
+  }
+}
+
+// the window's selections go to the outputs (by all warps); ends with a barrier
+template <bool DENSE>
+DAN_D void apply_window(const EncArgs& A, const ImageGt& ig, int b, int q0, int nq, const P3Smem& S) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int g = warp; g < nq; g += kP3Warps) {
+    const unsigned long long sel = S.sel[g];
+    const int gj = S.needy_j[q0 + g];
+    if ((sel >> lane) & 1ull) apply_compensation<DENSE>(A, ig, b, S.cand[g][lane].id, gj, S.cand[g][lane].key);
+    if ((sel >> (lane + 32)) & 1ull) apply_compensation<DENSE>(A, ig, b, S.cand[g][lane + 32].id, gj, S.cand[g][lane + 32].key);
+  }
+  __syncthreads();
+}
+
 template <bool DENSE>
 __global__ void __launch_bounds__(kP3Threads) enc_pass3_kernel(const EncArgs A) {
   extern __shared__ __align__(16) unsigned char p3_raw[];
   P3Smem& S = *reinterpret_cast<P3Smem*>(p3_raw);
-
   const int b = blockIdx.x;
-  const int tid = threadIdx.x;
-  const int lane = tid & 31;
-  const int warp = tid >> 5;
-  const unsigned lt_mask = (1u << lane) - 1u;
   const ImageGt ig = image_gt<DENSE>(A, b);
-  const P3Hash hash{S.hash_key, S.hash_val};
-
   for (int j0 = 0; j0 < ig.m_eff; j0 += kP3Range) {
-    // ---- GTs of this range that are short of min_match, in ascending order
-    int nneedy = 0;
-    for (int jb = 0; jb < kP3Range && j0 + jb < ig.m_eff; jb += kP3Threads) {
-      const int j = j0 + jb + tid;
-      int need = 0, fill = 0;
-      if (j < ig.m_eff) {
-        need = A.min_match - A.cnt[ig.slot0 + j];
-        fill = A.fill[ig.slot0 + j];
-      }
-      const unsigned m = __ballot_sync(0xffffffffu, need > 0);
-      if (lane == 0) S.warp_cnt[warp] = __popc(m);
-      __syncthreads();
-      int before = nneedy;
-      for (int w = 0; w < kP3Warps; ++w) {
-        if (w < warp) before += S.warp_cnt[w];
-        nneedy += S.warp_cnt[w];
-      }
-      if (need > 0) {
-        const int pos = before + __popc(m & lt_mask);
-        S.needy_j[pos] = j;
-        S.needy_need[pos] = need;
-        S.needy_fill[pos] = fill;
-      }
-      __syncthreads();
-    }
-
+    const int nneedy = list_needy(A, ig, j0, S);
     int q0 = 0;
     while (q0 < nneedy) {                                    // (all decisions below are CTA-uniform)
       if (S.needy_fill[q0] > kBucketCap) {
-        // ---- bucket overflowed: rescan every anchor of the image in index order; everything before this GT is already
-        // in the outputs, the GT is alone in its "window", and its patches are applied at once (warp 0)
-        if (warp == 0) {
-          const int gj = S.needy_j[q0];
-          HeapItem* list = A.spill + (int64_t)b * 2 * A.n;
-          int c = 0;
-          const float4 gb = DENSE ? make_float4(0.f, 0.f, 0.f, 0.f) : gt_box(A, ig, gj);
-          const float garea = box_area(gb.x, gb.y, gb.z, gb.w);
-          for (int a0 = 0; a0 < A.n; a0 += 32) {
-            const int a = a0 + lane;
-            bool ok = false;
-            float ov = 0.f;
-            if (a < A.n) {
-              if (DENSE) {
-                ov = A.overlaps[(int64_t)a * ig.m_eff + gj];
-              } else if (A.mask == nullptr || A.mask[a] != 0) {
-                const AnchorBox ab = load_anchor(A, a);
-                bool hit;
-                ov = pair_iou(ab.my0, ab.mx0, ab.my1, ab.mx1, ab.marea, gb.x, gb.y, gb.z, gb.w, garea, hit);
-              }
-              ok = (ov > A.stop) && still_unmatched<DENSE>(A, (int64_t)b * A.n + a);
-            }
-            const unsigned mm = __ballot_sync(0xffffffffu, ok);
-            if (ok) list[c + __popc(mm & lt_mask)] = HeapItem{ov, a};
-            c += __popc(mm);
-          }
-          __threadfence_block();
-          __syncwarp();
-          compensate_from_spill<DENSE>(A, ig, b, gj, S.needy_need[q0], list, c, list + A.n);
-        }
+        if ((threadIdx.x >> 5) == 0) rescan_overflowed<DENSE>(A, ig, b, q0, S);
         __syncthreads();
         q0 += 1;
         continue;
       }
-      // ---- window [q0, q1): consecutive needy GTs with intact buckets, at most kP3SelCap selections in total
-      int q1 = q0, budget = 0;
-      while (q1 < nneedy && q1 - q0 < kP3Window && S.needy_fill[q1] <= kBucketCap) {
-        const int take = min(S.needy_need[q1], S.needy_fill[q1]);
-        if (q1 > q0 && budget + take > kP3SelCap) break;
-        budget += take;
-        ++q1;
-      }
-      const int nq = q1 - q0;
-      // candidates still unmatched after stage 2 and after the windows before this one (already in HBM)
-      for (int g = warp; g < nq; g += kP3Warps) {
-        const int gj = S.needy_j[q0 + g], gfill = S.needy_fill[q0 + g];
-        bool a0 = false, a1 = false;
-        if (lane < gfill) {
-          const HeapItem it = A.bucket[(int64_t)(ig.slot0 + gj) * kBucketCap + lane];
-          S.cand[g][lane] = it;
-          a0 = still_unmatched<DENSE>(A, (int64_t)b * A.n + it.id);
-        }
-        if (lane + 32 < gfill) {
-          const HeapItem it = A.bucket[(int64_t)(ig.slot0 + gj) * kBucketCap + lane + 32];
-          S.cand[g][lane + 32] = it;
-          a1 = still_unmatched<DENSE>(A, (int64_t)b * A.n + it.id);
-        }
-        const unsigned lo = __ballot_sync(0xffffffffu, a0), hi = __ballot_sync(0xffffffffu, a1);
-        if (lane == 0) {
-          S.alive[g] = ((unsigned long long)hi << 32) | lo;
-          S.blocked[g] = 0ull;
-          S.dirty[g] = 1;
-        }
-      }
-      __syncthreads();
-      // ---- rounds
-      while (true) {
-        // selections under the current blocked sets (a GT whose blocked set did not change keeps its selection)
-        for (int g = warp; g < nq; g += kP3Warps) {
-          if (S.dirty[g] == 0) continue;                        // (warp-uniform: written by this warp in the last round)
-          const unsigned long long live = S.alive[g] & ~S.blocked[g];
-          const unsigned long long sel = select_from_bucket(S.cand[g], S.needy_fill[q0 + g], live, S.needy_need[q0 + g],
-                                                            S.sort_buf[warp], S.heap[warp], S.sort_slot[warp]);
-          if (lane == 0) S.sel[g] = sel;
-        }
-        for (int i = tid; i < kP3Hash; i += kP3Threads) { S.hash_key[i] = -1; S.hash_val[i] = 0x7fffffff; }
-        __syncthreads();
-        if (nq == 1) break;                                     // a lone GT has nobody to compete with
-        for (int g = warp; g < nq; g += kP3Warps) {
-          const unsigned long long sel = S.sel[g];
-          if ((sel >> lane) & 1ull) p3_hash_put(hash, S.cand[g][lane].id, g);
-          if ((sel >> (lane + 32)) & 1ull) p3_hash_put(hash, S.cand[g][lane + 32].id, g);
-        }
-        __syncthreads();
-        bool changed = false;
-        for (int g = warp; g < nq; g += kP3Warps) {
-          const unsigned long long alive = S.alive[g];
-          const bool b0 = ((alive >> lane) & 1ull) && p3_hash_get(hash, S.cand[g][lane].id) < g;
-          const bool b1 = ((alive >> (lane + 32)) & 1ull) && p3_hash_get(hash, S.cand[g][lane + 32].id) < g;
-          const unsigned lo = __ballot_sync(0xffffffffu, b0), hi = __ballot_sync(0xffffffffu, b1);
-          const unsigned long long blocked = ((unsigned long long)hi << 32) | lo;
-          const bool diff = blocked != S.blocked[g];
-          changed |= diff;
-          __syncwarp();
-          if (lane == 0) {
-            S.blocked[g] = blocked;
-            S.dirty[g] = diff ? 1 : 0;
-          }
-        }
-        if (!__syncthreads_or(changed ? 1 : 0)) break;
-      }
-      // ---- the window's selections go to the outputs
-      for (int g = warp; g < nq; g += kP3Warps) {
-        const unsigned long long sel = S.sel[g];
-        const int gj = S.needy_j[q0 + g];
-        if ((sel >> lane) & 1ull) apply_compensation<DENSE>(A, ig, b, S.cand[g][lane].id, gj, S.cand[g][lane].key);
-        if ((sel >> (lane + 32)) & 1ull) apply_compensation<DENSE>(A, ig, b, S.cand[g][lane + 32].id, gj, S.cand[g][lane + 32].key);
-      }
-      __syncthreads();
+      const int q1 = window_end(S, q0, nneedy);
+      load_window<DENSE>(A, ig, b, q0, q1 - q0, S);
+      resolve_window(q0, q1 - q0, S);
+      apply_window<DENSE>(A, ig, b, q0, q1 - q0, S);
       q0 = q1;
     }
     __syncthreads();
@@ -1243,7 +1295,7 @@ static void bind_workspace(EncArgs& A, void* workspace, const WsLayout& w) {
 template <bool NEED_ROW, bool MINING, bool TILED>
 static void launch_pass1(const EncArgs& A, int batch, int fine_chunks, cudaStream_t st) {
   const int coarse_chunks = (A.n + kFusedThreads - 1) / kFusedThreads - fine_chunks;
-  const int grid = coarse_chunks * batch + fine_chunks * ((batch + kFineImages - 1) / kFineImages);
+  const int grid = pass1_grid(batch, coarse_chunks, fine_chunks);
   enc_pass1_fused_kernel<NEED_ROW, MINING, TILED><<<grid, kFusedThreads, 0, st>>>(A, batch, coarse_chunks);
 }
 
@@ -1330,13 +1382,6 @@ static int timed_sequence(int n_events, float* h_ms, Fn fn) {
 using namespace dan;
 
 extern "C" {
-
-#ifdef DAN_PASS1_TIMELINE
-int dan_debug_pass1_timeline(unsigned long long* h_out, int32_t warps) {
-  if (warps < 0 || warps > kTimelineWarps) return DAN_ERR_INVALID_ARGUMENT;
-  return cudaMemcpyFromSymbol(h_out, g_p1_timeline, sizeof(unsigned long long) * 3 * warps) == cudaSuccess ? DAN_OK : -3;
-}
-#endif
 
 size_t dan_match_workspace_bytes(int32_t num_anchors, int32_t num_gt) {
   if (num_anchors < 0 || num_gt < 0) return 0;
