@@ -18,7 +18,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libdan_b200.so")
-SOURCES = ["api.cu", "anchors.cu", "encode.cu", "postprocess.cu", "mining.cu", "routing.cu", "vote.cu", "handoff.cu", "gather.cu"]
+SOURCES = ["api.cu", "anchors.cu", "encode.cu", "postprocess.cu", "mining.cu", "routing.cu", "vote.cu", "detect_face.cu", "handoff.cu", "gather.cu"]
 HEADERS = ["common.cuh", "heap_order.cuh", "sort.cuh", os.path.join(ROOT, "include", "dan_b200.h")]
 
 NVCC_FLAGS = [
